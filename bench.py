@@ -4,6 +4,7 @@ data_cases.py:269-291; README/BASELINE.json say 76), FP32 fast mode, env batch s
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our arm (CUDA kernels through the C-ABI)
     python bench.py --impl reference [--gpus N] ...                 # the reference's CPU path (oracle port, all cores)
+    python bench.py ... --dump-outputs DIR                          # also write the last timed step's outputs as .npy
 
 For N > 1 launch under torchrun (one rank per GPU).  Rank 0 prints ONE JSON line.
 A "step" = one env step (constraint + yaw transition + full FLORIS GCH wake solve + measures + reward) for EVERY env of
@@ -29,6 +30,23 @@ LAYOUT = "HornsRev1_"
 ENVS_PER_GPU = 8192          # BASELINE.json configs[4]: 65536 envs over 8 GPUs
 MAX_NUM_STEPS = 500          # simple_env.py:24 default episode length (truncation at step 499)
 L2_FLUSH_BYTES = 256 << 20   # > 126 MB L2
+DUMP_MAX_BYTES = 64 << 20    # --dump-outputs: above this, a fixed seeded sample of env rows is written
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Writes the step outputs (numpy arrays, leading dim = env) as path/<name>.npy, float32 / float64 as computed (the
+    uint8 `truncated` flag as float32).  Over DUMP_MAX_BYTES the same seeded sample of env rows is taken from every
+    array, in env order, and its env indices are written as env_index.npy."""
+    arrays = {k: a if a.dtype in (np.float32, np.float64) else a.astype(np.float32) for k, a in arrays.items()}
+    B = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a.nbytes for a in arrays.values()) // B
+    if row_bytes * B > DUMP_MAX_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_MAX_BYTES // (row_bytes + 8), replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -485,6 +503,8 @@ def run_ours(args):
     barrier()
     t_wall1 = time.time()
     launches = fb.launch_count() - launches0
+    if args.dump_outputs and rank == 0:  # before the legs below overwrite fb.out in place
+        dump_outputs(args.dump_outputs, {k: v.cpu().numpy() for k, v in out.items()})
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = float(sum(step_ms))
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
@@ -705,7 +725,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="headline + e2e only (no relaxed / sustained / other-config legs)")
     ap.add_argument("--sustained-seconds", type=float, default=6.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                    "(rank 0's envs; at most 64 MB, a fixed seeded sample of envs beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours (the reference arm's steps run in worker processes)")
     if args.impl == "reference":
         run_reference(args)
     else:
