@@ -1,6 +1,9 @@
-"""The warp-per-env kernels evaluate the transverse (vortex) velocities either directly from the positions or through the
-per-env vortex table built at reset (wf_vortex_table_kernel; DESIGN.md section 5).  Both routes must reproduce the oracle;
-x-ties (wd = 270 on the row layouts) always take the direct route inside a table-enabled launch."""
+"""The FP64 warp-per-env kernels evaluate the transverse (vortex) velocities either directly from the positions or through
+the per-env vortex table built at reset (wf_vortex_table_kernel; DESIGN.md section 5).  Both routes must reproduce the oracle;
+x-ties (wd = 270 on the row layouts) always take the direct route inside a table-enabled launch.  On an FP64 handle the
+table route is the gather form of the step kernel and the direct route its scatter form.  The FP32 step kernel always
+evaluates directly; on a strict FP32 handle the two routes are those of the FP64 re-solve of the flagged envs, which reads
+source-major double rows."""
 import numpy as np
 import pytest
 
@@ -9,18 +12,13 @@ from tests._util import host_trig, layout, rel_err, sample_winds
 pytestmark = pytest.mark.gpu
 
 
-def _solve(name, precision, B, seed, monkeypatch, table, gather=True):
+def _solve(name, precision, B, seed, monkeypatch, table):
     import torch
 
     from wfcrl_b200.backend import FlorisBatch
 
-    if gather:  # FP64 handle: target-major table + gather kernel (default) or source-major table + scatter kernel
-        monkeypatch.delenv("WFCRL_B200_NO_GATHER", raising=False)
-    else:
-        monkeypatch.setenv("WFCRL_B200_NO_GATHER", "1")
-    if table:  # FP64 handles build the table by default, FP32 handles on request
+    if table:  # FP64 and strict FP32 handles build the table by default
         monkeypatch.delenv("WFCRL_B200_NO_VTAB", raising=False)
-        monkeypatch.setenv("WFCRL_B200_VTAB", "1")
     else:
         monkeypatch.setenv("WFCRL_B200_NO_VTAB", "1")
     lx, ly = layout(name)
@@ -58,15 +56,6 @@ def test_table_and_direct_routes_match_oracle(cuda_device, monkeypatch, name, pr
         assert rel_err(got["load"], loads_ref, 1e4) <= (tol if precision == "f64" else 2e-3)
     # the two routes agree with each other far inside the tolerance
     assert rel_err(tab["power"], direct["power"], 1.0) <= (1e-11 if precision == "f64" else 2e-5)
-
-
-@pytest.mark.parametrize("name", ["Turb32_Row5_", "HornsRev1_"])
-def test_fp64_scatter_form_with_source_major_table_matches_gather_form(cuda_device, monkeypatch, name):
-    """WFCRL_B200_NO_GATHER=1 keeps the scatter form of the FP64 step kernel (source-major rows) alive for A/B runs."""
-    gather, _ = _solve(name, "f64", 24, 33, monkeypatch, table=True)
-    scatter, _ = _solve(name, "f64", 24, 33, monkeypatch, table=True, gather=False)
-    for key in ("power", "wind_speed", "wind_direction", "load"):
-        assert rel_err(scatter[key], gather[key], 1e-6) <= 1e-11, key
 
 
 def test_moving_wind_falls_back_to_direct_route(cuda_device):

@@ -60,7 +60,6 @@ struct WfHandle_t {
     int* h_fix_n = nullptr;
     int fix_rec_cap = 0;
     cudaEvent_t ev_chunk[kHostStreams] = {};
-    bool fast_uses_vtab = false;  // FP32 step kernel reads the vortex table (off by default: measured slower than direct)
     bool vtab_stale = false;  // some env's vortex-table rows do not match its geometry: launch the kernels that ignore the table
     // wf_set_kernel_timing: events around the step-kernel launch and the re-solve launch of the last step call
     bool timing = false, timing_pending = false;
@@ -256,11 +255,11 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
     if ((rc = dev_alloc(h, &s.tab_lo, BT)) || (rc = dev_alloc(h, &s.tab_glo, BT))) return fail(rc);
     // The vortex table trades the V sweep's arithmetic for one streamed read of 36 reals per turbine pair.  Measured on B200
     // (profiles/r2_vortex_table.md): it pays in the FP64 kernels (whose sweep is 3x more expensive), but not in the FP32 kernel,
-    // where the instructions that remain are latency-bound and the direct evaluation wins by 6 % -- so an FP32 handle builds
-    // float rows for its own kernel only when WFCRL_B200_VTAB=1 asks for it.  A strict FP32 handle builds DOUBLE rows for its
-    // FP64 re-solve kernel, which reads those of the few flagged envs (float rows would cost it 1e-9 of the rotor speed, too
-    // much at the foot of the power curve).  WFCRL_B200_NO_VTAB=1 disables every table; tables that would not fit
-    // comfortably are skipped and the kernels evaluate every pair directly.
+    // where the instructions that remain are latency-bound and the direct evaluation wins by 6 % -- so the FP32 step kernel
+    // never reads it.  A strict FP32 handle builds DOUBLE rows for its FP64 re-solve kernel, which reads those of the few
+    // flagged envs (float rows would cost it 1e-9 of the rotor speed, too much at the foot of the power curve).
+    // WFCRL_B200_NO_VTAB=1 disables every table; tables that would not fit comfortably are skipped and the kernels evaluate
+    // every pair directly.
     if (cfg->kernel == WF_KERNEL_FAST && T >= 2 && !getenv("WFCRL_B200_NO_VTAB")) {
         const size_t rows_all = (size_t)B * ((size_t)T * (T - 1) / 2) * 36;
         const size_t cap = (size_t)(getenv("WFCRL_B200_VTAB_MAX_MB") ? atof(getenv("WFCRL_B200_VTAB_MAX_MB")) : 24576.0) << 20;
@@ -273,20 +272,21 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
             h->allocs.push_back(p);
             return p;
         };
-        const bool vtab_in_main = getenv("WFCRL_B200_VTAB") && atoi(getenv("WFCRL_B200_VTAB")) != 0;
         if (cfg->precision == WF_PREC_F64) {
-            s.vtab64 = (double*)try_alloc(rows_all * 8);
-            s.vtab = s.vtab64;
-            // the FP64 step kernel gathers: target-major rows + the (v, w) scratch (WFCRL_B200_NO_GATHER=1: source-major rows
-            // and the scatter form of the kernel, for A/B measurements)
-            if (s.vtab64 && !getenv("WFCRL_B200_NO_GATHER")) s.vwg = (double2*)try_alloc(BT * 9 * sizeof(double2));
-            m.vtab_tmajor = s.vwg != nullptr;
-        } else {
-            if (m.amb_eps > 0.f) s.vtab64 = (double*)try_alloc(rows_all * 8);
-            if (vtab_in_main) s.vtab = try_alloc(rows_all * 4);
-            h->fast_uses_vtab = s.vtab != nullptr;
+            // the FP64 step kernel gathers: target-major rows + the (v, w) scratch, both or neither (then it runs the scatter
+            // form with direct evaluation)
+            s.vtab = (double*)try_alloc(rows_all * 8);
+            if (s.vtab) s.vwg = (double2*)try_alloc(BT * 9 * sizeof(double2));
+            if (s.vtab && !s.vwg) {
+                cudaFree(s.vtab);
+                h->allocs.pop_back();
+                s.vtab = nullptr;
+            }
+            m.vtab_tmajor = s.vtab != nullptr;
+        } else if (m.amb_eps > 0.f) {
+            s.vtab = (double*)try_alloc(rows_all * 8);
         }
-        if (s.vtab || s.vtab64)
+        if (s.vtab)
             if ((rc = dev_alloc(h, &s.vtab_ok, (size_t)B))) return fail(rc);
     }
     if (cudaMallocHost((void**)&h->h_mask, B) != cudaSuccess || cudaMallocHost((void**)&h->h_rws, sizeof(double) * B) != cudaSuccess ||
@@ -377,8 +377,8 @@ static int launch_step(WfHandle h, int mode, const uint8_t* d_mask, const float*
         e = wf_launch_step_fast64(mode, !h->vtab_stale, h->model, h->fast64, h->st, d_mask, d_action, d_yaw, out, env_begin, env_count, st);
     else if (h->cfg.kernel == WF_KERNEL_FAST)
     {
-        e = wf_launch_step_fast(mode, h->fast_baked, h->fast_uses_vtab && !h->vtab_stale, h->model, h->fast, h->st, d_mask, d_action, d_yaw, out, env_begin,
-                                env_count, 0, st);
+        e = wf_launch_step_fast(mode, h->fast_baked, h->model, h->fast, h->st, d_mask, d_action, d_yaw, out, env_begin, env_count, 0,
+                                st);
         if (e == cudaSuccess && is_strict_f32(h) && !defer_fixup) {  // strict FP32: FP64 re-solve of whatever the launch flagged
             if (timed) { cudaEventRecord(h->ev_t[1], st); tail.mid = true; }
             h->launches += 1;
@@ -730,7 +730,7 @@ int wf_device_info(WfHandle h, int32_t* sm_count, int32_t* sm_clock_khz, int32_t
     if (h->cfg.kernel == WF_KERNEL_FAST && h->cfg.precision == WF_PREC_F64) {
         CUDA_TRY(wf_step_fast64_attributes(h->model, h->st, &attr, &ctas, &thr, &sm));
     } else if (h->cfg.kernel == WF_KERNEL_FAST) {
-        CUDA_TRY(wf_step_fast_attributes(h->fast_baked, h->fast_uses_vtab && h->st.vtab && !h->vtab_stale, h->model, &attr, &ctas, &thr, &sm));
+        CUDA_TRY(wf_step_fast_attributes(h->fast_baked, h->model, &attr, &ctas, &thr, &sm));
     } else {
         CUDA_TRY(wf_step_basic_attributes(h->cfg.precision, &attr, &ctas, thr));
         sm = (int)attr.sharedSizeBytes;

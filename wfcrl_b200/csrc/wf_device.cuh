@@ -74,16 +74,15 @@ struct WfState {
     float2* yhl;        // [B][T] (hi, lo) of ys - yc
     uchar4* idx;        // [B][T] .x: first t with X[t]-x_i >= 0 ; .y: first t with X[t] > x_i+0.1 ;
                         //         .z: first t with X[t] > x_i ; .w: first t with X[t] > x_i+15D   (T if none)
-    // Vortex table (warp-per-env kernels): the transverse velocities one source induces on one rotor point are LINEAR in
+    // Vortex table (FP64 warp-per-env kernels): the transverse velocities one source induces on one rotor point are LINEAR in
     // the source's two circulations (tip pair Gt -- the bottom tip vortex is -vel_bot/vel_top times the top one -- and
     // wake rotation Gwr) with coefficients that depend on the geometry only.  Built once per wind direction by
-    // wf_vortex_table_kernel in SORTED order, so that the step kernel streams it front to back:
+    // wf_vortex_table_kernel in SORTED order, so that a kernel streams it front to back:
     //   row(i, t) for sorted source i < target t at index i*T - i*(i+1)/2 + (t - i - 1); a row is [3 columns j][3 heights k]
     //   [cVt, cVw, cWt, cWw]:  V += Gt*cVt + Gwr*cVw ;  W += max(Gt*cWt + Gwr*cWw, 0)            (SURVEY A.7)
-    void* vtab;         // [B][T(T-1)/2][36] rows read by the handle's own step kernel: double (FP64 handle) or float (FP32
-                        //     handle, only with WFCRL_B200_VTAB=1); NULL = that kernel evaluates every pair directly
-    double* vtab64;     // the same rows in double for the FP64 kernels: == vtab on an FP64 handle; on a strict FP32 handle a
-                        //     table of its own, read by the re-solve of the few flagged envs; NULL = disabled
+    double* vtab;       // [B][T(T-1)/2][36] rows, read by the FP64 kernels only: on an FP64 handle target-major (m.vtab_tmajor)
+                        //     for the gather step kernel, on a strict FP32 handle source-major for the re-solve of the few
+                        //     flagged envs; NULL = every pair is evaluated directly
     uint8_t* vtab_ok;   // [B] 1 = the env's rows match its current geometry (cleared by the geometry kernel)
     uint8_t* tab_lo;    // [B][T] per sorted source i: first t with xs[t] - xs[i] > 1e-6 m; closer targets (x-ties) are
                         //         evaluated directly from the positions, never through the table
@@ -92,7 +91,7 @@ struct WfState {
     // FP64 gather kernel (target-major table, m.vtab_tmajor): row(j, t) of source j < target t at index t*(t-1)/2 + j, so
     // that the rows one target sums in its prologue are contiguous; the finished (v, w) of every rotor point and the direct
     // contributions between x-tied turbines live in this scratch (rewritten by every launch; L2-resident while an env runs)
-    double2* vwg;       // [B][9T] or NULL
+    double2* vwg;       // [B][9T]; an FP64 handle has both the table and this scratch, or neither
 };
 
 // Constants of the tuned warp-per-env kernels, precomputed on the host in FP64 (wf_host_const.h: build_fast_const);
@@ -155,12 +154,12 @@ cudaError_t wf_launch_sample_reset(const WfModel& m, const WfState& s, const uin
 cudaError_t wf_launch_reset_state(const WfModel& m, const WfState& s, const uint8_t* d_mask, const double* d_ws,
                                   const double* d_wd, cudaStream_t stream);
 cudaError_t wf_step_basic_attributes(int precision, cudaFuncAttributes* attr, int* ctas_per_sm, int threads);
-cudaError_t wf_launch_step_fast(int mode, bool baked, bool use_vtab, const WfModel& m, const WfFastConst& fc, const WfState& s,
+cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                 const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
                                 const WfOutPtrs& out, int env_begin, int env_count, int slot, cudaStream_t stream);
 cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                               const WfOutPtrs& out, int env_count, int slot, float* d_rec, int rec_cap, cudaStream_t stream);
-cudaError_t wf_step_fast_attributes(bool baked, bool use_vtab, const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
+cudaError_t wf_step_fast_attributes(bool baked, const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                     int* smem);
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,

@@ -10,7 +10,8 @@
 //         scalar chain (Ct, induction, secondary steering, deflection / velocity-model scalars, yaw-added recovery)
 //         evaluated redundantly by every lane -- no broadcast needed;
 //      2. V sweep over ALL downstream targets, 10 turbines x 3 lateral grid columns per pass (30 of 32 lanes), each lane
-//         doing the 3 vertical points of its column: the three vortex pairs (real + ground mirror) and the (v, w)
+//         doing the 3 vertical points of its column: the three vortex pairs (real + ground mirror), evaluated directly
+//         (the FP64 kernels' per-pair vortex table measured slower here: DESIGN.md section 5), and the (v, w)
 //         update; the same pass ballots a compacted queue of the targets that can see the velocity deficit;
 //         a source at exactly zero yaw sheds no tip vortices and runs an instantiation with the wake-rotation pair only;
 //      3. D sweep over the queue only: deflection, wake widths, Gaussian deficit, sum-of-squares update, overlap count
@@ -30,8 +31,6 @@
 #include "wf_device.cuh"
 #include "wf_reset_device.cuh"
 #include "wf_fast_baked.inc"
-
-#include <stdlib.h>
 
 namespace {
 
@@ -56,13 +55,6 @@ constexpr int kMaxEvt = 8;  // ambiguous-decision records kept per env; more tha
 #define WF_FAST_UNROLL_D 1
 #endif
 #define WF_UNROLL_D WF_PRAGMA_UNROLL_(WF_FAST_UNROLL_D)
-#ifndef WF_VTAB_PF_DIST
-#define WF_VTAB_PF_DIST 1  // (1 measured best: 2 -> +7 %, 4 -> +20 % step time, L2 capacity) the table rows of source i + WF_VTAB_PF_DIST are prefetched to L2 while source i is processed
-#endif
-#ifndef WF_FAST_UNROLL_T
-#define WF_FAST_UNROLL_T 2  // table passes in flight
-#endif
-#define WF_UNROLL_T WF_PRAGMA_UNROLL_(WF_FAST_UNROLL_T)
 #ifndef WF_FAST_MINB
 #define WF_FAST_MINB 12  // lower bound on resident env-CTAs per SM for the register allocator (16 are reached)
 #endif
@@ -72,29 +64,6 @@ __device__ __forceinline__ float fsqrt(float x) { float y; asm("sqrt.approx.ftz.
 __device__ __forceinline__ float fex2(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float flg2(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float fclamp(float x, float lo, float hi) { return fminf(fmaxf(x, lo), hi); }
-
-// Pull the vortex-table rows of sorted source `i` (contiguous: targets i+1 .. T-1) into L2 ahead of their use with ONE bulk
-// prefetch; the rows are read exactly once per step, so without this every pass of the V sweep would wait for HBM.
-template <int ROW_BYTES>
-__device__ __forceinline__ void prefetch_rows(const void* env_rows, int i, int T, int lane) {
-    if (i >= T - 1 || lane != 0) return;
-    const char* p = (const char*)env_rows + ((size_t)i * T - (size_t)i * (i + 1) / 2) * ROW_BYTES;
-    const unsigned bytes = (unsigned)(T - 1 - i) * ROW_BYTES;  // a multiple of 16, p is 16-byte aligned
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-
-// Table rows are read exactly once per step: fetch them with an evict-first L2 policy so that consumed lines make room for
-// the rows being prefetched instead of ageing through the LRU.
-__device__ __forceinline__ float4 ldg_stream(const float4* p, unsigned long long pol) {
-    float4 v;
-#ifndef WF_VTAB_EVICT_HINT  // the hint measured 3-9 % slower on B200 (profiles/r2_vortex_table.md)
-    v = __ldg(p);
-#else
-    asm volatile("ld.global.nc.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;"
-                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
-#endif
-    return v;
-}
 
 // piecewise-linear table lookup (np.interp + scipy fill values), warp-uniform or per-lane x
 __device__ __forceinline__ float interp_f(const WfFastConst& fc, const float* __restrict__ fp, float x, float left,
@@ -167,8 +136,8 @@ __device__ __forceinline__ SmemView carve(unsigned char* base, int T) {
 struct wf_true_tag { static constexpr bool value = true; };
 struct wf_false_tag { static constexpr bool value = false; };
 
-template <bool BAKED, bool VTAB>
-__global__ void __launch_bounds__(32, (VTAB || BAKED) ? 16 : WF_FAST_MINB)
+template <bool BAKED>
+__global__ void __launch_bounds__(32, BAKED ? 16 : WF_FAST_MINB)
 wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const WfModel m, const __grid_constant__ WfFastConst fc,
                     const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
                     const double* __restrict__ yaw_cmd, const WfOutPtrs out) {
@@ -256,19 +225,9 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
     const double two_D_d = 2.0 * m.D;
     int nevt = 0;
     bool flagged = false;
-    // vortex table of this env (streamed front to back, one row per sorted pair i < t), or NULL: evaluate every pair directly
-    const float4* __restrict__ vrow = nullptr;
-    if (VTAB && s.vtab && s.vtab_ok[b]) vrow = (const float4*)s.vtab + (size_t)b * ((size_t)T * (T - 1) / 2) * 9;
-    unsigned long long pol_stream = 0;
-    if (VTAB) asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_stream));
-    if (VTAB && vrow) {
-#pragma unroll
-        for (int d = 0; d < WF_VTAB_PF_DIST; ++d) prefetch_rows<144>(vrow, d, T, lane);
-    }
 
     // ---- sequential solver over sources (SURVEY A.4-A.8) -------------------------------------------------------------
     for (int i = 0; i < T; ++i) {
-        if (VTAB && vrow) prefetch_rows<144>(vrow, i + WF_VTAB_PF_DIST, T, lane);
         // ===== source prologue =====
         // rotor sums over the source's 9 points: one point per lane, butterfly over 16-lane halves -> uniform values
         float su3, sv, sw, vq, wwq;
@@ -386,13 +345,10 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
         // A source at exactly zero yaw sheds no tip vortices (Gt = Gb = 0): the sweep then evaluates the wake-rotation
         // pair only -- same bits, 45 % of the work.  Warp-uniform choice, one instantiation of the loop per case.
         int qn = 0;
-        // with the table only the x-ties of the source (targets within 1e-6 m in x; none for a generic wind direction) take
-        // the direct path
-        const int t_hi = vrow ? (int)s.tab_lo[row + i] : T;
         auto v_pass = [&](auto yawed_tag, const int t0) {
             constexpr bool YAWED = decltype(yawed_tag)::value;
             const int tr = t0 + g;
-            const bool active = lane_ok && tr < t_hi && tr != i;
+            const bool active = lane_ok && tr < T && tr != i;
             const int t = min(tr, T - 1);  // inactive lanes compute on a valid turbine; only their stores are masked
             const float2 xt = sm.xhl[t], yt = sm.yhl[t];
             const float dx = (xt.x - xi.x) + (xt.y - xi.y);
@@ -451,47 +407,12 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
                 }
             }
         };
-        if (VTAB) {  // only x-ties come here (lo == i and t_hi == i + 1 without ties): one rolled, generic copy of the pass
-            if (t_hi - lo > 1) {
-#pragma unroll 1
-                for (int t0 = lo; t0 < t_hi; t0 += kTurbPerPass) v_pass(wf_true_tag{}, t0);
-            }
-        } else if (sy != 0.f) {
+        if (sy != 0.f) {
             WF_UNROLL_V
-            for (int t0 = lo; t0 < t_hi; t0 += kTurbPerPass) v_pass(wf_true_tag{}, t0);
+            for (int t0 = lo; t0 < T; t0 += kTurbPerPass) v_pass(wf_true_tag{}, t0);
         } else {
             WF_UNROLL_V
-            for (int t0 = lo; t0 < t_hi; t0 += kTurbPerPass) v_pass(wf_false_tag{}, t0);
-        }
-        if (VTAB && vrow) {
-            // ===== V sweep through the table: V += Gt*cVt + Gwr*cVw ; W += max(Gt*cWt + Gwr*cWw, 0) per rotor point; a lane
-            //       reads the 48 contiguous bytes of its (target, column): a pass is one 1440-byte segment of the stream =====
-            const float4* __restrict__ src = vrow + ((size_t)i * T - (size_t)i * (i + 1) / 2) * 9 + 3 * j;
-            WF_UNROLL_T
-            for (int t0 = t_hi; t0 < T; t0 += kTurbPerPass) {
-                const int tr = t0 + g;
-                const bool active = lane_ok && tr < T;
-                const int t = min(tr, T - 1);
-                const float4* __restrict__ rp = src + (size_t)(t - i - 1) * 9;
-                const float4 c0 = ldg_stream(rp, pol_stream), c1 = ldg_stream(rp + 1, pol_stream), c2 = ldg_stream(rp + 2, pol_stream);
-                const float2 xt = sm.xhl[t], yt = sm.yhl[t];
-                const float dx = (xt.x - xi.x) + (xt.y - xi.y);
-                const float dyc = ((yt.x - yi.x) + (yt.y - yi.y)) + offj;
-                const bool need = active && (t >= near_i) &&
-                                  (fabsf(dyc) < fmaf(reach1, dx, reach0) + fabsf(fmaf(KC(bd), dx, KC(ad))));
-                const unsigned nb = __ballot_sync(0xffffffffu, need);
-                const bool leader = (j == 0) && active && (((nb >> (3 * g)) & 7u) != 0u);
-                const unsigned lb = __ballot_sync(0xffffffffu, leader);
-                if (leader) sm.queue[qn + __popc(lb & ((1u << lane) - 1u))] = (unsigned char)t;
-                qn += __popc(lb);
-                if (active) {
-                    const int qb = 9 * t + 3 * j;
-                    const float2 o0 = sm.vw[qb], o1 = sm.vw[qb + 1], o2 = sm.vw[qb + 2];
-                    sm.vw[qb] = make_float2(o0.x + fmaf(Gt, c0.x, Gwr * c0.y), o0.y + fmaxf(fmaf(Gt, c0.z, Gwr * c0.w), 0.f));
-                    sm.vw[qb + 1] = make_float2(o1.x + fmaf(Gt, c1.x, Gwr * c1.y), o1.y + fmaxf(fmaf(Gt, c1.z, Gwr * c1.w), 0.f));
-                    sm.vw[qb + 2] = make_float2(o2.x + fmaf(Gt, c2.x, Gwr * c2.y), o2.y + fmaxf(fmaf(Gt, c2.z, Gwr * c2.w), 0.f));
-                }
-            }
+            for (int t0 = lo; t0 < T; t0 += kTurbPerPass) v_pass(wf_false_tag{}, t0);
         }
         __syncwarp();
 
@@ -694,7 +615,7 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
 
 }  // namespace
 
-template <bool BAKED, bool VTAB>
+template <bool BAKED>
 static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                  const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
                                  const WfOutPtrs& out, int env_begin, int env_count, int slot, cudaStream_t stream) {
@@ -703,43 +624,37 @@ static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& 
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED, VTAB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED, VTAB>, cudaFuncAttributePreferredSharedMemoryCarveout,
+        e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                  cudaSharedmemCarveoutMaxShared);
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) configured[dev] = true;
     }
-    static const size_t pad = getenv("WFCRL_SMEM_PAD") ? (size_t)atoi(getenv("WFCRL_SMEM_PAD")) : 0;  // tuning experiments
-    wf_step_fast_kernel<BAKED, VTAB><<<env_count, 32, smem + pad, stream>>>(mode, env_begin, slot, m, fc, s, d_mask, d_action, d_yaw_cmd, out);
+    wf_step_fast_kernel<BAKED><<<env_count, 32, smem, stream>>>(mode, env_begin, slot, m, fc, s, d_mask, d_action, d_yaw_cmd, out);
     return cudaGetLastError();
 }
 
-cudaError_t wf_launch_step_fast(int mode, bool baked, bool use_vtab, const WfModel& m, const WfFastConst& fc, const WfState& s,
+cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                 const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
                                 const WfOutPtrs& out, int env_begin, int env_count, int slot, cudaStream_t stream) {
-#define WF_GO(B_, V_) launch_fast_t<B_, V_>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, slot, stream)
-    const bool vtab = use_vtab && s.vtab != nullptr;
-    return baked ? (vtab ? WF_GO(true, true) : WF_GO(true, false)) : (vtab ? WF_GO(false, true) : WF_GO(false, false));
-#undef WF_GO
+    return baked ? launch_fast_t<true>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, slot, stream)
+                 : launch_fast_t<false>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, slot, stream);
 }
 
-template <bool BAKED, bool VTAB>
+template <bool BAKED>
 static cudaError_t attrs_fast_t(const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads, int* smem) {
     *threads = 32;
     *smem = (int)fast_smem_bytes(m.T);
-    cudaError_t e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED, VTAB>, cudaFuncAttributePreferredSharedMemoryCarveout,
+    cudaError_t e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                          cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return e;
-    e = cudaFuncGetAttributes(attr, wf_step_fast_kernel<BAKED, VTAB>);
+    e = cudaFuncGetAttributes(attr, wf_step_fast_kernel<BAKED>);
     if (e != cudaSuccess) return e;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, wf_step_fast_kernel<BAKED, VTAB>, 32, *smem);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, wf_step_fast_kernel<BAKED>, 32, *smem);
 }
 
-cudaError_t wf_step_fast_attributes(bool baked, bool use_vtab, const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm,
-                                    int* threads, int* smem) {
-    if (use_vtab) return baked ? attrs_fast_t<true, true>(m, attr, ctas_per_sm, threads, smem)
-                               : attrs_fast_t<false, true>(m, attr, ctas_per_sm, threads, smem);
-    return baked ? attrs_fast_t<true, false>(m, attr, ctas_per_sm, threads, smem)
-                 : attrs_fast_t<false, false>(m, attr, ctas_per_sm, threads, smem);
+cudaError_t wf_step_fast_attributes(bool baked, const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
+                                    int* smem) {
+    return baked ? attrs_fast_t<true>(m, attr, ctas_per_sm, threads, smem) : attrs_fast_t<false>(m, attr, ctas_per_sm, threads, smem);
 }

@@ -219,7 +219,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     auto vw_st = [&](const int q, const double2 v) { if (GATHER) __stcg(vwp + q, v); else vwp[q] = v; };
     // vortex table of this env (wf_device.cuh), or NULL: evaluate every pair directly
     const double* __restrict__ vrow = nullptr;
-    if (use_vtab && s.vtab64 && s.vtab_ok[b] && (GATHER || !m.vtab_tmajor)) vrow = s.vtab64 + (size_t)b * ((size_t)T * (T - 1) / 2) * 36;
+    if (use_vtab && s.vtab && s.vtab_ok[b] && (GATHER || !m.vtab_tmajor)) vrow = s.vtab + (size_t)b * ((size_t)T * (T - 1) / 2) * 36;
 
     // ---- env prologue on the ORIGINAL turbine order (mdp.py:291-319, simple_env.py:64-72) -------------------------
     int nm = 0;
@@ -962,7 +962,7 @@ cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const W
     }
 }
 
-static bool fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab64 && s.vwg && s.tab_glo; }
+static bool fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
 template <typename K> static cudaError_t configure_fast64(K kernel) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
     if (e != cudaSuccess) return e;
@@ -972,13 +972,9 @@ template <typename K> static cudaError_t configure_fast64(K kernel) {
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
                                   const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
-    // a target-major table (and its scratch) belongs to the gather kernel; the scatter kernel reads a source-major one or
-    // evaluates every pair directly
+    // a target-major table (and its scratch) belongs to the gather kernel; the scatter kernel evaluates every pair directly
     const bool gather = fast64_gathers(m, s) && use_vtab;
-    size_t smem = fast64_smem_bytes(m.T, gather);
-#ifdef WF_EXP_SMEM_PAD
-    if (const char* e = getenv("WFCRL_B200_F64_SMEM_PAD")) smem += (size_t)atoi(e);
-#endif
+    const size_t smem = fast64_smem_bytes(m.T, gather);
     static bool configured[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
@@ -1000,9 +996,6 @@ cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFu
     *threads = 32;
     const bool gather = fast64_gathers(m, s);
     *smem = (int)fast64_smem_bytes(m.T, gather);
-#ifdef WF_EXP_SMEM_PAD
-    if (const char* e = getenv("WFCRL_B200_F64_SMEM_PAD")) *smem += atoi(e);
-#endif
     cudaError_t e = gather ? configure_fast64(wf_step_fast64_kernel<true>) : configure_fast64(wf_step_fast64_kernel<false>);
     if (e != cudaSuccess) return e;
     e = gather ? cudaFuncGetAttributes(attr, wf_step_fast64_kernel<true>) : cudaFuncGetAttributes(attr, wf_step_fast64_kernel<false>);

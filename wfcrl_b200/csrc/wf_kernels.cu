@@ -269,7 +269,7 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
 
 // ---------------------------------------------------------------------------------------------------------------
 // vortex table: geometry-only coefficients of the transverse velocities (SURVEY A.7), one row per sorted pair i < t.
-// Evaluated in FP64 with the accurate math functions whatever the handle's precision; stored as R.
+// Evaluated in FP64 with the accurate math functions whatever the handle's precision; stored in double.
 // One CTA per env; a thread owns one (row, lateral column) and writes its 12 coefficients [k][cVt, cVw, cWt, cWw].
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
@@ -290,8 +290,7 @@ wf_vortex_table_kernel(const WfModel m, const __grid_constant__ WfFastConst64 fc
     }
     __syncthreads();
     const int rows = T * (T - 1) / 2;
-    double* __restrict__ tab64 = s.vtab64 ? s.vtab64 + (size_t)b * rows * 36 : nullptr;
-    float* __restrict__ tab32 = (s.vtab && (void*)s.vtab != (void*)s.vtab64) ? (float*)s.vtab + (size_t)b * rows * 36 : nullptr;
+    double* __restrict__ tab = s.vtab + (size_t)b * rows * 36;
     const double rho = fc.c_bot / fc.c_top;  // Gb = -rho * Gt
     const double c_dec = fc.eps2 * fc.inv_2pi;
     for (int task = threadIdx.x; task < rows * 3; task += blockDim.x) {
@@ -323,10 +322,7 @@ wf_vortex_table_kernel(const WfModel m, const __grid_constant__ WfFastConst64 fc
             const double dec = c_dec / (fc.nu4[k] * dx + fc.eps2);
             const double c4[4] = {dec * (A[0] - rho * A[1]), dec * A[2], -yL * dec * (Bc[0] - rho * Bc[1]), -yL * dec * Bc[2]};
 #pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                if (tab64) tab64[dst + 4 * k + e] = c4[e];
-                if (tab32) tab32[dst + 4 * k + e] = (float)c4[e];
-            }
+            for (int e = 0; e < 4; ++e) tab[dst + 4 * k + e] = c4[e];
         }
     }
     __syncthreads();
@@ -807,7 +803,7 @@ cudaError_t wf_launch_geometry(const WfModel& m, const WfState& s, const uint8_t
 
 cudaError_t wf_launch_vortex_table(const WfModel& m, const WfFastConst64& fc, const WfState& s, const uint8_t* d_mask,
                                    cudaStream_t stream) {
-    if ((!s.vtab && !s.vtab64) || m.T < 2) return cudaSuccess;
+    if (!s.vtab || m.T < 2) return cudaSuccess;
     wf_vortex_table_kernel<<<m.B, 256, 0, stream>>>(m, fc, s, d_mask);
     return cudaGetLastError();
 }
