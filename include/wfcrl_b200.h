@@ -111,11 +111,36 @@ int wf_default_config(WfConfig* cfg);
 
 /*
  * Replaces FlorisInterface.from_case / __init__ (interface.py:462-501, 526-547) and WindFarmMDP.__init__'s
- * accumulators (mdp.py:157-160) for `num_envs` envs sharing one layout.  layout_x/y: HOST, [T] metres.
+ * accumulators (mdp.py:157-160) for `num_envs` envs.  layout_x/y: HOST, [T] metres: the handle's layout pool holds this
+ * one layout and every env has layout id 0 (wf_set_layouts / wf_assign_layouts give envs different farms).
  * All envs start with wind (8 m/s, 270 deg) (data_cases.py:99-100), zero yaw, zero counters.
  */
 int wf_create(const WfConfig* cfg, const double* h_layout_x, const double* h_layout_y, WfHandle* out);
 int wf_destroy(WfHandle h);
+
+/*
+ * Layout pool: a handle holds n_layouts >= 1 farm layouts of its num_turbines turbines, and each env builds its geometry
+ * from one of them, its "layout id" (state array "layout_id").  Each layout is rotated about the centre of its own bounding
+ * box, (min + max) / 2 per axis, as a single-layout handle does; an env's results equal those of a handle created with
+ * its layout alone.
+ * wf_set_layouts replaces the pool: h_x, h_y HOST double [n_layouts][T] metres (finite).  Every env gets layout id 0 and
+ * the geometry of all envs is rebuilt with their current wind; counters and yaw are kept (as in wf_update_wind).
+ * Synchronous: it waits for every earlier asynchronous call on the handle.
+ */
+int wf_set_layouts(WfHandle h, int32_t n_layouts, const double* h_x, const double* h_y);
+/*
+ * Sets the layout ids of the listed envs and rebuilds their geometry.  h_env_ids: HOST int32 [n] or NULL with
+ * n == num_envs meaning "all envs in order"; h_layout_ids: HOST int32 [n] in [0, n_layouts).  Out-of-range env or layout
+ * ids are rejected before anything changes.  Synchronous (the stream is synchronised before returning).
+ */
+int wf_assign_layouts(WfHandle h, const int32_t* h_env_ids, int32_t n, const int32_t* h_layout_ids, void* stream);
+/*
+ * While enabled, every library-sampled reset (wf_reset_sampled and the in-kernel auto-reset) also draws the env's layout
+ * id uniformly from the pool: id = floor(u53(r.x, r.y) * n_layouts) with r = Philox4x32-10 of counter (global env id lo,
+ * hi, episode index, 2) under key = seed, the same key and counter as that reset's wind draw (which uses draw words 0 and 1),
+ * so the winds and TI of every reset are the same with sampling on or off.  Disabled at creation.
+ */
+int wf_set_layout_sampling(WfHandle h, int32_t enabled);
 
 /*
  * Replaces WindFarmMDP.reset -> FlorisInterface.init + (start_iter+1) x update_command() (mdp.py:260-270,
@@ -143,7 +168,9 @@ int wf_reset_masked(WfHandle h, const uint8_t* d_mask, const double* d_ws, const
  * of env b): an env's winds depend on its GLOBAL id and on how many sampled resets it has had ("episode" state array),
  * never on how the envs are sharded over handles / GPUs.  ws by Weibull inversion, wd by Box-Muller.  When
  * ti_hi > ti_lo the ambient turbulence intensity of the selected envs is drawn U(ti_lo, ti_hi) as well (extension; the
- * reference fixes 0.06, case.yaml:33); pass ti_lo = ti_hi = 0 to leave it alone.  d_mask NULL = all envs.  Asynchronous.
+ * reference fixes 0.06, case.yaml:33); pass ti_lo = ti_hi = 0 to leave it alone.  With wf_set_layout_sampling on, the
+ * layout id of each selected env is drawn too, and its geometry is built from that layout; otherwise each env keeps its
+ * layout.  d_mask NULL = all envs.  Asynchronous.
  */
 int wf_reset_sampled(WfHandle h, const uint8_t* d_mask, uint64_t seed, int64_t env_id_offset, double ti_lo, double ti_hi,
                      int32_t warmup_solves, const WfStepOut* out, void* stream);
@@ -163,7 +190,8 @@ int wf_step(WfHandle h, const float* d_action, const WfStepOut* out, void* strea
  * In-kernel auto-reset: the batched counterpart of "env.reset() as soon as the episode truncates" (mdp.py:260-262 behind
  * simple_env.py:49-56) without a reset launch chain of its own.  Once armed, a wf_step whose env reaches
  * _num_iter == max_iter ALSO starts that env's next episode inside the step kernel: the wind is drawn as by
- * wf_reset_sampled (key = seed, counter = (env_id_offset + b, episode index)), yaw / accumulators / counters / shaper state
+ * wf_reset_sampled (key = seed, counter = (env_id_offset + b, episode index)), as is its layout id when
+ * wf_set_layout_sampling is on (otherwise the env keeps its layout), yaw / accumulators / counters / shaper state
  * are zeroed, and the env is marked.  The outputs of that wf_step still hold the FINAL observation of the finished episode.
  * wf_autoreset_finish then rebuilds the geometry of the marked envs, runs their warm-up solve(s) -- overwriting their rows
  * of `out` with the start observation -- and clears the marks; with no env marked its launches exit at once, so it may be
@@ -220,7 +248,9 @@ int wf_set_turbulence_intensity(WfHandle h, const double* d_ti, void* stream);
  *   episode bookkeeping kept by the env-mode step kernels: "ep_return" f64[B], "ep_len" i32[B] (running episode) and, over the
  *   episodes the env has finished, "fin_sum" f64[B], "fin_sumsq" f64[B], "fin_n" i32[B], "fin_len" i64[B] |
  *   "ws" f64[B] | "wd" f64[B] | "ws_norm" f64[B] | "shaper_ref" f64[B] | "ti_ambient" f64[B] |
- *   "order" i32[B][T] | "xs" f64[B][T] | "ys" f64[B][T] | "xi" f64[B][T] | "yi" f64[B][T] | "cs" f64[B][2]
+ *   "order" i32[B][T] | "xs" f64[B][T] | "ys" f64[B][T] | "xi" f64[B][T] | "yi" f64[B][T] | "cs" f64[B][2] |
+ *   "layout_id" i32[B] (row of the layout pool each env uses; read-only here: wf_set_state refuses it, wf_assign_layouts
+ *   sets it)
  * `bytes` must equal the full array size.
  */
 int wf_get_state(WfHandle h, const char* name, void* h_dst, size_t bytes);

@@ -25,7 +25,7 @@ _STATE_DTYPES = {
     "fin_n": (np.int32, "B"), "fin_len": (np.int64, "B"), "ws": (np.float64, "B"), "wd": (np.float64, "B"),
     "ws_norm": (np.float64, "B"), "shaper_ref": (np.float64, "B"), "ti_ambient": (np.float64, "B"),
     "order": (np.int32, "BT"), "xs": (np.float64, "BT"), "ys": (np.float64, "BT"), "xi": (np.float64, "BT"),
-    "yi": (np.float64, "BT"), "cs": (np.float64, "B2"),
+    "yi": (np.float64, "BT"), "cs": (np.float64, "B2"), "layout_id": (np.int32, "B"),
 }
 
 
@@ -40,7 +40,8 @@ def _ptr(t: Optional[torch.Tensor]):
 
 
 class FlorisBatch:
-    """``num_envs`` independent Floris-backed wind-farm envs sharing one layout, resident on one GPU."""
+    """``num_envs`` independent Floris-backed wind-farm envs resident on one GPU.  They share the layout given here
+    unless ``set_layouts`` gives the handle a pool of layouts of the same turbine count to assign per env."""
 
     def __init__(self, layout_x: Sequence[float], layout_y: Sequence[float], num_envs: int, *, device: int = 0,
                  precision: str = "f64", kernel: str = "basic", max_iter: int = 500,
@@ -109,6 +110,30 @@ class FlorisBatch:
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     # ------------------------------------------------------------------------------------------------------
+    def set_layouts(self, xs, ys) -> None:
+        """Replace the layout pool by ``xs``, ``ys`` [L, T] (metres).  Every env gets layout 0 and its geometry is rebuilt
+        with its current wind; counters and yaw are kept.  Waits for all queued work of the handle."""
+        x = np.ascontiguousarray(xs, dtype=np.float64)
+        y = np.ascontiguousarray(ys, dtype=np.float64)
+        if x.ndim != 2 or x.shape != y.shape or x.shape[1] != self.T:
+            raise ValueError(f"layout pool must be two [L, {self.T}] arrays, got {x.shape} and {y.shape}")
+        _lib.check(self.lib.wf_set_layouts(self.handle, x.shape[0], x.ctypes.data_as(C.c_void_p),
+                                           y.ctypes.data_as(C.c_void_p)))
+
+    def assign_layouts(self, env_ids, layout_ids) -> None:
+        """Give the envs ``env_ids`` (None = all) the pool layouts ``layout_ids`` (scalar or per env) and rebuild their
+        geometry with their current wind."""
+        ids = None if env_ids is None else np.ascontiguousarray(env_ids, dtype=np.int32).reshape(-1)
+        n = self.B if ids is None else ids.shape[0]
+        lids = np.ascontiguousarray(np.broadcast_to(np.asarray(layout_ids, dtype=np.int32), (n,)))
+        _lib.check(self.lib.wf_assign_layouts(self.handle, None if ids is None else ids.ctypes.data_as(C.c_void_p), n,
+                                              lids.ctypes.data_as(C.c_void_p), self._stream()))
+
+    def set_layout_sampling(self, enabled: bool) -> None:
+        """While enabled, ``reset_sampled`` and the in-kernel auto-reset also draw each reset env's layout id uniformly
+        from the pool, with the same counter-based generator as its wind (draw word 2)."""
+        _lib.check(self.lib.wf_set_layout_sampling(self.handle, int(bool(enabled))))
+
     def reset(self, wind_speed, wind_direction, env_ids=None, *, host_trig: bool = True, warmup_solves: int = 1):
         """WindFarmMDP.reset for the selected envs (mdp.py:260-270).  ``host_trig=True`` ships numpy's FP64 cosd/sind of
         the wind deviation so the rotated geometry is bit-identical to a host (numpy) reference (SURVEY 7.3)."""
@@ -260,14 +285,17 @@ class FlorisBatch:
                    "ti_ambient", "ep_return", "ep_len", "fin_sum", "fin_sumsq", "fin_n", "fin_len")
 
     def state_dict(self) -> Dict[str, np.ndarray]:
-        """Host copy of everything needed to resume the batch exactly where it is (geometry is rebuilt from wd)."""
+        """Host copy of everything needed to resume the batch exactly where it is (geometry is rebuilt from wd and the
+        layout ids; the layout pool itself is configuration and is not saved)."""
         sd = {name: self.get_state(name) for name in self._CHECKPOINT}
         sd["cs"] = self.get_state("cs")
+        sd["layout_id"] = self.get_state("layout_id")
         return sd
 
     def load_state_dict(self, sd: Dict[str, np.ndarray]) -> None:
-        """Restore a ``state_dict``: wind first (rebuilds the rotated/sorted geometry with the saved cos/sin so the
-        geometry is bit-identical), then counters, yaw and accumulators."""
+        """Restore a ``state_dict``: layout ids (0 for a dict saved without them), then wind (rebuilds the rotated/sorted
+        geometry with the saved cos/sin so the geometry is bit-identical), then counters, yaw and accumulators."""
+        self.assign_layouts(None, sd.get("layout_id", 0))
         ws = torch.as_tensor(np.ascontiguousarray(sd["ws"]), device=self.device)
         wd = torch.as_tensor(np.ascontiguousarray(sd["wd"]), device=self.device)
         cs = torch.as_tensor(np.ascontiguousarray(sd["cs"]), device=self.device)

@@ -67,6 +67,7 @@ struct WfHandle_t {
     double t_step_ms = 0.0, t_fix_ms = 0.0;
     int t_calls = 0;
     uint64_t steps_since_wind_update = 1u << 30;  // wf_update_wind rebuilds the vortex table only when it is not called every step
+    double* d_pool = nullptr;  // the layout pool in one allocation: [L][T] x, [L][T] y, [L][2] centres (WfModel.layout_*)
 };
 
 template <typename T> static int dev_alloc(WfHandle_t* h, T** p, size_t n) {
@@ -107,6 +108,50 @@ static cudaError_t launch_geometry(WfHandle h, const uint8_t* d_mask, const doub
     return e;
 }
 
+static int check_layouts(size_t n, const double* lx, const double* ly) {
+    for (size_t k = 0; k < n; ++k)
+        if (!isfinite(lx[k]) || !isfinite(ly[k])) return set_err(WF_ERR_INVALID, "layout coordinates must be finite");
+    return WF_OK;
+}
+
+// Replace the layout pool by L validated host layouts [L][T] and store the centre of each one's bounding box, the point the
+// geometry kernel rotates it about.  The caller makes sure that no queued kernel still reads the old pool.
+static int set_pool(WfHandle h, int L, const double* lx, const double* ly) {
+    const size_t T = h->model.T, LT = (size_t)L * T;
+    std::vector<double> pool(LT * 2 + (size_t)L * 2);
+    memcpy(pool.data(), lx, sizeof(double) * LT);
+    memcpy(pool.data() + LT, ly, sizeof(double) * LT);
+    for (int l = 0; l < L; ++l) {
+        const double *x = lx + l * T, *y = ly + l * T;
+        double xmin = x[0], xmax = x[0], ymin = y[0], ymax = y[0];
+        for (size_t t = 1; t < T; ++t) {
+            xmin = fmin(xmin, x[t]); xmax = fmax(xmax, x[t]);
+            ymin = fmin(ymin, y[t]); ymax = fmax(ymax, y[t]);
+        }
+        pool[2 * LT + 2 * l] = (xmin + xmax) / 2;
+        pool[2 * LT + 2 * l + 1] = (ymin + ymax) / 2;
+    }
+    double* d = nullptr;
+    cudaError_t e = cudaMalloc(&d, sizeof(double) * pool.size());
+    if (e != cudaSuccess) return set_err(WF_ERR_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    e = cudaMemcpy(d, pool.data(), sizeof(double) * pool.size(), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) {
+        cudaFree(d);
+        return set_err(WF_ERR_CUDA, std::string("cudaMemcpy: ") + cudaGetErrorString(e));
+    }
+    if (h->d_pool) cudaFree(h->d_pool);
+    h->d_pool = d;
+    WfModel& m = h->model;
+    m.layout_x = d; m.layout_y = d + LT; m.layout_c = d + 2 * LT; m.n_layouts = L;
+    return WF_OK;
+}
+
+// Rebuild the geometry (and table rows) of the masked envs from their current layout ids, rotated by the cos/sin each env
+// already uses, so that host-computed cos/sin (wf_reset with h_cos / h_sin) are kept.
+static cudaError_t rebuild_geometry(WfHandle h, const uint8_t* d_mask, cudaStream_t st) {
+    cudaError_t e = cudaMemcpyAsync(h->d_rcs, h->st.cs, sizeof(double) * 2 * h->model.B, cudaMemcpyDeviceToDevice, st);
+    return e != cudaSuccess ? e : launch_geometry(h, d_mask, h->d_rcs, st);
+}
 
 extern "C" {
 
@@ -128,6 +173,7 @@ int wf_destroy(WfHandle h) {
     if (!h) return WF_OK;
     cudaSetDevice(h->device);
     for (void* p : h->allocs) cudaFree(p);
+    if (h->d_pool) cudaFree(h->d_pool);
     if (h->h_mask) cudaFreeHost(h->h_mask);
     if (h->h_rws) cudaFreeHost(h->h_rws);
     if (h->h_rwd) cudaFreeHost(h->h_rwd);
@@ -167,8 +213,7 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
         if (!isfinite(cfg->table_ws[i]) || !isfinite(cfg->table_cp[i]) || !isfinite(cfg->table_ct[i]) ||
             (i > 0 && !(cfg->table_ws[i] > cfg->table_ws[i - 1])))
             return set_err(WF_ERR_INVALID, "turbine table: wind speeds must be finite and strictly increasing");
-    for (int t = 0; t < T; ++t)
-        if (!isfinite(lx[t]) || !isfinite(ly[t])) return set_err(WF_ERR_INVALID, "layout coordinates must be finite");
+    TRY(check_layouts(T, lx, ly));
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0)
@@ -203,24 +248,17 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
     m.dm = cfg->dm;
     m.ch_const = cfg->ch_constant; m.ch_ai = cfg->ch_ai; m.ch_init = cfg->ch_initial; m.ch_down = cfg->ch_downstream;
     m.e3_112 = 3 * exp(1.0 / 12.0); m.e3_13 = 3 * exp(1.0 / 3.0);
-    double xmin = lx[0], xmax = lx[0], ymin = ly[0], ymax = ly[0];
-    for (int t = 1; t < T; ++t) {
-        xmin = fmin(xmin, lx[t]); xmax = fmax(xmax, lx[t]);
-        ymin = fmin(ymin, ly[t]); ymax = fmax(ymax, ly[t]);
-    }
-    m.xc = (xmin + xmax) / 2; m.yc = (ymin + ymax) / 2;
     build_fast_const(*cfg, &h->fast);
     build_fast_const(*cfg, &h->fast64);
     h->fast_baked = wf_baked_matches(h->fast) && !getenv("WFCRL_B200_NO_BAKED");  // env var: force the generic kernel (tests)
 
     int rc = WF_OK;
     auto fail = [&](int r) { wf_destroy(h); return r; };
-    double *d_ws, *d_ct, *d_pw, *d_lx, *d_ly;
+    double *d_ws, *d_ct, *d_pw;
     if ((rc = dev_alloc(h, &d_ws, cfg->table_len))) return fail(rc);
     if ((rc = dev_alloc(h, &d_ct, cfg->table_len))) return fail(rc);
     if ((rc = dev_alloc(h, &d_pw, cfg->table_len))) return fail(rc);
-    if ((rc = dev_alloc(h, &d_lx, T))) return fail(rc);
-    if ((rc = dev_alloc(h, &d_ly, T))) return fail(rc);
+    if ((rc = set_pool(h, 1, lx, ly))) return fail(rc);  // a pool of one layout; every env has layout id 0
     {
         std::vector<double> pw(cfg->table_len);
         const double area = 3.141592653589793 * pow(cfg->rotor_diameter / 2.0, 2.0);
@@ -229,10 +267,8 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
         cudaMemcpy(d_ws, cfg->table_ws, sizeof(double) * cfg->table_len, cudaMemcpyHostToDevice);
         cudaMemcpy(d_ct, cfg->table_ct, sizeof(double) * cfg->table_len, cudaMemcpyHostToDevice);
         cudaMemcpy(d_pw, pw.data(), sizeof(double) * cfg->table_len, cudaMemcpyHostToDevice);
-        cudaMemcpy(d_lx, lx, sizeof(double) * T, cudaMemcpyHostToDevice);
-        cudaMemcpy(d_ly, ly, sizeof(double) * T, cudaMemcpyHostToDevice);
     }
-    m.tab_ws = d_ws; m.tab_ct = d_ct; m.tab_pw = d_pw; m.layout_x = d_lx; m.layout_y = d_ly;
+    m.tab_ws = d_ws; m.tab_ct = d_ct; m.tab_pw = d_pw;
 
     WfState& s = h->st;
     const size_t BT = (size_t)B * T;
@@ -250,7 +286,7 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
         (rc = dev_alloc(h, &s.cs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.xhl, BT)) ||
         (rc = dev_alloc(h, &s.yhl, BT)) || (rc = dev_alloc(h, &s.idx, BT)) || (rc = dev_alloc(h, &h->d_mask, (size_t)B)) ||
         (rc = dev_alloc(h, &h->d_rws, (size_t)B)) || (rc = dev_alloc(h, &h->d_rwd, (size_t)B)) ||
-        (rc = dev_alloc(h, &h->d_rcs, (size_t)2 * B)))
+        (rc = dev_alloc(h, &h->d_rcs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.layout_id, (size_t)B)))
         return fail(rc);
     if ((rc = dev_alloc(h, &s.tab_lo, BT)) || (rc = dev_alloc(h, &s.tab_glo, BT))) return fail(rc);
     // The vortex table trades the V sweep's arithmetic for one streamed read of 36 reals per turbine pair.  Measured on B200
@@ -447,6 +483,54 @@ int wf_reset(WfHandle h, const int32_t* ids, int32_t n, const double* ws, const 
     for (int k = 0; k < warmup; ++k)
         TRY(launch_step(h, WF_MODE_WARMUP, h->d_mask, nullptr, nullptr, to_ptrs(out), st));
     CUDA_TRY(cudaStreamSynchronize(st));  // the handle-owned pinned staging is reusable when this call returns
+    return WF_OK;
+}
+
+int wf_set_layouts(WfHandle h, int32_t n_layouts, const double* lx, const double* ly) {
+    if (!h || !lx || !ly) return set_err(WF_ERR_INVALID, "NULL argument");
+    if (n_layouts < 1) return set_err(WF_ERR_INVALID, "n_layouts must be >= 1");
+    TRY(check_layouts((size_t)n_layouts * h->model.T, lx, ly));
+    CUDA_TRY(cudaSetDevice(h->device));
+    CUDA_TRY(cudaDeviceSynchronize());  // after every earlier asynchronous call: no queued kernel reads the old pool any more
+    TRY(set_pool(h, n_layouts, lx, ly));
+    CUDA_TRY(cudaMemset(h->st.layout_id, 0, sizeof(int) * h->model.B));
+    CUDA_TRY(rebuild_geometry(h, nullptr, 0));
+    CUDA_TRY(cudaDeviceSynchronize());
+    return WF_OK;
+}
+
+int wf_assign_layouts(WfHandle h, const int32_t* ids, int32_t n, const int32_t* layout_ids, void* stream) {
+    if (!h || !layout_ids) return set_err(WF_ERR_INVALID, "NULL argument");
+    const int B = h->model.B, L = h->model.n_layouts;
+    if (n < 0 || n > B) return set_err(WF_ERR_INVALID, "bad n");
+    if (!ids && n != B) return set_err(WF_ERR_INVALID, "h_env_ids == NULL requires n == num_envs");
+    for (int k = 0; k < n; ++k) {
+        if (ids && (ids[k] < 0 || ids[k] >= B)) return set_err(WF_ERR_INVALID, "env id out of range");
+        if (layout_ids[k] < 0 || layout_ids[k] >= L)
+            return set_err(WF_ERR_INVALID, "layout id out of range [0, n_layouts)");
+    }
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    // read-modify-write of the id array: the envs not listed keep theirs
+    std::vector<int32_t> lid(B);
+    CUDA_TRY(cudaMemcpyAsync(lid.data(), h->st.layout_id, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    memset(h->h_mask, 0, B);
+    for (int k = 0; k < n; ++k) {
+        const int b = ids ? ids[k] : k;
+        lid[b] = layout_ids[k];
+        h->h_mask[b] = 1;
+    }
+    CUDA_TRY(cudaMemcpyAsync(h->st.layout_id, lid.data(), sizeof(int32_t) * B, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(h->d_mask, h->h_mask, B, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(rebuild_geometry(h, h->d_mask, st));
+    CUDA_TRY(cudaStreamSynchronize(st));  // the host staging is reusable when this call returns
+    return WF_OK;
+}
+
+int wf_set_layout_sampling(WfHandle h, int32_t enabled) {
+    if (!h) return set_err(WF_ERR_INVALID, "NULL handle");
+    h->model.sample_layouts = enabled ? 1 : 0;
     return WF_OK;
 }
 
@@ -693,7 +777,7 @@ static int find_state(WfHandle h, const char* name, void** p, size_t* bytes) {
         {"fin_sumsq", s.fin_sumsq, B * 8}, {"fin_n", s.fin_n, B * 4}, {"fin_len", s.fin_len, B * 8}, {"ws", s.ws, B * 8}, {"wd", s.wd, B * 8},
         {"ws_norm", s.ws_norm, B * 8}, {"shaper_ref", s.shaper_ref, B * 8}, {"ti_ambient", s.ti_amb, B * 8},
         {"order", s.order, BT * 4}, {"xs", s.xs, BT * 8}, {"ys", s.ys, BT * 8}, {"xi", s.xi, BT * 8},
-        {"yi", s.yi, BT * 8}, {"cs", s.cs, B * 16}};
+        {"yi", s.yi, BT * 8}, {"cs", s.cs, B * 16}, {"layout_id", s.layout_id, B * 4}};
     for (auto& e : tab)
         if (!strcmp(e.n, name)) { *p = e.p; *bytes = e.b; return WF_OK; }
     return set_err(WF_ERR_INVALID, std::string("unknown state array '") + name + "'");
@@ -712,6 +796,9 @@ int wf_get_state(WfHandle h, const char* name, void* dst, size_t bytes) {
 
 int wf_set_state(WfHandle h, const char* name, const void* src, size_t bytes) {
     if (!h || !name || !src) return set_err(WF_ERR_INVALID, "NULL argument");
+    if (!strcmp(name, "layout_id"))
+        return set_err(WF_ERR_INVALID, "\"layout_id\" is read-only here: wf_assign_layouts sets it, validates the ids and "
+                                       "rebuilds the geometry");
     void* p; size_t b;
     TRY(find_state(h, name, &p, &b));
     if (b != bytes) return set_err(WF_ERR_INVALID, "size mismatch for state array");

@@ -26,12 +26,16 @@ struct WfModel {
     double alpha, beta, ka, kb, ad, bd, dm;
     double ch_const, ch_ai, ch_init, ch_down;
     double e3_112, e3_13;          // 3*exp(1/12), 3*exp(1/3) (Gauss deflection E0)
-    double xc, yc;                 // centre of the layout bounding box (rotation centre)
+    // The pool fields below fill the 16 bytes of the single layout's former (xc, yc), so that neither the offsets of the
+    // fields after them nor the size of the struct (and with it every later kernel parameter) moved.
+    const double* layout_c;        // [L][2] device: centre of each pool layout's bounding box (its rotation centre)
+    int n_layouts;                 // L: layouts in the pool (wf_set_layouts)
+    int sample_layouts;            // 1 = library-sampled resets also draw the env's layout id (wf_set_layout_sampling)
     const double* tab_ws;          // [table_len] device
     const double* tab_ct;          // [table_len]
     const double* tab_pw;          // [table_len] 0.5*area*Cp*eta*ws^3 (power / density)
-    const double* layout_x;        // [T] device
-    const double* layout_y;        // [T]
+    const double* layout_x;        // [L][T] device: the layout pool; env b's geometry is built from row layout_id[b]
+    const double* layout_y;        // [L][T]
 };
 
 // Per-env state, device pointers (owned by the handle).
@@ -70,7 +74,7 @@ struct WfState {
     double* cs;         // [B][2] cosd/sind of the deviation from west actually used
     // FP32 fast-kernel geometry: positions relative to the rotation centre as float-float pairs and, per SOURCE
     // position i, the first sorted target index for which each FP64 x-mask of SURVEY A.7/A.8 becomes true
-    float2* xhl;        // [B][T] (hi, lo) of xs - xc
+    float2* xhl;        // [B][T] (hi, lo) of xs - xc (xc, yc: the centre of the env's layout)
     float2* yhl;        // [B][T] (hi, lo) of ys - yc
     uchar4* idx;        // [B][T] .x: first t with X[t]-x_i >= 0 ; .y: first t with X[t] > x_i+0.1 ;
                         //         .z: first t with X[t] > x_i ; .w: first t with X[t] > x_i+15D   (T if none)
@@ -92,6 +96,7 @@ struct WfState {
     // that the rows one target sums in its prologue are contiguous; the finished (v, w) of every rotor point and the direct
     // contributions between x-tied turbines live in this scratch (rewritten by every launch; L2-resident while an env runs)
     double2* vwg;       // [B][9T]; an FP64 handle has both the table and this scratch, or neither
+    int* layout_id;     // [B] row of the layout pool (WfModel.layout_x / _y / _c) the env's geometry is built from
 };
 
 // Constants of the tuned warp-per-env kernels, precomputed on the host in FP64 (wf_host_const.h: build_fast_const);

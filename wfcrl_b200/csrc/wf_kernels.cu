@@ -184,7 +184,8 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
     __shared__ double xr[WF_MAX_TURBINES_K], yr[WF_MAX_TURBINES_K], xsrt[WF_MAX_TURBINES_K];
     __shared__ double cs[2];
     if (t == 0) {
-        if (autoreset_draw) wfreset::autoreset_wind(m, s, b);  // second half of an in-kernel auto-reset: the new episode's wind
+        // second half of an in-kernel auto-reset: the new episode's wind (and layout id)
+        if (autoreset_draw) wfreset::autoreset_wind(m, s, b);
         double c, sn;
         if (cs_override) {
             c = cs_override[2 * b];
@@ -202,11 +203,14 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
         s.cs[2 * b + 1] = sn;
     }
     __syncthreads();
+    const int lay = s.layout_id[b];  // after the barrier: thread 0 may just have drawn it
+    const double cx = m.layout_c[2 * lay], cy = m.layout_c[2 * lay + 1];
     if (t < T) {
-        const double xo = __dsub_rn(m.layout_x[t], m.xc), yo = __dsub_rn(m.layout_y[t], m.yc);
+        const size_t lt = (size_t)lay * T + t;
+        const double xo = __dsub_rn(m.layout_x[lt], cx), yo = __dsub_rn(m.layout_y[lt], cy);
         // every product / sum separately rounded: no FMA contraction (SURVEY 7.3)
-        xr[t] = __dadd_rn(__dsub_rn(__dmul_rn(xo, cs[0]), __dmul_rn(yo, cs[1])), m.xc);
-        yr[t] = __dadd_rn(__dadd_rn(__dmul_rn(xo, cs[1]), __dmul_rn(yo, cs[0])), m.yc);
+        xr[t] = __dadd_rn(__dsub_rn(__dmul_rn(xo, cs[0]), __dmul_rn(yo, cs[1])), cx);
+        yr[t] = __dadd_rn(__dadd_rn(__dmul_rn(xo, cs[1]), __dmul_rn(yo, cs[0])), cy);
     }
     __syncthreads();
     if (t < T) {
@@ -237,7 +241,7 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
             s.yi[o] = np_mean(gy, G * G);
         }
         // float-float positions relative to the rotation centre for the FP32 kernel
-        const double xrel = x - m.xc, yrel = y - m.yc;
+        const double xrel = x - cx, yrel = y - cy;
         const float xh = (float)xrel, yh = (float)yrel;
         s.xhl[o] = make_float2(xh, (float)(xrel - (double)xh));
         s.yhl[o] = make_float2(yh, (float)(yrel - (double)yh));
@@ -346,6 +350,7 @@ __global__ void wf_sample_reset_kernel(const WfModel m, const WfState s, const u
                                        const double ti_hi, double* __restrict__ ws, double* __restrict__ wd) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= m.B || (mask && !mask[b])) return;
+    if (m.sample_layouts) wfreset::sample_layout(s, b, seed, env_id_offset, m.n_layouts);  // read by the geometry kernel next
     wfreset::sample_wind(s, b, seed, env_id_offset, ti_lo, ti_hi, &ws[b], &wd[b]);
 }
 

@@ -56,6 +56,17 @@ __device__ __forceinline__ void sample_wind(const WfState& s, int b, unsigned lo
     s.episode[b] = (int)(ep + 1u);
 }
 
+// Layout draw of the same (env b, episode index): id = floor(u53 * L) from draw word 2 of sample_wind's key and counter, so
+// the winds and TI of a reset are the same whether layouts are drawn or not.  Call BEFORE sample_wind advances the episode
+// counter.  u53 < 1 rounds below L after the product, so the id is in [0, L).
+__device__ __forceinline__ void sample_layout(const WfState& s, int b, unsigned long long seed, long long env_id_offset,
+                                              int n_layouts) {
+    const unsigned long long gid = (unsigned long long)(env_id_offset + b);
+    const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
+    const uint4 r2 = philox4x32_10(make_uint4((unsigned)gid, (unsigned)(gid >> 32), (unsigned)s.episode[b], 2u), key);
+    s.layout_id[b] = (int)floor(u53(r2.x, r2.y) * n_layouts);
+}
+
 // per-env scalars of a reset (one thread); the per-turbine arrays (yaw, acc, acc_prev) are zeroed by the caller's threads
 __device__ __forceinline__ void reset_scalars(const WfState& s, int b, double ws, double wd) {
     s.ws[b] = ws;
@@ -97,8 +108,10 @@ __device__ __forceinline__ void autoreset_mark(const WfState& s, int b) {
     s.reset_mask[b] = 1;
 }
 
-// second half, first thing in the geometry kernel of a marked env: draw the wind, finish the scalar reset
+// second half, first thing in the geometry kernel of a marked env: draw the layout id (when sampling is on) and the wind,
+// finish the scalar reset
 __device__ __forceinline__ void autoreset_wind(const WfModel& m, const WfState& s, int b) {
+    if (m.sample_layouts) sample_layout(s, b, m.ar_seed, m.ar_offset, m.n_layouts);
     double ws, wd;
     sample_wind(s, b, m.ar_seed, m.ar_offset, m.ar_ti_lo, m.ar_ti_hi, &ws, &wd);
     s.ws[b] = ws;

@@ -5,7 +5,7 @@ from __future__ import annotations
 
 import math
 import re
-from typing import Union
+from typing import List, Union
 
 from ..layouts import ALIASES
 from .data_cases import DefaultControl, floris_case, registered_layouts as _layouts
@@ -66,22 +66,37 @@ def make(env_id: str, controls: Union[dict, list] = ["yaw"], log=True, **env_kwa
     return env
 
 
-def make_vec(env_id: str, num_envs: int, controls: Union[dict, list] = ["yaw"], log: int = 0, **env_kwargs):
+def make_vec(env_id: Union[str, List[str]], num_envs: int, controls: Union[dict, list] = ["yaw"], log: int = 0,
+             **env_kwargs):
     """Batched counterpart of ``make``: ``num_envs`` independent copies of ``env_id`` on one GPU, stepped by one kernel
     launch (``VecWindFarmEnv`` / ``VecMAWindFarmEnv``).  Extra kwargs: device, precision ("f32" fast / "f64" bit-check),
-    auto_reset, env_id_offset (global id of env 0 when the batch is sharded over ranks); ``log=N`` wraps the env in a
-    ``VecLogWrapper`` keeping the last N steps in device-side ring buffers."""
-    from ..vector_env import VecMAWindFarmEnv, VecWindFarmEnv
+    auto_reset, env_id_offset (global id of env 0 when the batch is sharded over ranks), layout_assignment; ``log=N``
+    wraps the env in a ``VecLogWrapper`` keeping the last N steps in device-side ring buffers.
 
-    decentralized, name, simulator = _parse(env_id)
-    case = get_case(name, simulator)
-    validate_case(env_id, case)
+    A list of env ids gives one batch over several farms (the layout pool of ``VecWindFarmEnv``): the ids must be all
+    centralised or all ``Dec_``, and their layouts must share the turbine count, ``dt`` and ``t_init``."""
+    from ..vector_env import VecMAWindFarmEnv, VecWindFarmEnv, layout_pool
+
+    env_ids = [env_id] if isinstance(env_id, str) else list(env_id)
+    if not env_ids:
+        raise ValueError("env_id list is empty")
+    parsed = [_parse(e) for e in env_ids]
+    decentralized = parsed[0][0]
+    if any(p[0] != decentralized for p in parsed):
+        raise ValueError(f"cannot batch centralised and decentralised (Dec_) envs together: {env_ids}")
+    layouts = []
+    for e, (_dec, name, simulator) in zip(env_ids, parsed):
+        case = get_case(name, simulator)
+        validate_case(e, case)
+        layouts.append({"num_turbines": case.num_turbines, "xcoords": case.xcoords, "ycoords": case.ycoords,
+                        "dt": case.dt, "t_init": case.t_init})
+    layout_pool(layouts)  # same turbine count, dt and t_init, checked before any device work
     if not isinstance(controls, dict):
         controls = get_default_control(controls)
-    layout = {"num_turbines": case.num_turbines, "xcoords": case.xcoords, "ycoords": case.ycoords, "dt": case.dt,
-              "t_init": case.t_init}
+    case = layouts[0]
+    layout = case if len(layouts) == 1 else layouts
     cls = VecMAWindFarmEnv if decentralized else VecWindFarmEnv
-    env = cls(layout, num_envs, controls=controls, start_iter=math.ceil(case.t_init / case.dt), **env_kwargs)
+    env = cls(layout, num_envs, controls=controls, start_iter=math.ceil(case["t_init"] / case["dt"]), **env_kwargs)
     if log:
         from ..wrappers import VecLogWrapper
 

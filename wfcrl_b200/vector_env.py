@@ -14,7 +14,7 @@ full agent cycle of the reference's AEC env, wfcrl/multiagent_env.py:159-254).
 from __future__ import annotations
 
 from collections import OrderedDict
-from typing import Dict, Optional, Union
+from typing import Dict, List, Optional, Union
 
 import numpy as np
 import torch
@@ -27,25 +27,54 @@ from .rewards import DoNothingReward, RewardShaper
 _OBS_BOUNDS = {"wind_speed": (3.0, 28.0), "wind_direction": (0.0, 360.0)}
 
 
+def layout_pool(layout) -> List[Dict]:
+    """The farm cases of ``layout``: one layout name or dict, or a list of them.  The layouts of a pool must share the
+    turbine count (the observation and action spaces), ``dt`` and ``t_init``; raises ValueError otherwise."""
+    items = list(layout) if isinstance(layout, (list, tuple)) else [layout]
+    if not items:
+        raise ValueError("layout list is empty")
+    cases = [get_layout(c) if isinstance(c, str) else c for c in items]
+    for key, default in (("num_turbines", None), ("dt", 60), ("t_init", None)):
+        values = [c.get(key, default) for c in cases]
+        if any(v != values[0] for v in values):
+            raise ValueError(f"the layouts of one batch must share {key}, got {values}")
+    return cases
+
+
 class VecWindFarmEnv:
     """``num_envs`` copies of one ``*_Floris`` env on one GPU (see the module docstring).
 
     ALIASING: ``reset`` / ``step`` return observation, reward, ``info["power"]`` and ``info["load"]`` as VIEWS of the
     backend's output buffers, which the next ``step`` overwrites in place (and, on auto-reset steps, the warm-up solve of
     the restarted envs already has).  A rollout buffer must ``.clone()`` what it keeps, or construct the env with
-    ``copy_outputs=True`` to get fresh tensors from every call (one extra device copy of ~10 floats per turbine)."""
+    ``copy_outputs=True`` to get fresh tensors from every call (one extra device copy of ~10 floats per turbine).
+
+    LAYOUT POOL: ``layout`` may be a list of layouts (names or dicts) of one turbine count, ``dt`` and ``t_init``.  With
+    ``layout_assignment="cycle"`` the env of global id ``g = env_id_offset + b`` runs layout ``g % L`` for good; with
+    ``"sample"`` every reset draws the env's layout uniformly (in the library for ``reset(seed=None)`` and auto-resets,
+    with numpy's ``default_rng((seed + g, 2))`` for ``reset(seed=seed)``).  ``reset(options={"layout": ids})`` sets the
+    layout of the reset envs explicitly; ``layout_ids`` returns the current ones."""
 
     metadata = {"name": "vectorized-windfarm"}
 
-    def __init__(self, layout: Union[str, Dict], num_envs: int, *, device: int = 0, precision: str = "f32",
+    def __init__(self, layout: Union[str, Dict, List], num_envs: int, *, device: int = 0, precision: str = "f32",
                  kernel: Optional[str] = None, controls: Optional[dict] = None, continuous_control: bool = True,
                  reward_shaper: Optional[RewardShaper] = None, max_num_steps: int = 500, load_coef: float = 0.1,
                  start_iter: int = 0, auto_reset: bool = True, multi_agent: bool = False, env_id_offset: int = 0,
                  wind_time_series: Optional[Union[str, np.ndarray]] = None, exact_host_trig: Optional[bool] = None,
-                 turbulence_intensity_range: Optional[tuple] = None, copy_outputs: bool = False):
-        case = get_layout(layout) if isinstance(layout, str) else layout
+                 turbulence_intensity_range: Optional[tuple] = None, copy_outputs: bool = False,
+                 layout_assignment: str = "cycle"):
+        cases = layout_pool(layout)
+        if layout_assignment not in ("cycle", "sample"):
+            raise ValueError(f"layout_assignment must be 'cycle' or 'sample', got {layout_assignment!r}")
+        if layout_assignment == "sample" and wind_time_series is not None:
+            raise ValueError("layout_assignment='sample' draws layouts at library-sampled resets, which time-series mode "
+                             "does not use; assign layouts with 'cycle' or reset(options={'layout': ...})")
+        case = cases[0]
         self.copy_outputs = bool(copy_outputs)
         self.farm_case = case
+        self.farm_cases = cases
+        self.layout_assignment = layout_assignment
         self.num_envs = int(num_envs)
         self.num_turbines = case["num_turbines"]
         self.dt = case.get("dt", 60)
@@ -78,6 +107,12 @@ class VecWindFarmEnv:
                                    shaper_reference=float(getattr(self.reward_shaper, "reference", 0.0)),
                                    continuous_control=continuous_control, multi_agent=multi_agent)
         self.device = self.backend.device
+        if len(cases) > 1:
+            self.backend.set_layouts([c["xcoords"] for c in cases], [c["ycoords"] for c in cases])
+            if layout_assignment == "cycle":
+                self.backend.assign_layouts(None, (self.env_id_offset + np.arange(self.num_envs)) % len(cases))
+        if layout_assignment == "sample":
+            self.backend.set_layout_sampling(True)
         T = self.num_turbines
         self.single_action_space = spaces.Dict({"yaw": spaces.Box(-step, step, shape=(T,))}) if continuous_control \
             else spaces.Dict({"yaw": spaces.MultiDiscrete([3] * T)})
@@ -158,7 +193,8 @@ class VecWindFarmEnv:
 
     def reset(self, seed: Optional[int] = None, options: Optional[dict] = None, env_ids=None):
         """Reset all (or ``env_ids``) envs.  ``options`` may carry ``wind_speed`` / ``wind_direction`` (scalars or
-        per-env arrays) exactly like the reference; otherwise both are sampled per env.
+        per-env arrays) exactly like the reference; otherwise both are sampled per env.  ``options["layout"]`` (a scalar or
+        per-env pool index) sets the layout of the reset envs; otherwise ``layout_assignment="sample"`` draws it.
 
         ``seed=s`` draws env ``g``'s wind with numpy exactly as the reference's ``reset(seed=s + g)`` would and makes
         ``s`` the key of all later in-loop resets; ``seed=None`` draws on the device (``wf_reset_sampled``).  Either way
@@ -177,11 +213,24 @@ class VecWindFarmEnv:
         if self._series is not None:
             start = np.random.randint(0, self._series.shape[0], size=len(ids))  # interface.py:517
             self._series_pos[idt] = torch.as_tensor(start, device=self.device)
-        if seed is None and not any_given and self._series is None:
-            # nothing to reproduce on the host: winds (and TI) drawn by the library for the selected envs
+        in_library = seed is None and not any_given and self._series is None
+        sampling = self.layout_assignment == "sample"
+        if "layout" in options:
+            self.backend.assign_layouts(ids, options["layout"])
+        elif sampling and not in_library:  # as the sampled TI below: one numpy stream per (seed + global id, 2)
+            n_layouts = len(self.farm_cases)
+            self.backend.assign_layouts(ids, [np.random.default_rng(
+                None if seed is None else (seed + self.env_id_offset + int(b), 2)).integers(n_layouts) for b in ids])
+        if in_library:
+            # nothing to reproduce on the host: winds (and TI, layouts) drawn by the library for the selected envs
             mask = torch.zeros(self.num_envs, dtype=torch.uint8, device=self.device)
             mask[idt] = 1
+            keep_layouts = sampling and "layout" in options  # the layouts given in options are not redrawn
+            if keep_layouts:
+                self.backend.set_layout_sampling(False)
             out = self.backend.reset_sampled(mask, self._seed, self.env_id_offset, warm, self.turbulence_intensity_range)
+            if keep_layouts:
+                self.backend.set_layout_sampling(True)
         else:
             if self._series is not None:
                 first = self._series[self._series_pos[idt]].cpu().numpy()
@@ -248,6 +297,11 @@ class VecWindFarmEnv:
             obs = self._obs(out)
         self.last_info = info  # joint (un-split) info of this step, incl. final_observation on auto-reset steps
         return obs, reward, self._zeros_bool, truncated, info
+
+    @property
+    def layout_ids(self):
+        """Index into the layout list of the layout every env currently runs (int32 [B], device copy)."""
+        return torch.as_tensor(self.backend.get_state("layout_id"), device=self.device)
 
     @property
     def episode_returns(self):
