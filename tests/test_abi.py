@@ -2,6 +2,7 @@
 import ctypes as C
 import os
 import re
+import subprocess
 
 import numpy as np
 import pytest
@@ -122,3 +123,53 @@ def test_version_string_carries_the_hash_of_the_sources():
     version = _lib.load().wf_version().decode()
     assert version.startswith("wfcrl_b200 ") and version.endswith("wfcrl_b200-src-sha256:" + build.source_hash())
     assert _lib.binary_matches_source()
+
+
+def test_compiled_code_is_a_function_of_the_sources(monkeypatch, tmp_path):
+    """The source hash stands for the binary: the sources select no code by a macro from outside (their only conditional
+    is on the hash itself), and no environment variable the package reads changes the nvcc command."""
+    from wfcrl_b200 import build
+
+    for f in sorted(os.listdir(build.CSRC)):
+        if f.endswith((".cu", ".cuh", ".h")):
+            for line in open(os.path.join(build.CSRC, f)):
+                if re.match(r"\s*#\s*(if|elif)", line):
+                    assert "WF_SOURCE_HASH" in line, (f, line)
+
+    names = set()
+    for dirpath, _dirs, files in os.walk(os.path.join(ROOT, "wfcrl_b200")):
+        for f in files:
+            if f.endswith((".py", ".cu", ".cuh", ".h")):
+                names.update(re.findall(r"\bWFCRL_[A-Z0-9_]*[A-Z0-9]\b", open(os.path.join(dirpath, f)).read()))
+    names.update({"WFCRL_NVCC_FLAGS", "WFCRL_DEBUG"})
+
+    src_hash = build.source_hash()
+    # every file the build writes goes to tmp_path (source_hash() would follow HERE there)
+    monkeypatch.setattr(build, "source_hash", lambda: src_hash)
+    monkeypatch.setattr(build, "HERE", str(tmp_path))
+    monkeypatch.setattr(build, "BAKED", str(tmp_path / "wf_fast_baked.inc"))
+    monkeypatch.setattr(build, "LIB", str(tmp_path / "libwfcrl_b200.so"))
+    monkeypatch.setattr(build, "_nvcc", lambda: "nvcc")
+    calls = []
+
+    def run(cmd, **_kw):
+        calls.append(list(cmd))
+        if "-o" in cmd:
+            open(cmd[cmd.index("-o") + 1], "w").close()
+        return subprocess.CompletedProcess(cmd, 0, stdout="", stderr="")
+
+    monkeypatch.setattr(subprocess, "run", run)
+
+    def library_command(env):
+        for k in [k for k in os.environ if k.startswith("WFCRL_")]:
+            monkeypatch.delenv(k)
+        for k, v in env.items():
+            monkeypatch.setenv(k, v)
+        calls.clear()
+        build.build_library(force=True)
+        return calls[-1]
+
+    plain = library_command({})
+    assert plain[-len(build.SOURCES):] == [os.path.join(build.CSRC, s) for s in build.SOURCES]
+    assert f'-DWF_SOURCE_HASH="{src_hash}"' in plain
+    assert library_command({k: "-DWF_OUTSIDE_SWITCH=1 -O0" for k in names}) == plain

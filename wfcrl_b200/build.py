@@ -72,9 +72,9 @@ def build_library(force: bool = False, verbose: bool = False) -> str:
         fp.write(subprocess.run([gen_exe], check=True, capture_output=True, text=True).stdout)
     os.remove(gen_exe)
     # step 2: the library
-    extra = os.environ.get("WFCRL_NVCC_EXTRA", "").split()  # e.g. -DWF_FAST_MINB=14 for tuning experiments
-    extra.append(f'-DWF_SOURCE_HASH="{source_hash()}"')      # wf_version() reports what the binary was built from
-    cmd = [_nvcc()] + NVCC_FLAGS + extra + ["-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES]
+    # a function of the tree alone, so that the source hash wf_version() reports stands for the binary
+    cmd = ([_nvcc()] + NVCC_FLAGS + [f'-DWF_SOURCE_HASH="{source_hash()}"', "-o", LIB] +
+           [os.path.join(CSRC, s) for s in SOURCES])
     proc = subprocess.run(cmd, capture_output=True, text=True)
     log = proc.stdout + proc.stderr
     with open(os.path.join(HERE, "build.log"), "w") as fp:

@@ -220,6 +220,8 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
         return set_err(WF_ERR_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(e));
     if (cfg->device < 0 || cfg->device >= ndev) return set_err(WF_ERR_INVALID, "bad device ordinal");
     CUDA_TRY(cudaSetDevice(cfg->device));
+    CUDA_TRY(wf_configure_fast_kernels());
+    CUDA_TRY(wf_configure_fast64_kernels());
 
     WfHandle_t* h = new WfHandle_t();
     h->cfg = *cfg;
@@ -278,7 +280,7 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
         (rc = dev_alloc(h, &s.reset_mask, (size_t)B)) || (rc = dev_alloc(h, &s.ep_return, (size_t)B)) ||
         (rc = dev_alloc(h, &s.ep_len, (size_t)B)) || (rc = dev_alloc(h, &s.fin_sum, (size_t)B)) ||
         (rc = dev_alloc(h, &s.fin_sumsq, (size_t)B)) || (rc = dev_alloc(h, &s.fin_n, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.fin_len, (size_t)B)) || (rc = dev_alloc(h, &s.fix_list, (size_t)B)) || (rc = dev_alloc(h, &s.fix_count, (size_t)4 * WF_FIX_SLOTS)) ||
+        (rc = dev_alloc(h, &s.fin_len, (size_t)B)) || (rc = dev_alloc(h, &s.fix_list, (size_t)B)) || (rc = dev_alloc(h, &s.fix_count, (size_t)4)) ||
         (rc = dev_alloc(h, &s.ws, (size_t)B)) || (rc = dev_alloc(h, &s.wd, (size_t)B)) ||
         (rc = dev_alloc(h, &s.ws_norm, (size_t)B)) || (rc = dev_alloc(h, &s.shaper_ref, (size_t)B)) ||
         (rc = dev_alloc(h, &s.ti_amb, (size_t)B)) || (rc = dev_alloc(h, &s.xs, BT)) || (rc = dev_alloc(h, &s.ys, BT)) ||
@@ -369,7 +371,7 @@ static bool is_strict_f32(WfHandle h) {
 // FP64 re-solve of the envs flagged by the FP32 launches issued since the previous fix-up (all of them must precede this launch
 // in stream order); d_rec / rec_cap: optional compact copies of the re-solved envs' results (host path)
 static int launch_fixup(WfHandle h, int mode, const WfOutPtrs& out, cudaStream_t st, float* d_rec = nullptr, int rec_cap = 0) {
-    cudaError_t e = wf_launch_fixup64(mode, !h->vtab_stale, h->model, h->fast64, h->st, out, h->model.B, 0, d_rec, rec_cap, st);
+    cudaError_t e = wf_launch_fixup64(mode, !h->vtab_stale, h->model, h->fast64, h->st, out, h->model.B, d_rec, rec_cap, st);
     h->launches += 1;
     if (e != cudaSuccess) return set_err(WF_ERR_CUDA, std::string("fix-up kernel launch: ") + cudaGetErrorString(e));
     return WF_OK;
@@ -413,7 +415,7 @@ static int launch_step(WfHandle h, int mode, const uint8_t* d_mask, const float*
         e = wf_launch_step_fast64(mode, !h->vtab_stale, h->model, h->fast64, h->st, d_mask, d_action, d_yaw, out, env_begin, env_count, st);
     else if (h->cfg.kernel == WF_KERNEL_FAST)
     {
-        e = wf_launch_step_fast(mode, h->fast_baked, h->model, h->fast, h->st, d_mask, d_action, d_yaw, out, env_begin, env_count, 0,
+        e = wf_launch_step_fast(mode, h->fast_baked, h->model, h->fast, h->st, d_mask, d_action, d_yaw, out, env_begin, env_count,
                                 st);
         if (e == cudaSuccess && is_strict_f32(h) && !defer_fixup) {  // strict FP32: FP64 re-solve of whatever the launch flagged
             if (timed) { cudaEventRecord(h->ev_t[1], st); tail.mid = true; }

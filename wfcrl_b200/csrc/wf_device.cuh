@@ -4,7 +4,6 @@
 #include <stdint.h>
 
 #define WF_MAX_TURBINES_K 128  // == WF_MAX_TURBINES of the public header
-#define WF_FIX_SLOTS 2  // fix-up counter sets (only slot 0 is used: launches of one handle that may overlap share one list)
 #define WF_FIX_REC_HDR 5  // floats ahead of the per-turbine part of a fix-up record (see wf_fixup64_kernel)
 #define WF_NP 9  // 3x3 rotor grid (case.yaml:16), p = 3*j + k with j lateral, k vertical
 
@@ -58,8 +57,8 @@ struct WfState {
     long long* fin_len; // [B]   and the sum of their lengths
     uint8_t* reset_mask;// [B] 1 = the env was reset inside a step kernel and still needs its geometry + warm-up solve
     int* fix_list;      // [B] ids of the envs flagged by the FP32 launches since the last fix-up launch (appended atomically)
-    int* fix_count;     // [4 * WF_FIX_SLOTS] per slot: number of flagged envs, number of fix-up CTAs that have left, the
-                        //     number of envs the last fix-up launch re-solved, (pad)
+    int* fix_count;     // [4] number of flagged envs, number of fix-up CTAs that have left, the number of envs the last fix-up
+                        //     launch re-solved, (pad)
     double* ws;         // [B] free-stream wind speed
     double* wd;         // [B] free-stream wind direction (already % 360)
     double* ws_norm;    // [B] free-stream speed of the PREVIOUS state (reward normalisation, simple_env.py:79)
@@ -159,11 +158,15 @@ cudaError_t wf_launch_sample_reset(const WfModel& m, const WfState& s, const uin
 cudaError_t wf_launch_reset_state(const WfModel& m, const WfState& s, const uint8_t* d_mask, const double* d_ws,
                                   const double* d_wd, cudaStream_t stream);
 cudaError_t wf_step_basic_attributes(int precision, cudaFuncAttributes* attr, int* ctas_per_sm, int threads);
+// Kernel attributes of the tuned kernels (dynamic shared memory above 48 KB, carveout).  They belong to the current
+// device, so wf_create sets them once per handle, before the handle's first launch.
+cudaError_t wf_configure_fast_kernels();    // wf_fast.cu
+cudaError_t wf_configure_fast64_kernels();  // wf_fast64.cu
 cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                 const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                const WfOutPtrs& out, int env_begin, int env_count, int slot, cudaStream_t stream);
+                                const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream);
 cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                              const WfOutPtrs& out, int env_count, int slot, float* d_rec, int rec_cap, cudaStream_t stream);
+                              const WfOutPtrs& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream);
 cudaError_t wf_step_fast_attributes(bool baked, const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                     int* smem);
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,

@@ -45,19 +45,6 @@ constexpr float kRad = 0.017453292519943295f;
 constexpr float kNumEpsF = 0.001f;
 constexpr int kTurbPerPass = 10;
 constexpr int kMaxEvt = 8;  // ambiguous-decision records kept per env; more than that flags the env outright
-#define WF_STR_(x) #x
-#define WF_PRAGMA_UNROLL_(n) _Pragma(WF_STR_(unroll n))
-#ifndef WF_FAST_UNROLL_V
-#define WF_FAST_UNROLL_V 2  // two V-sweep passes in flight per warp (ILP); measured +3.5 % on B200
-#endif
-#define WF_UNROLL_V WF_PRAGMA_UNROLL_(WF_FAST_UNROLL_V)
-#ifndef WF_FAST_UNROLL_D
-#define WF_FAST_UNROLL_D 1
-#endif
-#define WF_UNROLL_D WF_PRAGMA_UNROLL_(WF_FAST_UNROLL_D)
-#ifndef WF_FAST_MINB
-#define WF_FAST_MINB 12  // lower bound on resident env-CTAs per SM for the register allocator (16 are reached)
-#endif
 
 __device__ __forceinline__ float frcp(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float fsqrt(float x) { float y; asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
@@ -136,9 +123,10 @@ __device__ __forceinline__ SmemView carve(unsigned char* base, int T) {
 struct wf_true_tag { static constexpr bool value = true; };
 struct wf_false_tag { static constexpr bool value = false; };
 
+// generic instantiation: 12 is a lower bound for the register allocator; 16 envs per SM are reached
 template <bool BAKED>
-__global__ void __launch_bounds__(32, BAKED ? 16 : WF_FAST_MINB)
-wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const WfModel m, const __grid_constant__ WfFastConst fc,
+__global__ void __launch_bounds__(32, BAKED ? 16 : 12)
+wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
                     const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
                     const double* __restrict__ yaw_cmd, const WfOutPtrs out) {
     const int b = blockIdx.x + env_begin;
@@ -407,17 +395,18 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
                 }
             }
         };
+        // two passes in flight per warp (ILP): +3.5 %; unrolling the D sweep and 3-pass V unrolling measured slower
         if (sy != 0.f) {
-            WF_UNROLL_V
+#pragma unroll 2
             for (int t0 = lo; t0 < T; t0 += kTurbPerPass) v_pass(wf_true_tag{}, t0);
         } else {
-            WF_UNROLL_V
+#pragma unroll 2
             for (int t0 = lo; t0 < T; t0 += kTurbPerPass) v_pass(wf_false_tag{}, t0);
         }
         __syncwarp();
 
         // ===== D sweep: deflection + Gaussian deficit + wake-added TI, only on the queued targets =====
-        WF_UNROLL_D
+#pragma unroll 1
         for (int q0 = 0; q0 < qn; q0 += kTurbPerPass) {
             const int e = q0 + g;
             const bool active = lane_ok && e < qn;
@@ -575,7 +564,7 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
     if (any_flag && strict) {
         // the FP64 re-solve (wf_fixup64_kernel, next launch on this stream) redoes this env from the committed yaw state and
         // commits the per-env epilogue state itself
-        if (lane == 0) s.fix_list[atomicAdd(&s.fix_count[4 * slot], 1)] = b;
+        if (lane == 0) s.fix_list[atomicAdd(&s.fix_count[0], 1)] = b;
         return;
     }
     int it = 0;
@@ -615,41 +604,37 @@ wf_step_fast_kernel(const int mode, const int env_begin, const int slot, const W
 
 }  // namespace
 
+cudaError_t wf_configure_fast_kernels() {
+    for (auto k : {wf_step_fast_kernel<true>, wf_step_fast_kernel<false>}) {
+        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 template <bool BAKED>
 static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                  const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                 const WfOutPtrs& out, int env_begin, int env_count, int slot, cudaStream_t stream) {
-    const size_t smem = fast_smem_bytes(m.T);
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                 cudaSharedmemCarveoutMaxShared);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    wf_step_fast_kernel<BAKED><<<env_count, 32, smem, stream>>>(mode, env_begin, slot, m, fc, s, d_mask, d_action, d_yaw_cmd, out);
+                                 const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
+    wf_step_fast_kernel<BAKED><<<env_count, 32, fast_smem_bytes(m.T), stream>>>(mode, env_begin, m, fc, s, d_mask, d_action,
+                                                                               d_yaw_cmd, out);
     return cudaGetLastError();
 }
 
 cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                 const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                const WfOutPtrs& out, int env_begin, int env_count, int slot, cudaStream_t stream) {
-    return baked ? launch_fast_t<true>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, slot, stream)
-                 : launch_fast_t<false>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, slot, stream);
+                                const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
+    return baked ? launch_fast_t<true>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, stream)
+                 : launch_fast_t<false>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, stream);
 }
 
 template <bool BAKED>
 static cudaError_t attrs_fast_t(const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads, int* smem) {
     *threads = 32;
     *smem = (int)fast_smem_bytes(m.T);
-    cudaError_t e = cudaFuncSetAttribute(wf_step_fast_kernel<BAKED>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                         cudaSharedmemCarveoutMaxShared);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncGetAttributes(attr, wf_step_fast_kernel<BAKED>);
+    cudaError_t e = cudaFuncGetAttributes(attr, wf_step_fast_kernel<BAKED>);
     if (e != cudaSuccess) return e;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, wf_step_fast_kernel<BAKED>, 32, *smem);
 }

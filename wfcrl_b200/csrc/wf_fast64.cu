@@ -26,11 +26,6 @@
 #include "wf_reset_device.cuh"
 
 #include <math.h>
-#include <stdlib.h>
-
-#ifndef WF_VTAB64_PF_DIST
-#define WF_VTAB64_PF_DIST 1  // table rows of source i + 1 are prefetched to L2 while source i is processed (2: -4 %, 4: -8 %)
-#endif
 
 namespace {
 
@@ -68,19 +63,15 @@ template <int BASE> __device__ __forceinline__ void bar_sync(int parity, int cou
 // division / sqrt / cbrt (IEEE rounding, full range, special cases) are 15-50 dependent instructions each.  The quantities
 // in the chain are positive, finite and far inside the float range, and the kernels owe 1e-9, not the last bit: seed with the
 // single-precision special-function unit and refine with Newton steps in double (error ~1e-15, a quarter of the instructions).
-#ifndef WF_LEAN_NEWTON
-#define WF_LEAN_NEWTON 2  // Newton steps after the single-precision seed.  1 was measured (profiles/r2_exp_newton.log): +2.8 % on
-                          // the FP64 step kernels, +0.5 % on the strict FP32 step, FP64 parity max 1.1e-12 -> 5.9e-11 (median
-                          // 3e-16 -> 5e-15); the bit-check mode keeps the margin
-#endif
+// Two Newton steps each: one was measured (profiles/r2_exp_newton.log) +2.8 % faster on the FP64 step kernels and +0.5 % on
+// the strict FP32 step, but took the FP64 parity max from 1.1e-12 to 5.9e-11 (median 3e-16 -> 5e-15); the bit-check mode
+// keeps the margin.
 __device__ __forceinline__ double rcp64(double b) {
     float rf;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rf) : "f"((float)b));
     double r = (double)rf;
     r = fma(r, fma(-b, r, 1.0), r);  // 6e-8 -> 4e-15
-#if WF_LEAN_NEWTON > 1
     r = fma(r, fma(-b, r, 1.0), r);  // -> rounding
-#endif
     return r;
 }
 __device__ __forceinline__ double sqrt64(double x) {  // x > 0
@@ -89,9 +80,7 @@ __device__ __forceinline__ double sqrt64(double x) {  // x > 0
     const double r = (double)rf, h = 0.5 * r;
     double y = x * r;
     y = fma(h, fma(-y, y, x), y);  // 1e-7 -> 1e-14
-#if WF_LEAN_NEWTON > 1
     y = fma(h, fma(-y, y, x), y);
-#endif
     return y;
 }
 __device__ __forceinline__ double sqrt64z(double x) { return x > 1e-30 ? sqrt64(x) : sqrt(x); }  // x >= 0, possibly tiny
@@ -101,9 +90,7 @@ __device__ __forceinline__ double cbrt64(double x) {  // x > 0
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(rf) : "f"((float)(3.0 * y0 * y0)));
     const double rc = (double)rf;
     double y = fma(fma(-y0 * y0, y0, x), rc, y0);  // Newton on y^3 = x with a single-precision slope: 1e-7 -> 1e-14
-#if WF_LEAN_NEWTON > 1
     y = fma(fma(-y * y, y, x), rc, y);
-#endif
     return y;
 }
 
@@ -292,10 +279,9 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     const double cwl0 = fc.cw[0][plc], cwl1 = fc.cw[1][plc], cwl2 = fc.cw[2][plc];
     const double c_dec = fc.eps2 * fc.inv_2pi;
     const double eps2 = fc.eps2;
-    if (vrow && warp == 0) {
-        if (!GATHER)
-            for (int d = 0; d < WF_VTAB64_PF_DIST; ++d) prefetch_rows64(vrow, d, T, lane, 288);
-    }
+    // scatter form: the table rows of source 0 are prefetched to L2 here, those of source i + 1 while source i is processed
+    // (prefetching 2 sources ahead measured -4 %, 4 ahead -8 %)
+    if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, 0, T, lane, 288);
 
     // W > 1, chain warp: the transverse velocities source i - 1 induces on turbine i are not written to shared memory but added
     // in registers at the head of source i's prologue, from table coefficients loaded one source earlier (no load latency on
@@ -304,7 +290,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     double2 near_c0 = make_double2(0.0, 0.0), near_c1 = make_double2(0.0, 0.0);
     bool near_tab = false;
     for (int i = 0; i < T; ++i) {
-        if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, i + WF_VTAB64_PF_DIST, T, lane, 288);
+        if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, i + 1, T, lane, 288);
         double2 next_c0 = make_double2(0.0, 0.0), next_c1 = make_double2(0.0, 0.0);
         bool next_tab = false;
         if (W > 1 && warp == 0 && vrow && i + 1 < T && i + 1 >= (int)s.tab_lo[row + i]) {
@@ -377,11 +363,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
                 sw += __shfl_xor_sync(0xffffffffu, sw, sft);
             }
         }
-#ifdef WF_DBG_SKIP_CBRT  // timing experiment only
-        const double avg = 8.0 + 1e-9 * su3;
-#else
         const double avg = cbrt64(su3 * (1.0 / 9.0));
-#endif
         const double ct_raw = dclamp(interp_d(fc, fc.tab_ct, avg, 0.0001, 0.9999), 0.0001, 0.9999);
         const double cy = sm.cyaw[i], sy = sm.syaw[i], yd = sm.ynew[sm.ordr[i]];
         const double ct = ct_raw * cy;
@@ -396,15 +378,9 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         // A.5 secondary steering through the per-model grid integrals (the denominator is (c_top a_top - c_bot a_bot) ws ct)
         double val = 2.0 * (sv * (1.0 / 9.0) - Gwr * fc.a_core) * (rct * fc.inv_ss_den) * rws;
         val = dclamp(val, -1.0, 1.0);
-#ifdef WF_DBG_SKIP_TRIG  // timing experiment only
-        const double g_deg = -(yd + kDeg * (0.5 * val));
-        const double g_rad = g_deg * kRad;
-        const double cg = 1.0 - 0.5 * g_rad * g_rad;
-#else
         const double g_deg = -(yd + kDeg * (0.5 * asin(val)));  // minus the effective yaw, degrees
         const double g_rad = g_deg * kRad;
         const double cg = cos(g_rad);
-#endif
         const double rcg = rcp64(cg);
 
         // A.6 deflection scalars.  M0 = C0 (2 - C0) = 1 - (1 - C0)^2 = ct.
@@ -496,11 +472,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         const double ctc = ct * cy * fc.d2_8;
         // Crespo-Hernandez constant ch_const a^ai I0^init.  W > 1: only the deficit sweeps need it, so the chain warp hands over
         // `a` and the power is taken where a sweep finds a target within reach (off the chain's critical path)
-#ifdef WF_DBG_SKIP_POW  // timing experiment only
-        const double watK = fc.ch_const * a * I0p;
-#else
         const double watK = (W == 1) ? fc.ch_const * exp(fc.ch_ai * log(a)) * I0p : a;  // a^ai (pow(): 3x the instructions, same to 1e-15)
-#endif
 
         constexpr double kCut = 9.5;
         const double reach1 = kCut * kyv;
@@ -732,20 +704,14 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
                 const double dx = sm.xs[t] - x_i;
                 const double dyc = __dsub_rn(__dadd_rn(sm.ys[t], offj), y_i);
                 const bool tab = vrow && t >= t_hi;
-#ifndef WF_DBG_SKIP_V  // timing experiment only
                 if (__any_sync(0xffffffffu, active && !tab)) v_direct(t, dx, dyc, active && !tab);
                 if (tab && !skip_vtab) v_table(t, active);
-#endif
                 const bool need = active && (t >= near_i) && (fabs(dyc) < reach(dx));
                 const unsigned nb = __ballot_sync(0xffffffffu, need);
-#ifndef WF_DBG_SKIP_D  // timing experiment only
                 if (nb) {
-#ifndef WF_DBG_SKIP_POW
                     if (!have_watK) { watK = fc.ch_const * exp(fc.ch_ai * log(watK)) * I0p; have_watK = true; }
-#endif
                     d_apply(t, dx, dyc, active && (((nb >> (3 * g)) & 7u) != 0u));
                 }
-#endif
             };
             if (warp == 0) {
                 if (i > 0) bar_sync<3>(i - 1, NT);
@@ -887,11 +853,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
 // sub-partition with two others (12 per SM), one of 128 registers with three (16 per SM; 12-48 bytes of spills).  The kernels
 // are latency-bound, throughput grows with the resident envs (measured on Turb32_Row5: 6 per SM 4.9 M env-steps/s, 9: 6.2 M,
 // 12: 7.6 M, 16: 8.2 M); at 80 turbines shared memory holds 14 envs of the gather kernel per SM (9 of the scatter kernel).
-#ifndef WF_FAST64_GATHER_MINB
-#define WF_FAST64_GATHER_MINB 16
-#endif
 template <bool GATHER>
-__global__ void __launch_bounds__(32, WF_FAST64_GATHER_MINB)
+__global__ void __launch_bounds__(32, 16)
 wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                       const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
                       const double* __restrict__ yaw_cmd, const WfOutPtrs out) {
@@ -900,14 +863,14 @@ wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, 
     solve_env64<1, double, false, GATHER>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out);
 }
 
-// Re-solve, in FP64, of the envs an FP32 launch flagged (their ids sit in s.fix_list[env_begin ...], their number in
-// s.fix_count[2 slot]); launched right behind every FP32 step launch of a strict handle, usually with nothing or a handful of
-// envs to do, so it is built for latency: W warps per env.  The last CTA to leave re-arms the counters.
+// Re-solve, in FP64, of the envs an FP32 launch flagged (their ids sit in s.fix_list[0, n), n in s.fix_count[0]); launched
+// right behind every FP32 step launch of a strict handle, usually with nothing or a handful of envs to do, so it is built for
+// latency: W warps per env.  The last CTA to leave re-arms the counters.
 template <int W>
 __global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
-wf_fixup64_kernel(const int mode, const int slot, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
+wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                   const WfState s, const WfOutPtrs out, float* __restrict__ rec, const int rec_cap) {
-    const int n = *(volatile int*)&s.fix_count[4 * slot];
+    const int n = *(volatile int*)&s.fix_count[0];
     const int rec_len = WF_FIX_REC_HDR + 8 * m.T;  // header (env id, reward, freewind x2, truncated) + yaw, ws, wd, power, load x4
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
         solve_env64<W, float, true>(s.fix_list[k], mode, use_vtab, m, fc, s, nullptr, nullptr, out,
@@ -916,33 +879,40 @@ wf_fixup64_kernel(const int mode, const int slot, const bool use_vtab, const WfM
     }
     if (threadIdx.x == 0) {
         __threadfence();
-        if (atomicAdd(&s.fix_count[4 * slot + 1], 1) == (int)gridDim.x - 1) {
-            s.fix_count[4 * slot + 2] = n;
-            s.fix_count[4 * slot] = 0;
-            s.fix_count[4 * slot + 1] = 0;
+        if (atomicAdd(&s.fix_count[1], 1) == (int)gridDim.x - 1) {
+            s.fix_count[2] = n;
+            s.fix_count[0] = 0;
+            s.fix_count[1] = 0;
         }
     }
 }
 
 }  // namespace
 
+// Dynamic shared memory up to 100 KB for every FP64 kernel; the step kernels also prefer the largest shared-memory carveout.
+cudaError_t wf_configure_fast64_kernels() {
+    for (auto k : {wf_step_fast64_kernel<false>, wf_step_fast64_kernel<true>}) {
+        cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (e != cudaSuccess) return e;
+    }
+    for (auto k : {wf_fixup64_kernel<1>, wf_fixup64_kernel<2>, wf_fixup64_kernel<4>, wf_fixup64_kernel<8>}) {
+        const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 template <int W>
 static cudaError_t launch_fixup_t(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                  const WfOutPtrs& out, int grid, int slot, float* d_rec, int rec_cap, cudaStream_t stream) {
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(wf_fixup64_kernel<W>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
-    wf_fixup64_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, slot, use_vtab, m, fc, s, out, d_rec, rec_cap);
+                                  const WfOutPtrs& out, int grid, float* d_rec, int rec_cap, cudaStream_t stream) {
+    wf_fixup64_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_rec, rec_cap);
     return cudaGetLastError();
 }
 
 cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                              const WfOutPtrs& out, int env_count, int slot, float* d_rec, int rec_cap, cudaStream_t stream) {
+                              const WfOutPtrs& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream) {
     // The launch is latency-bound while the flagged envs (1-2 % of the batch) are fewer than the CTAs the GPU holds at once,
     // and each env is a sequential sweep over its turbines: W warps per env cover 10 W targets in one fused pass per source.
     // So: as many warps as the farm can use (T / 10), fewer when the batch is large enough for the flagged envs to outnumber
@@ -950,24 +920,17 @@ cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const W
     int w = m.T > 40 ? 8 : (m.T > 20 ? 4 : (m.T > 10 ? 2 : 1));
     const int expected = env_count / 64 + 1;  // ~1.5 % of the envs
     while (w > 1 && expected > 148 * 8 / w) w >>= 1;
-    static const int forced = getenv("WFCRL_B200_FIX_WARPS") ? atoi(getenv("WFCRL_B200_FIX_WARPS")) : 0;  // tuning experiments
-    if (forced == 1 || forced == 2 || forced == 4 || forced == 8) w = forced;
     const int resident = 148 * 8 / w;  // two ~196-register warps per SM sub-partition = 8 warps per SM
     const int grid = env_count < resident ? env_count : resident;
     switch (w) {
-        case 8: return launch_fixup_t<8>(mode, use_vtab, m, fc, s, out, grid, slot, d_rec, rec_cap, stream);
-        case 4: return launch_fixup_t<4>(mode, use_vtab, m, fc, s, out, grid, slot, d_rec, rec_cap, stream);
-        case 2: return launch_fixup_t<2>(mode, use_vtab, m, fc, s, out, grid, slot, d_rec, rec_cap, stream);
-        default: return launch_fixup_t<1>(mode, use_vtab, m, fc, s, out, grid, slot, d_rec, rec_cap, stream);
+        case 8: return launch_fixup_t<8>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
+        case 4: return launch_fixup_t<4>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
+        case 2: return launch_fixup_t<2>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
+        default: return launch_fixup_t<1>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
     }
 }
 
 static bool fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
-template <typename K> static cudaError_t configure_fast64(K kernel) {
-    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-}
 
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
@@ -975,15 +938,6 @@ cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, con
     // a target-major table (and its scratch) belongs to the gather kernel; the scatter kernel evaluates every pair directly
     const bool gather = fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = configure_fast64(wf_step_fast64_kernel<false>);
-        if (e == cudaSuccess) e = configure_fast64(wf_step_fast64_kernel<true>);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
     if (gather)
         wf_step_fast64_kernel<true><<<env_count, 32, smem, stream>>>(mode, env_begin, true, m, fc, s, d_mask, d_action, d_yaw_cmd, out);
     else
@@ -996,9 +950,7 @@ cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFu
     *threads = 32;
     const bool gather = fast64_gathers(m, s);
     *smem = (int)fast64_smem_bytes(m.T, gather);
-    cudaError_t e = gather ? configure_fast64(wf_step_fast64_kernel<true>) : configure_fast64(wf_step_fast64_kernel<false>);
-    if (e != cudaSuccess) return e;
-    e = gather ? cudaFuncGetAttributes(attr, wf_step_fast64_kernel<true>) : cudaFuncGetAttributes(attr, wf_step_fast64_kernel<false>);
+    cudaError_t e = gather ? cudaFuncGetAttributes(attr, wf_step_fast64_kernel<true>) : cudaFuncGetAttributes(attr, wf_step_fast64_kernel<false>);
     if (e != cudaSuccess) return e;
     return gather ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, wf_step_fast64_kernel<true>, 32, *smem)
                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(ctas_per_sm, wf_step_fast64_kernel<false>, 32, *smem);
