@@ -14,7 +14,8 @@
  *    reference arithmetic) and float with WF_PREC_F32 (fast mode, <=1e-4 relative on every turbine with the tuned
  *    kernel unless WfConfig.fp32_relaxed is set).
  *  - all `d_*` pointers are DEVICE pointers on the handle's device, all `h_*` pointers are HOST pointers.
- *  - per-turbine arrays are row-major [num_envs][num_turbines] in the ORIGINAL turbine order of the layout.
+ *  - per-turbine arrays are row-major [num_envs][num_turbines] in the ORIGINAL turbine order of the layout.  An env whose
+ *    layout has n < num_turbines turbines (wf_set_layouts_sized) uses columns 0..n-1; columns n.. are padding.
  *  - output buffers must be aligned to 16 bytes (`load` is written with 128-bit stores, `freewind` with 64-bit stores).
  *  - all launches are asynchronous on the `stream` argument (a cudaStream_t passed as void*; NULL = default
  *    stream); no host synchronisation happens inside unless stated.
@@ -128,6 +129,21 @@ int wf_destroy(WfHandle h);
  * Synchronous: it waits for every earlier asynchronous call on the handle.
  */
 int wf_set_layouts(WfHandle h, int32_t n_layouts, const double* h_x, const double* h_y);
+/*
+ * The same with a turbine count per layout: layout l has h_counts[l] in [1, T] turbines, its first h_counts[l] entries of
+ * h_x[l], h_y[l] ([n_layouts][T]); entries at or beyond the count are ignored and need not be finite, and the bounding-box
+ * centre is taken over the layout's own turbines.  wf_set_layouts is the case of every count equal to T.
+ * An env of n < T turbines runs them in columns 0..n-1 of every [B][T] array ("turbine_count" i32[B] in wf_get_state):
+ *  - columns n..T-1 (padding) of yaw, wind_speed, wind_direction, power and load are written as 0 by every call;
+ *  - the padding of the yaw / acc / acc_prev state holds 0 at all times (wf_set_state refuses nonzero padding; an env
+ *    that moves to a smaller layout through wf_assign_layouts or a layout draw has its new padding zeroed), and actions
+ *    and yaw commands in padding columns are ignored;
+ *  - the reward is the mean over the env's n turbines, and every output of the env's first n columns equals, bit for bit,
+ *    that of a handle created with its layout alone in the same precision and kernel mode.
+ * Counts below T are rejected (WF_ERR_INVALID, before anything changes) on WF_KERNEL_BASIC and multi_agent handles, which
+ * do not support padding; so are counts outside [1, T] and non-finite coordinates within a count.
+ */
+int wf_set_layouts_sized(WfHandle h, int32_t n_layouts, const int32_t* h_counts, const double* h_x, const double* h_y);
 /*
  * Sets the layout ids of the listed envs and rebuilds their geometry.  h_env_ids: HOST int32 [n] or NULL with
  * n == num_envs meaning "all envs in order"; h_layout_ids: HOST int32 [n] in [0, n_layouts).  Out-of-range env or layout
@@ -250,8 +266,9 @@ int wf_set_turbulence_intensity(WfHandle h, const double* d_ti, void* stream);
  *   "ws" f64[B] | "wd" f64[B] | "ws_norm" f64[B] | "shaper_ref" f64[B] | "ti_ambient" f64[B] |
  *   "order" i32[B][T] | "xs" f64[B][T] | "ys" f64[B][T] | "xi" f64[B][T] | "yi" f64[B][T] | "cs" f64[B][2] |
  *   "layout_id" i32[B] (row of the layout pool each env uses; read-only here: wf_set_state refuses it, wf_assign_layouts
- *   sets it)
- * `bytes` must equal the full array size.
+ *   sets it) | "turbine_count" i32[B] (turbine count of that layout; read-only)
+ * `bytes` must equal the full array size.  wf_set_state refuses "yaw", "acc" and "acc_prev" arrays that are nonzero in
+ * an env's padding columns (see wf_set_layouts_sized).
  */
 int wf_get_state(WfHandle h, const char* name, void* h_dst, size_t bytes);
 int wf_set_state(WfHandle h, const char* name, const void* h_src, size_t bytes);

@@ -52,6 +52,7 @@ SYMBOLS = {
     "wf_create": (C.c_int, [C.POINTER(WfConfig), _P, _P, C.POINTER(_P)]),
     "wf_destroy": (C.c_int, [_P]),
     "wf_set_layouts": (C.c_int, [_P, C.c_int32, _P, _P]),
+    "wf_set_layouts_sized": (C.c_int, [_P, C.c_int32, _P, _P, _P]),
     "wf_assign_layouts": (C.c_int, [_P, _P, C.c_int32, _P, _P]),
     "wf_set_layout_sampling": (C.c_int, [_P, C.c_int32]),
     "wf_reset": (C.c_int, [_P, _P, C.c_int32, _P, _P, _P, _P, C.c_int32, C.POINTER(WfStepOut), _P]),

@@ -26,6 +26,7 @@ _STATE_DTYPES = {
     "ws_norm": (np.float64, "B"), "shaper_ref": (np.float64, "B"), "ti_ambient": (np.float64, "B"),
     "order": (np.int32, "BT"), "xs": (np.float64, "BT"), "ys": (np.float64, "BT"), "xi": (np.float64, "BT"),
     "yi": (np.float64, "BT"), "cs": (np.float64, "B2"), "layout_id": (np.int32, "B"),
+    "turbine_count": (np.int32, "B"),
 }
 
 
@@ -41,7 +42,9 @@ def _ptr(t: Optional[torch.Tensor]):
 
 class FlorisBatch:
     """``num_envs`` independent Floris-backed wind-farm envs resident on one GPU.  They share the layout given here
-    unless ``set_layouts`` gives the handle a pool of layouts of the same turbine count to assign per env."""
+    unless ``set_layouts`` gives the handle a pool of layouts of the same turbine count to assign per env, or
+    ``set_mixed_layouts`` a pool of layouts of 1..T turbines (an env of n turbines uses columns 0..n-1 of every [B, T]
+    array; the other columns are padding and read 0)."""
 
     def __init__(self, layout_x: Sequence[float], layout_y: Sequence[float], num_envs: int, *, device: int = 0,
                  precision: str = "f64", kernel: str = "basic", max_iter: int = 500,
@@ -119,6 +122,27 @@ class FlorisBatch:
             raise ValueError(f"layout pool must be two [L, {self.T}] arrays, got {x.shape} and {y.shape}")
         _lib.check(self.lib.wf_set_layouts(self.handle, x.shape[0], x.ctypes.data_as(C.c_void_p),
                                            y.ctypes.data_as(C.c_void_p)))
+
+    def set_mixed_layouts(self, xs, ys) -> None:
+        """Replace the layout pool by layouts of different turbine counts: ``xs``, ``ys`` are lists of 1-D arrays
+        (metres), layout l of ``len(xs[l])`` in [1, T] turbines.  An env of n turbines runs them in columns 0..n-1;
+        columns n..T-1 of its outputs are 0, and its results equal those of a handle created with its layout alone.
+        Otherwise as ``set_layouts``."""
+        if len(xs) != len(ys) or len(xs) < 1:
+            raise ValueError("xs and ys must be non-empty lists of the same length")
+        L, T = len(xs), self.T
+        counts = np.empty(L, dtype=np.int32)
+        x = np.zeros((L, T), dtype=np.float64)
+        y = np.zeros((L, T), dtype=np.float64)
+        for l, (lx, ly) in enumerate(zip(xs, ys)):
+            lx, ly = np.asarray(lx, dtype=np.float64).reshape(-1), np.asarray(ly, dtype=np.float64).reshape(-1)
+            if lx.shape != ly.shape or not 1 <= lx.shape[0] <= T:
+                raise ValueError(f"layout {l}: x and y must be two 1-D arrays of the same length in [1, {T}], "
+                                 f"got {lx.shape} and {ly.shape}")
+            counts[l] = lx.shape[0]
+            x[l, :counts[l]], y[l, :counts[l]] = lx, ly
+        _lib.check(self.lib.wf_set_layouts_sized(self.handle, L, counts.ctypes.data_as(C.c_void_p),
+                                                 x.ctypes.data_as(C.c_void_p), y.ctypes.data_as(C.c_void_p)))
 
     def assign_layouts(self, env_ids, layout_ids) -> None:
         """Give the envs ``env_ids`` (None = all) the pool layouts ``layout_ids`` (scalar or per env) and rebuild their
@@ -286,7 +310,7 @@ class FlorisBatch:
 
     def state_dict(self) -> Dict[str, np.ndarray]:
         """Host copy of everything needed to resume the batch exactly where it is (geometry is rebuilt from wd and the
-        layout ids; the layout pool itself is configuration and is not saved)."""
+        layout ids, which also give each env's turbine count; the layout pool itself is configuration and is not saved)."""
         sd = {name: self.get_state(name) for name in self._CHECKPOINT}
         sd["cs"] = self.get_state("cs")
         sd["layout_id"] = self.get_state("layout_id")

@@ -67,7 +67,9 @@ struct WfHandle_t {
     double t_step_ms = 0.0, t_fix_ms = 0.0;
     int t_calls = 0;
     uint64_t steps_since_wind_update = 1u << 30;  // wf_update_wind rebuilds the vortex table only when it is not called every step
-    double* d_pool = nullptr;  // the layout pool in one allocation: [L][T] x, [L][T] y, [L][2] centres (WfModel.layout_*)
+    double* d_pool = nullptr;  // the layout pool in one allocation: [L][T] x, [L][T] y, [L][2] centres, [L] int32 turbine
+                               // counts (WfModel.layout_*)
+    std::vector<int> layout_n;  // host copy of the pool's turbine counts
 };
 
 template <typename T> static int dev_alloc(WfHandle_t* h, T** p, size_t n) {
@@ -114,23 +116,26 @@ static int check_layouts(size_t n, const double* lx, const double* ly) {
     return WF_OK;
 }
 
-// Replace the layout pool by L validated host layouts [L][T] and store the centre of each one's bounding box, the point the
-// geometry kernel rotates it about.  The caller makes sure that no queued kernel still reads the old pool.
-static int set_pool(WfHandle h, int L, const double* lx, const double* ly) {
+// Replace the layout pool by L validated host layouts [L][T] of counts[l] turbines each and store the centre of each one's
+// bounding box (over its own turbines), the point the geometry kernel rotates it about.  Entries at or beyond a layout's
+// count are stored as 0.  The caller makes sure that no queued kernel still reads the old pool.
+static int set_pool(WfHandle h, int L, const int* counts, const double* lx, const double* ly) {
     const size_t T = h->model.T, LT = (size_t)L * T;
-    std::vector<double> pool(LT * 2 + (size_t)L * 2);
-    memcpy(pool.data(), lx, sizeof(double) * LT);
-    memcpy(pool.data() + LT, ly, sizeof(double) * LT);
+    std::vector<double> pool(LT * 2 + (size_t)L * 2 + ((size_t)L + 1) / 2);  // + the int32 counts
     for (int l = 0; l < L; ++l) {
+        const int n = counts[l];
         const double *x = lx + l * T, *y = ly + l * T;
+        memcpy(pool.data() + l * T, x, sizeof(double) * n);
+        memcpy(pool.data() + LT + l * T, y, sizeof(double) * n);
         double xmin = x[0], xmax = x[0], ymin = y[0], ymax = y[0];
-        for (size_t t = 1; t < T; ++t) {
+        for (int t = 1; t < n; ++t) {
             xmin = fmin(xmin, x[t]); xmax = fmax(xmax, x[t]);
             ymin = fmin(ymin, y[t]); ymax = fmax(ymax, y[t]);
         }
         pool[2 * LT + 2 * l] = (xmin + xmax) / 2;
         pool[2 * LT + 2 * l + 1] = (ymin + ymax) / 2;
     }
+    memcpy(pool.data() + 2 * LT + 2 * L, counts, sizeof(int) * L);  // layout_counts(): behind the centres
     double* d = nullptr;
     cudaError_t e = cudaMalloc(&d, sizeof(double) * pool.size());
     if (e != cudaSuccess) return set_err(WF_ERR_NOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
@@ -141,6 +146,7 @@ static int set_pool(WfHandle h, int L, const double* lx, const double* ly) {
     }
     if (h->d_pool) cudaFree(h->d_pool);
     h->d_pool = d;
+    h->layout_n.assign(counts, counts + L);
     WfModel& m = h->model;
     m.layout_x = d; m.layout_y = d + LT; m.layout_c = d + 2 * LT; m.n_layouts = L;
     return WF_OK;
@@ -260,7 +266,7 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
     if ((rc = dev_alloc(h, &d_ws, cfg->table_len))) return fail(rc);
     if ((rc = dev_alloc(h, &d_ct, cfg->table_len))) return fail(rc);
     if ((rc = dev_alloc(h, &d_pw, cfg->table_len))) return fail(rc);
-    if ((rc = set_pool(h, 1, lx, ly))) return fail(rc);  // a pool of one layout; every env has layout id 0
+    if ((rc = set_pool(h, 1, &T, lx, ly))) return fail(rc);  // a pool of one layout; every env has layout id 0
     {
         std::vector<double> pw(cfg->table_len);
         const double area = 3.141592653589793 * pow(cfg->rotor_diameter / 2.0, 2.0);
@@ -288,7 +294,8 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
         (rc = dev_alloc(h, &s.cs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.xhl, BT)) ||
         (rc = dev_alloc(h, &s.yhl, BT)) || (rc = dev_alloc(h, &s.idx, BT)) || (rc = dev_alloc(h, &h->d_mask, (size_t)B)) ||
         (rc = dev_alloc(h, &h->d_rws, (size_t)B)) || (rc = dev_alloc(h, &h->d_rwd, (size_t)B)) ||
-        (rc = dev_alloc(h, &h->d_rcs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.layout_id, (size_t)B)))
+        (rc = dev_alloc(h, &h->d_rcs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.layout_id, (size_t)B)) ||
+        (rc = dev_alloc(h, &s.turbine_count, (size_t)B)))
         return fail(rc);
     if ((rc = dev_alloc(h, &s.tab_lo, BT)) || (rc = dev_alloc(h, &s.tab_glo, BT))) return fail(rc);
     // The vortex table trades the V sweep's arithmetic for one streamed read of 36 reals per turbine pair.  Measured on B200
@@ -489,12 +496,28 @@ int wf_reset(WfHandle h, const int32_t* ids, int32_t n, const double* ws, const 
 }
 
 int wf_set_layouts(WfHandle h, int32_t n_layouts, const double* lx, const double* ly) {
-    if (!h || !lx || !ly) return set_err(WF_ERR_INVALID, "NULL argument");
+    if (!h) return set_err(WF_ERR_INVALID, "NULL argument");
     if (n_layouts < 1) return set_err(WF_ERR_INVALID, "n_layouts must be >= 1");
-    TRY(check_layouts((size_t)n_layouts * h->model.T, lx, ly));
+    const std::vector<int32_t> counts(n_layouts, h->model.T);
+    return wf_set_layouts_sized(h, n_layouts, counts.data(), lx, ly);
+}
+
+int wf_set_layouts_sized(WfHandle h, int32_t n_layouts, const int32_t* counts, const double* lx, const double* ly) {
+    if (!h || !counts || !lx || !ly) return set_err(WF_ERR_INVALID, "NULL argument");
+    if (n_layouts < 1) return set_err(WF_ERR_INVALID, "n_layouts must be >= 1");
+    const int T = h->model.T;
+    for (int l = 0; l < n_layouts; ++l) {
+        if (counts[l] < 1 || counts[l] > T)
+            return set_err(WF_ERR_INVALID, "layout " + std::to_string(l) + ": turbine count " + std::to_string(counts[l]) +
+                                               " is outside [1, num_turbines = " + std::to_string(T) + "]");
+        if (counts[l] < T && (h->cfg.kernel == WF_KERNEL_BASIC || h->model.multi_agent))
+            return set_err(WF_ERR_INVALID, "layouts with fewer turbines than the handle (padding) are not supported on "
+                                           "WF_KERNEL_BASIC or multi_agent handles: every count must equal num_turbines");
+        TRY(check_layouts((size_t)counts[l], lx + (size_t)l * T, ly + (size_t)l * T));
+    }
     CUDA_TRY(cudaSetDevice(h->device));
     CUDA_TRY(cudaDeviceSynchronize());  // after every earlier asynchronous call: no queued kernel reads the old pool any more
-    TRY(set_pool(h, n_layouts, lx, ly));
+    TRY(set_pool(h, n_layouts, counts, lx, ly));
     CUDA_TRY(cudaMemset(h->st.layout_id, 0, sizeof(int) * h->model.B));
     CUDA_TRY(rebuild_geometry(h, nullptr, 0));
     CUDA_TRY(cudaDeviceSynchronize());
@@ -779,7 +802,8 @@ static int find_state(WfHandle h, const char* name, void** p, size_t* bytes) {
         {"fin_sumsq", s.fin_sumsq, B * 8}, {"fin_n", s.fin_n, B * 4}, {"fin_len", s.fin_len, B * 8}, {"ws", s.ws, B * 8}, {"wd", s.wd, B * 8},
         {"ws_norm", s.ws_norm, B * 8}, {"shaper_ref", s.shaper_ref, B * 8}, {"ti_ambient", s.ti_amb, B * 8},
         {"order", s.order, BT * 4}, {"xs", s.xs, BT * 8}, {"ys", s.ys, BT * 8}, {"xi", s.xi, BT * 8},
-        {"yi", s.yi, BT * 8}, {"cs", s.cs, B * 16}, {"layout_id", s.layout_id, B * 4}};
+        {"yi", s.yi, BT * 8}, {"cs", s.cs, B * 16}, {"layout_id", s.layout_id, B * 4},
+        {"turbine_count", s.turbine_count, B * 4}};
     for (auto& e : tab)
         if (!strcmp(e.n, name)) { *p = e.p; *bytes = e.b; return WF_OK; }
     return set_err(WF_ERR_INVALID, std::string("unknown state array '") + name + "'");
@@ -801,11 +825,25 @@ int wf_set_state(WfHandle h, const char* name, const void* src, size_t bytes) {
     if (!strcmp(name, "layout_id"))
         return set_err(WF_ERR_INVALID, "\"layout_id\" is read-only here: wf_assign_layouts sets it, validates the ids and "
                                        "rebuilds the geometry");
+    if (!strcmp(name, "turbine_count"))
+        return set_err(WF_ERR_INVALID, "\"turbine_count\" is read-only: it follows from the env's layout id");
     void* p; size_t b;
     TRY(find_state(h, name, &p, &b));
     if (b != bytes) return set_err(WF_ERR_INVALID, "size mismatch for state array");
     CUDA_TRY(cudaSetDevice(h->device));
     CUDA_TRY(cudaDeviceSynchronize());
+    const bool yaw = !strcmp(name, "yaw");
+    if (yaw || !strcmp(name, "acc") || !strcmp(name, "acc_prev")) {  // the padding columns of the state hold 0 at all times
+        const int B = h->model.B, T = h->model.T;
+        std::vector<int32_t> cnt(B);
+        CUDA_TRY(cudaMemcpy(cnt.data(), h->st.turbine_count, sizeof(int32_t) * B, cudaMemcpyDeviceToHost));
+        for (int e = 0; e < B; ++e)
+            for (int t = cnt[e]; t < T; ++t)
+                if (yaw ? ((const double*)src)[(size_t)e * T + t] != 0.0 : ((const float*)src)[(size_t)e * T + t] != 0.f)
+                    return set_err(WF_ERR_INVALID, std::string("\"") + name + "\": env " + std::to_string(e) + " has " +
+                                                       std::to_string(cnt[e]) + " turbines, but column " + std::to_string(t) +
+                                                       " (padding) is nonzero");
+    }
     CUDA_TRY(cudaMemcpy(p, src, b, cudaMemcpyHostToDevice));
     return WF_OK;
 }

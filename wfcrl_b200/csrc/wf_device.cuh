@@ -27,15 +27,20 @@ struct WfModel {
     double e3_112, e3_13;          // 3*exp(1/12), 3*exp(1/3) (Gauss deflection E0)
     // The pool fields below fill the 16 bytes of the single layout's former (xc, yc), so that neither the offsets of the
     // fields after them nor the size of the struct (and with it every later kernel parameter) moved.
-    const double* layout_c;        // [L][2] device: centre of each pool layout's bounding box (its rotation centre)
+    const double* layout_c;        // [L][2] device: centre of each pool layout's bounding box (its rotation centre),
+                                   //     followed by the [L] int32 turbine counts n <= T of the layouts (layout_counts())
     int n_layouts;                 // L: layouts in the pool (wf_set_layouts)
     int sample_layouts;            // 1 = library-sampled resets also draw the env's layout id (wf_set_layout_sampling)
     const double* tab_ws;          // [table_len] device
     const double* tab_ct;          // [table_len]
     const double* tab_pw;          // [table_len] 0.5*area*Cp*eta*ws^3 (power / density)
     const double* layout_x;        // [L][T] device: the layout pool; env b's geometry is built from row layout_id[b]
-    const double* layout_y;        // [L][T]
+    const double* layout_y;        // [L][T]; columns at or beyond the layout's turbine count are not read
 };
+
+// The pool's per-layout turbine counts, stored behind the centres (WfModel keeps its size: no kernel parameter moves).  Read
+// by the geometry kernel only, which copies the env's count to WfState.turbine_count for the other kernels.
+__host__ __device__ inline const int* layout_counts(const WfModel& m) { return (const int*)(m.layout_c + 2 * m.n_layouts); }
 
 // Per-env state, device pointers (owned by the handle).
 struct WfState {
@@ -96,6 +101,9 @@ struct WfState {
     // contributions between x-tied turbines live in this scratch (rewritten by every launch; L2-resident while an env runs)
     double2* vwg;       // [B][9T]; an FP64 handle has both the table and this scratch, or neither
     int* layout_id;     // [B] row of the layout pool (WfModel.layout_x / _y / _c) the env's geometry is built from
+    int* turbine_count; // [B] n = turbine count of that layout (written by the geometry kernel): the env runs turbines
+                        //     0..n-1 of every [B][T] row; columns n..T-1 are padding, 0 in the yaw / acc / acc_prev state
+                        //     and written as 0 in every per-turbine output
 };
 
 // Constants of the tuned warp-per-env kernels, precomputed on the host in FP64 (wf_host_const.h: build_fast_const);

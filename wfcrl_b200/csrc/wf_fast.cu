@@ -135,17 +135,19 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
     const int lane = threadIdx.x;
     const size_t row = (size_t)b * T;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const SmemView sm = carve(smem_raw, T);
+    const SmemView sm = carve(smem_raw, T);  // sized by T: every env of the handle reserves the same shared memory
+    // the env's turbine count: the one loop bound below.  Columns n..T-1 of its rows are padding (wf_device.cuh)
+    const int n = s.turbine_count[b];
 
     // ---- env prologue on the ORIGINAL turbine order (mdp.py:291-319, simple_env.py:64-72) -------------------------
     int nm = 0;
     if (mode == WF_MODE_ENV) nm = s.num_moves[b] + 1;
-    for (int tt = lane; tt < T; tt += 32) {
+    for (int tt = lane; tt < n; tt += 32) {
         float ynew;
         if (mode == WF_MODE_ENV) {
             float a = action[row + tt];
             const float acc = s.acc[row + tt];
-            const float acc_c = (m.multi_agent && tt != T - 1) ? s.acc_prev[row + tt] : acc;
+            const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
             const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
             if (frac >= 0.1f) a = 0.0f;
             if (m.continuous) a = fminf(fmaxf(a, -m.yaw_step_f), m.yaw_step_f);
@@ -169,10 +171,10 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
         sm.ordr[tt] = (unsigned char)s.order[row + tt];
     }
     if (lane < 12) sm.cblk[lane] = make_float4(fc.cblk[4 * lane], fc.cblk[4 * lane + 1], fc.cblk[4 * lane + 2], fc.cblk[4 * lane + 3]);
-    for (int q = lane; q < 9 * T; q += 32) { sm.wsq[q] = 0.f; sm.vw[q] = make_float2(0.f, 0.f); }
-    for (int q = lane; q < 3 * T; q += 32) sm.tia[q] = 0.f;
+    for (int q = lane; q < 9 * n; q += 32) { sm.wsq[q] = 0.f; sm.vw[q] = make_float2(0.f, 0.f); }
+    for (int q = lane; q < 3 * n; q += 32) sm.tia[q] = 0.f;
     __syncwarp();
-    for (int tt = lane; tt < T; tt += 32) {
+    for (int tt = lane; tt < n; tt += 32) {
         const float yr = sm.ynew[sm.ordr[tt]] * kRad;
         float sy, cy;
         sincosf(yr, &sy, &cy);
@@ -215,7 +217,7 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
     bool flagged = false;
 
     // ---- sequential solver over sources (SURVEY A.4-A.8) -------------------------------------------------------------
-    for (int i = 0; i < T; ++i) {
+    for (int i = 0; i < n; ++i) {
         // ===== source prologue =====
         // rotor sums over the source's 9 points: one point per lane, butterfly over 16-lane halves -> uniform values
         float su3, sv, sw, vq, wwq;
@@ -336,8 +338,8 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
         auto v_pass = [&](auto yawed_tag, const int t0) {
             constexpr bool YAWED = decltype(yawed_tag)::value;
             const int tr = t0 + g;
-            const bool active = lane_ok && tr < T && tr != i;
-            const int t = min(tr, T - 1);  // inactive lanes compute on a valid turbine; only their stores are masked
+            const bool active = lane_ok && tr < n && tr != i;
+            const int t = min(tr, n - 1);  // inactive lanes compute on a valid turbine; only their stores are masked
             const float2 xt = sm.xhl[t], yt = sm.yhl[t];
             const float dx = (xt.x - xi.x) + (xt.y - xi.y);
             const float dyc = ((yt.x - yi.x) + (yt.y - yi.y)) + offj;
@@ -398,10 +400,10 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
         // two passes in flight per warp (ILP): +3.5 %; unrolling the D sweep and 3-pass V unrolling measured slower
         if (sy != 0.f) {
 #pragma unroll 2
-            for (int t0 = lo; t0 < T; t0 += kTurbPerPass) v_pass(wf_true_tag{}, t0);
+            for (int t0 = lo; t0 < n; t0 += kTurbPerPass) v_pass(wf_true_tag{}, t0);
         } else {
 #pragma unroll 2
-            for (int t0 = lo; t0 < T; t0 += kTurbPerPass) v_pass(wf_false_tag{}, t0);
+            for (int t0 = lo; t0 < n; t0 += kTurbPerPass) v_pass(wf_false_tag{}, t0);
         }
         __syncwarp();
 
@@ -492,7 +494,7 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
     const bool env = (mode != WF_MODE_INTERFACE);
     const float wd = (float)wd_d;
     float rsum_p = 0.f, rsum_l = 0.f;
-    for (int tt = lane; tt < T; tt += 32) {
+    for (int tt = lane; tt < n; tt += 32) {
         float u[9], vv[9], ww[9];
         float su = 0.f, su3 = 0.f, svv = 0.f, sww = 0.f, sdd = 0.f;
 #pragma unroll
@@ -578,7 +580,7 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
         if (mode == WF_MODE_ENV) {
             s.num_moves[b] = nm;
             const float wn = (float)s.ws_norm[b];
-            const float invT = 1.f / (float)T;
+            const float invT = 1.f / (float)n;  // the mean over the env's own turbines
             float reward = rsum_p * 1e3f / (wn * wn * wn) * invT - fc.load_coef * rsum_l * (0.25f * invT);
             if (m.shaper == 1) {
                 reward = (reward - fc.shaper_reference) / fc.shaper_reference;
@@ -600,6 +602,18 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
         for (int tt = lane; tt < T; tt += 32) { s.yaw[row + tt] = 0.0; s.acc[row + tt] = 0.f; s.acc_prev[row + tt] = 0.f; }
         if (lane == 0) wfreset::autoreset_mark(s, b);
     }
+    // padding columns n..T-1 of every per-turbine output read 0, whatever an earlier layout left there (a flagged env
+    // returned above: the re-solve writes them); w = floats per turbine
+    auto zero_padding = [&](void* p, const int w) {
+        if (p)
+#pragma unroll 1
+            for (int q = n * w + lane; q < T * w; q += 32) ((float*)p)[row * w + q] = 0.f;
+    };
+    zero_padding(out.yaw, 1);
+    zero_padding(out.wind_speed, 1);
+    zero_padding(out.wind_direction, 1);
+    zero_padding(out.power, 1);
+    zero_padding(out.load, 4);
 }
 
 }  // namespace

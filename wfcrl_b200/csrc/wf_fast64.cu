@@ -36,11 +36,12 @@ constexpr double kNumEps = 0.001;
 constexpr int kTurbPerPass = 10;
 constexpr int kSrcPar = 24;  // doubles per source handed from the chain warp to the worker warps (solve_env64, W > 1)
 
-// see wf_fast.cu: pull the vortex-table rows of sorted source `i` into L2 ahead of their use (one bulk prefetch)
-__device__ __forceinline__ void prefetch_rows64(const void* env_rows, int i, int T, int lane, unsigned row_bytes) {
-    if (i >= T - 1 || lane != 0) return;
+// pull the vortex-table rows of sorted source `i` into L2 ahead of their use (one bulk prefetch): the rows of its targets
+// i+1 .. n-1 of an env of n turbines, in a table whose row strides are those of T
+__device__ __forceinline__ void prefetch_rows64(const void* env_rows, int i, int T, int n, int lane, unsigned row_bytes) {
+    if (i >= n - 1 || lane != 0) return;
     const char* p = (const char*)env_rows + ((size_t)i * T - (size_t)i * (i + 1) / 2) * row_bytes;
-    const unsigned bytes = (unsigned)(T - 1 - i) * row_bytes;
+    const unsigned bytes = (unsigned)(n - 1 - i) * row_bytes;
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
 }
 
@@ -196,6 +197,9 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     constexpr int NT = 32 * W;
     auto csync = [] { if (W == 1) __syncwarp(); else __syncthreads(); };
     const size_t row = (size_t)b * T;
+    // the env's turbine count, the bound of every loop below; columns n..T-1 of its rows are padding (wf_device.cuh).
+    // Shared memory and the table's row strides stay those of T.
+    const int n = s.turbine_count[b];
     extern __shared__ __align__(16) unsigned char smem_raw64[];
     static_assert(!GATHER || W == 1, "the gather form is the one-warp throughput kernel");
     const SmemView64 sm = carve64(smem_raw64, T, GATHER);
@@ -211,12 +215,12 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     // ---- env prologue on the ORIGINAL turbine order (mdp.py:291-319, simple_env.py:64-72) -------------------------
     int nm = 0;
     if (mode == WF_MODE_ENV) nm = s.num_moves[b] + 1;
-    for (int tt = tid; tt < T; tt += NT) {
+    for (int tt = tid; tt < n; tt += NT) {
         double ynew;
         if (!FIX && mode == WF_MODE_ENV) {
             float a = action[row + tt];
             const float acc = s.acc[row + tt];
-            const float acc_c = (m.multi_agent && tt != T - 1) ? s.acc_prev[row + tt] : acc;
+            const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
             const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
             if (frac >= 0.1f) a = 0.0f;
             if (m.continuous) a = fminf(fmaxf(a, -m.yaw_step_f), m.yaw_step_f);
@@ -239,20 +243,20 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         sm.idx[tt] = s.idx[row + tt];
         sm.ordr[tt] = (unsigned char)s.order[row + tt];
     }
-    for (int q = tid; q < 9 * T; q += NT) {
+    for (int q = tid; q < 9 * n; q += NT) {
         sm.wsq[q] = 0.0;
         if (!GATHER) sm.vw[q] = make_double2(0.0, 0.0);
     }
     if (GATHER) {  // scratch entries of the turbines that exchange direct (x-tie) contributions start from zero
-        for (int tt = tid; tt < T; tt += NT) {
+        for (int tt = tid; tt < n; tt += NT) {
             const bool tied = !vrow || (int)s.tab_glo[row + tt] < tt || (int)s.tab_lo[row + tt] > tt + 1;
             if (tied)
                 for (int p = 0; p < 9; ++p) __stcg(vwp + 9 * tt + p, make_double2(0.0, 0.0));
         }
     }
-    for (int q = tid; q < 3 * T; q += NT) sm.tia[q] = 0.0;
+    for (int q = tid; q < 3 * n; q += NT) sm.tia[q] = 0.0;
     csync();
-    for (int tt = tid; tt < T; tt += NT) {
+    for (int tt = tid; tt < n; tt += NT) {
         const double yd = sm.ynew[sm.ordr[tt]];
         double sy, cy;
         sincos(yd * kRad, &sy, &cy);
@@ -281,7 +285,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     const double eps2 = fc.eps2;
     // scatter form: the table rows of source 0 are prefetched to L2 here, those of source i + 1 while source i is processed
     // (prefetching 2 sources ahead measured -4 %, 4 ahead -8 %)
-    if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, 0, T, lane, 288);
+    if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, 0, T, n, lane, 288);
 
     // W > 1, chain warp: the transverse velocities source i - 1 induces on turbine i are not written to shared memory but added
     // in registers at the head of source i's prologue, from table coefficients loaded one source earlier (no load latency on
@@ -289,11 +293,11 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     double near_gt = 0.0, near_gwr = 0.0;
     double2 near_c0 = make_double2(0.0, 0.0), near_c1 = make_double2(0.0, 0.0);
     bool near_tab = false;
-    for (int i = 0; i < T; ++i) {
-        if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, i + 1, T, lane, 288);
+    for (int i = 0; i < n; ++i) {
+        if (!GATHER && vrow && warp == 0) prefetch_rows64(vrow, i + 1, T, n, lane, 288);
         double2 next_c0 = make_double2(0.0, 0.0), next_c1 = make_double2(0.0, 0.0);
         bool next_tab = false;
-        if (W > 1 && warp == 0 && vrow && i + 1 < T && i + 1 >= (int)s.tab_lo[row + i]) {
+        if (W > 1 && warp == 0 && vrow && i + 1 < n && i + 1 >= (int)s.tab_lo[row + i]) {
             next_tab = true;
             const double2* r = (const double2*)(vrow + ((size_t)i * T - (size_t)i * (i + 1) / 2) * 36 + 12 * (plc / 3) + 4 * (plc % 3));
             next_c0 = __ldg(r);
@@ -605,7 +609,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             }
         };
         auto reach = [&](const double dx) { return reach1 * dx + reach0 + fabs(fc.bd * dx + fc.ad); };
-        const int t_hi = vrow ? (int)s.tab_lo[row + i] : T;  // with the table only the x-ties take the direct path
+        const int t_hi = vrow ? (int)s.tab_lo[row + i] : n;  // with the table only the x-ties take the direct path
 
         if (W == 1 && GATHER) {
             // ===== direct (v, w) exchange with the x-tied turbines, queue of the targets within reach of the wake (32
@@ -614,7 +618,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             for (int t0 = lo; t0 < ((t_hi - lo > 1 || !vrow) ? t_hi : lo); t0 += kTurbPerPass) {  // without ties [lo, t_hi) = {i}
                 const int tr = t0 + g;
                 const bool active = lane_ok && tr < t_hi && tr != i;
-                const int t = min(tr, T - 1);
+                const int t = min(tr, n - 1);
                 const double dx = sm.xs[t] - x_i;
                 const double dyc = __dsub_rn(__dadd_rn(sm.ys[t], offj), y_i);
                 v_direct(t, dx, dyc, active);
@@ -623,14 +627,14 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             // 8192 x 80 (profiles/r2_exp_gather_prefetch.log): no prefetch 2.25 M env-steps/s; here 2.36 M (7.6 GB read from HBM
             // per launch = the table once); at the top of the iteration 2.31 M (8.6 GB); one iteration earlier still 2.10 M
             // (12.4 GB: with 2072 resident envs the prefetched lines no longer survive in L2 until they are used).
-            if (vrow && i + 1 < T) prefetch_target_rows64(vrow, i + 1, (int)s.tab_glo[row + i + 1], lane);
+            if (vrow && i + 1 < n) prefetch_target_rows64(vrow, i + 1, (int)s.tab_glo[row + i + 1], lane);
             int qn = 0;
 #pragma unroll 1
-            for (int t0 = near_i; t0 < T; t0 += 32) {
+            for (int t0 = near_i; t0 < n; t0 += 32) {
                 const int tr = t0 + lane;
-                const int t = min(tr, T - 1);
+                const int t = min(tr, n - 1);
                 const double r = reach(sm.xs[t] - x_i), yt = sm.ys[t];
-                const bool need = tr < T && (fabs(__dsub_rn(__dadd_rn(yt, fc.offj[0]), y_i)) < r ||
+                const bool need = tr < n && (fabs(__dsub_rn(__dadd_rn(yt, fc.offj[0]), y_i)) < r ||
                                              fabs(__dsub_rn(__dadd_rn(yt, fc.offj[1]), y_i)) < r ||
                                              fabs(__dsub_rn(__dadd_rn(yt, fc.offj[2]), y_i)) < r);
                 const unsigned nb = __ballot_sync(0xffffffffu, need);
@@ -661,7 +665,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             for (int t0 = lo; t0 < ((t_hi - lo > 1 || !vrow) ? t_hi : lo); t0 += kTurbPerPass) {  // without ties [lo, t_hi) = {i}
                 const int tr = t0 + g;
                 const bool active = lane_ok && tr < t_hi && tr != i;
-                const int t = min(tr, T - 1);
+                const int t = min(tr, n - 1);
                 const double dx = sm.xs[t] - x_i;
                 const double dyc = __dsub_rn(__dadd_rn(sm.ys[t], offj), y_i);
                 enqueue(t, active && (t >= near_i) && (fabs(dyc) < reach(dx)));
@@ -669,10 +673,10 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             }
             if (vrow) {
 #pragma unroll 2
-                for (int t0 = t_hi; t0 < T; t0 += kTurbPerPass) {
+                for (int t0 = t_hi; t0 < n; t0 += kTurbPerPass) {
                     const int tr = t0 + g;
-                    const bool active = lane_ok && tr < T;
-                    const int t = min(tr, T - 1);
+                    const bool active = lane_ok && tr < n;
+                    const int t = min(tr, n - 1);
                     const double dx = sm.xs[t] - x_i;
                     const double dyc = __dsub_rn(__dadd_rn(sm.ys[t], offj), y_i);
                     enqueue(t, active && (t >= near_i) && (fabs(dyc) < reach(dx)));
@@ -699,8 +703,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             //       is done. =====
             bool have_watK = false;
             auto sweep = [&](const int tr, const bool on, const bool skip_vtab) {
-                const bool active = on && tr >= lo && tr < T && tr != i;
-                const int t = min(max(tr, 0), T - 1);
+                const bool active = on && tr >= lo && tr < n && tr != i;
+                const int t = min(max(tr, 0), n - 1);
                 const double dx = sm.xs[t] - x_i;
                 const double dyc = __dsub_rn(__dadd_rn(sm.ys[t], offj), y_i);
                 const bool tab = vrow && t >= t_hi;
@@ -715,7 +719,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             };
             if (warp == 0) {
                 if (i > 0) bar_sync<3>(i - 1, NT);
-                if (i + 1 < T) sweep(i + 1, lane < 3, next_tab);  // (its table part is deferred to the next prologue)
+                if (i + 1 < n) sweep(i + 1, lane < 3, next_tab);  // (its table part is deferred to the next prologue)
                 __syncwarp();
                 near_gt = Gt; near_gwr = Gwr; near_c0 = next_c0; near_c1 = next_c1; near_tab = next_tab;
             } else {
@@ -723,14 +727,14 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
                 for (int t0 = lo; t0 < i; t0 += kTurbPerPass * (W - 1))  // x-tied predecessors (none without ties: lo >= i)
                     sweep(min(t0 + kTurbPerPass * (warp - 1) + g, i), lane_ok, false);
 #pragma unroll 1
-                for (int t0 = i + 2; t0 < T; t0 += kTurbPerPass * (W - 1)) sweep(t0 + kTurbPerPass * (warp - 1) + g, lane_ok, false);
+                for (int t0 = i + 2; t0 < n; t0 += kTurbPerPass * (W - 1)) sweep(t0 + kTurbPerPass * (warp - 1) + g, lane_ok, false);
                 __threadfence_block();
                 bar_arrive<3>(i, NT);
             }
         }
     }
     if (W > 1) {
-        if (warp == 0) bar_sync<3>(T - 1, NT);  // the workers' last sweep
+        if (warp == 0) bar_sync<3>(n - 1, NT);  // the workers' last sweep
         __syncthreads();
     }
 
@@ -738,7 +742,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     if (warp != 0) return;
     const bool env = (mode != WF_MODE_INTERFACE);
     double rsum_p = 0.0, rsum_l = 0.0;
-    for (int tt = lane; tt < T; tt += 32) {
+    for (int tt = lane; tt < n; tt += 32) {
         double u[9], vv[9], ww[9], c3[9], dd[9];
 #pragma unroll
         for (int p = 0; p < 9; ++p) {
@@ -808,6 +812,23 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             r[4 * T + 4 * orig + 2] = (float)loads[2]; r[4 * T + 4 * orig + 3] = (float)loads[3];
         }
     }
+#pragma unroll 1
+    for (int tt = n + lane; tt < T; tt += 32) {  // padding columns: no stale value of an earlier layout shows
+        const size_t o = row + tt;
+        if (out.yaw) ((OutT*)out.yaw)[o] = (OutT)0;
+        if (out.wind_speed) ((OutT*)out.wind_speed)[o] = (OutT)0;
+        if (out.wind_direction) ((OutT*)out.wind_direction)[o] = (OutT)0;
+        if (out.power) ((OutT*)out.power)[o] = (OutT)0;
+        if (out.load) {
+            OutT* Lp = (OutT*)out.load + 4 * o;
+            Lp[0] = (OutT)0; Lp[1] = (OutT)0; Lp[2] = (OutT)0; Lp[3] = (OutT)0;
+        }
+        if (FIX && rec) {
+            float* r = rec + WF_FIX_REC_HDR;
+            r[tt] = 0.f; r[T + tt] = 0.f; r[2 * T + tt] = 0.f; r[3 * T + tt] = 0.f;
+            r[4 * T + 4 * tt] = 0.f; r[4 * T + 4 * tt + 1] = 0.f; r[4 * T + 4 * tt + 2] = 0.f; r[4 * T + 4 * tt + 3] = 0.f;
+        }
+    }
 #pragma unroll
     for (int sft = 16; sft > 0; sft >>= 1) {
         rsum_p += __shfl_xor_sync(0xffffffffu, rsum_p, sft);
@@ -825,7 +846,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         if (mode == WF_MODE_ENV) {
             s.num_moves[b] = nm;
             const double wn = s.ws_norm[b];
-            double reward = rsum_p * 1e3 / (wn * wn * wn) / T - m.load_coef * (rsum_l / (4.0 * T));
+            double reward = rsum_p * 1e3 / (wn * wn * wn) / n - m.load_coef * (rsum_l / (4.0 * n));  // mean over the env's turbines
             if (m.shaper == 1) {
                 reward = (reward - m.shaper_reference) / m.shaper_reference;
             } else if (m.shaper == 2) {

@@ -204,8 +204,9 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
     }
     __syncthreads();
     const int lay = s.layout_id[b];  // after the barrier: thread 0 may just have drawn it
+    const int n = layout_counts(m)[lay];   // the env's turbines are 0..n-1; slots n..T-1 are padding
     const double cx = m.layout_c[2 * lay], cy = m.layout_c[2 * lay + 1];
-    if (t < T) {
+    if (t < n) {
         const size_t lt = (size_t)lay * T + t;
         const double xo = __dsub_rn(m.layout_x[lt], cx), yo = __dsub_rn(m.layout_y[lt], cy);
         // every product / sum separately rounded: no FMA contraction (SURVEY 7.3)
@@ -213,10 +214,10 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
         yr[t] = __dadd_rn(__dadd_rn(__dmul_rn(xo, cs[1]), __dmul_rn(yo, cs[0])), cy);
     }
     __syncthreads();
-    if (t < T) {
+    if (t < n) {
         const double x = xr[t], y = yr[t];
         int rank = 0;
-        for (int q = 0; q < T; ++q) {
+        for (int q = 0; q < n; ++q) {
             const double xq = xr[q];
             rank += (xq < x) || (xq == x && q < t);  // stable ascending
         }
@@ -246,16 +247,28 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
         s.xhl[o] = make_float2(xh, (float)(xrel - (double)xh));
         s.yhl[o] = make_float2(yh, (float)(yrel - (double)yh));
         xsrt[rank] = x;
+    } else if (t < T) {
+        // padding slot: sorted position t holds "turbine" t at the origin, its masks say "none" (n), and the env's padding
+        // state is zeroed (an env that moved to a smaller layout must not keep the larger layout's yaw / accumulators)
+        const size_t o = (size_t)b * T + t;
+        s.xs[o] = 0.0; s.ys[o] = 0.0; s.xi[o] = 0.0; s.yi[o] = 0.0;
+        s.order[o] = t;
+        s.xhl[o] = make_float2(0.f, 0.f);
+        s.yhl[o] = make_float2(0.f, 0.f);
+        s.idx[o] = make_uchar4((unsigned char)n, (unsigned char)n, (unsigned char)n, (unsigned char)n);
+        s.tab_lo[o] = (unsigned char)n;
+        s.tab_glo[o] = 0;
+        s.yaw[o] = 0.0; s.acc[o] = 0.f; s.acc_prev[o] = 0.f;
     }
     __syncthreads();
-    if (t < T) {
+    if (t < n) {
         // t is now a SORTED source position: first target index at which each FP64 x-mask turns true
         const size_t o = (size_t)b * T + t;
         const double x_i = s.xi[o];
         const double x01 = __dadd_rn(x_i, 0.1), x15 = __dadd_rn(15 * m.D, x_i);
         const double xtie = __dadd_rn(xsrt[t], 1e-6);
-        int i0 = T, i1 = T, i2 = T, i3 = T, i4 = T, i5 = 0;
-        for (int q = T - 1; q >= 0; --q) {
+        int i0 = n, i1 = n, i2 = n, i3 = n, i4 = n, i5 = 0;
+        for (int q = n - 1; q >= 0; --q) {
             const double xq = xsrt[q];
             i5 += xsrt[t] > __dadd_rn(xq, 1e-6);  // q's tab_lo <= t
             if (__dsub_rn(xq, x_i) >= 0.0) i0 = q;
@@ -268,6 +281,7 @@ wf_geometry_kernel(const WfModel m, const WfState s, const uint8_t* __restrict__
         s.tab_lo[o] = (unsigned char)i4;
         s.tab_glo[o] = (unsigned char)i5;
     }
+    if (t == 0) s.turbine_count[b] = n;  // what the step kernels and the vortex-table kernel read
     if (t == 0 && s.vtab_ok) s.vtab_ok[b] = 0;  // the vortex table of this env no longer matches its geometry
 }
 
@@ -284,23 +298,24 @@ wf_vortex_table_kernel(const WfModel m, const __grid_constant__ WfFastConst64 fc
     const int T = m.T;
     __shared__ double xs[WF_MAX_TURBINES_K], ys[WF_MAX_TURBINES_K], xi[WF_MAX_TURBINES_K], yi[WF_MAX_TURBINES_K];
     __shared__ int rowoff[WF_MAX_TURBINES_K];
+    const int n = s.turbine_count[b];  // rows of pairs inside the env's n turbines; row strides stay those of T
     const size_t row0 = (size_t)b * T;
-    for (int t = threadIdx.x; t < T; t += blockDim.x) {
+    for (int t = threadIdx.x; t < n; t += blockDim.x) {
         xs[t] = s.xs[row0 + t];
         ys[t] = s.ys[row0 + t];
         xi[t] = s.xi[row0 + t];
         yi[t] = s.yi[row0 + t];
-        rowoff[t] = t * T - t * (t + 1) / 2;
+        rowoff[t] = t * n - t * (t + 1) / 2;
     }
     __syncthreads();
-    const int rows = T * (T - 1) / 2;
-    double* __restrict__ tab = s.vtab + (size_t)b * rows * 36;
+    const int rows = n * (n - 1) / 2;
+    double* __restrict__ tab = s.vtab + (size_t)b * (T * (T - 1) / 2) * 36;
     const double rho = fc.c_bot / fc.c_top;  // Gb = -rho * Gt
     const double c_dec = fc.eps2 * fc.inv_2pi;
     for (int task = threadIdx.x; task < rows * 3; task += blockDim.x) {
         const int row = task / 3, j = task - 3 * row;
         // row -> (i, t): largest i with rowoff[i] <= row
-        int lo = 0, hi = T - 2;
+        int lo = 0, hi = n - 2;
         while (lo < hi) {
             const int mid = (lo + hi + 1) >> 1;
             if (rowoff[mid] <= row) lo = mid; else hi = mid - 1;
@@ -311,7 +326,7 @@ wf_vortex_table_kernel(const WfModel m, const __grid_constant__ WfFastConst64 fc
         const double yL = dyc + kNumEps;
         const double q = yL * yL;
         const double E = exp(-q * fc.inv_eps2);
-        const size_t dst = (m.vtab_tmajor ? (size_t)(t * (t - 1) / 2 + i) : (size_t)row) * 36 + j * 12;
+        const size_t dst = (m.vtab_tmajor ? (size_t)(t * (t - 1) / 2 + i) : (size_t)(i * T - i * (i + 1) / 2 + (t - i - 1))) * 36 + j * 12;
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
             double A[3], Bc[3];  // per unit circulation of (top pair, bottom pair, wake-rotation pair): V and W sums

@@ -74,7 +74,8 @@ def make_vec(env_id: Union[str, List[str]], num_envs: int, controls: Union[dict,
     wraps the env in a ``VecLogWrapper`` keeping the last N steps in device-side ring buffers.
 
     A list of env ids gives one batch over several farms (the layout pool of ``VecWindFarmEnv``): the ids must be all
-    centralised or all ``Dec_``, and their layouts must share the turbine count, ``dt`` and ``t_init``."""
+    centralised or all ``Dec_``, and their layouts must share the turbine count, ``dt`` and ``t_init``.  With
+    ``pad_turbines=True`` (centralised ids only) the turbine counts may differ: see ``VecWindFarmEnv``."""
     from ..vector_env import VecMAWindFarmEnv, VecWindFarmEnv, layout_pool
 
     env_ids = [env_id] if isinstance(env_id, str) else list(env_id)
@@ -84,13 +85,16 @@ def make_vec(env_id: Union[str, List[str]], num_envs: int, controls: Union[dict,
     decentralized = parsed[0][0]
     if any(p[0] != decentralized for p in parsed):
         raise ValueError(f"cannot batch centralised and decentralised (Dec_) envs together: {env_ids}")
+    pad_turbines = bool(env_kwargs.get("pad_turbines", False))
+    if pad_turbines and decentralized:
+        raise ValueError(f"pad_turbines is not supported by the decentralised (Dec_) envs: {env_ids}")
     layouts = []
     for e, (_dec, name, simulator) in zip(env_ids, parsed):
         case = get_case(name, simulator)
         validate_case(e, case)
         layouts.append({"num_turbines": case.num_turbines, "xcoords": case.xcoords, "ycoords": case.ycoords,
                         "dt": case.dt, "t_init": case.t_init})
-    layout_pool(layouts)  # same turbine count, dt and t_init, checked before any device work
+    layout_pool(layouts, pad_turbines)  # same turbine count (unless padded), dt and t_init, checked before any device work
     if not isinstance(controls, dict):
         controls = get_default_control(controls)
     case = layouts[0]

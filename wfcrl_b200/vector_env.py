@@ -27,14 +27,16 @@ from .rewards import DoNothingReward, RewardShaper
 _OBS_BOUNDS = {"wind_speed": (3.0, 28.0), "wind_direction": (0.0, 360.0)}
 
 
-def layout_pool(layout) -> List[Dict]:
-    """The farm cases of ``layout``: one layout name or dict, or a list of them.  The layouts of a pool must share the
-    turbine count (the observation and action spaces), ``dt`` and ``t_init``; raises ValueError otherwise."""
+def layout_pool(layout, pad_turbines: bool = False) -> List[Dict]:
+    """The farm cases of ``layout``: one layout name or dict, or a list of them.  The layouts of a pool must share
+    ``dt`` and ``t_init`` and, unless ``pad_turbines``, the turbine count (the observation and action spaces); raises
+    ValueError otherwise."""
     items = list(layout) if isinstance(layout, (list, tuple)) else [layout]
     if not items:
         raise ValueError("layout list is empty")
     cases = [get_layout(c) if isinstance(c, str) else c for c in items]
-    for key, default in (("num_turbines", None), ("dt", 60), ("t_init", None)):
+    keys = (("dt", 60), ("t_init", None)) if pad_turbines else (("num_turbines", None), ("dt", 60), ("t_init", None))
+    for key, default in keys:
         values = [c.get(key, default) for c in cases]
         if any(v != values[0] for v in values):
             raise ValueError(f"the layouts of one batch must share {key}, got {values}")
@@ -53,7 +55,13 @@ class VecWindFarmEnv:
     ``layout_assignment="cycle"`` the env of global id ``g = env_id_offset + b`` runs layout ``g % L`` for good; with
     ``"sample"`` every reset draws the env's layout uniformly (in the library for ``reset(seed=None)`` and auto-resets,
     with numpy's ``default_rng((seed + g, 2))`` for ``reset(seed=seed)``).  ``reset(options={"layout": ids})`` sets the
-    layout of the reset envs explicitly; ``layout_ids`` returns the current ones."""
+    layout of the reset envs explicitly; ``layout_ids`` returns the current ones.
+
+    MIXED TURBINE COUNTS: with ``pad_turbines=True`` the layouts may differ in turbine count.  ``T`` is then the largest
+    count; an env whose farm has n turbines uses columns 0..n-1 of every [B, T] array, and the other columns are padding:
+    actions there are ignored and observations, power and load read 0.  The observation gains ``"turbine_mask"`` (bool
+    [B, T], True on the env's turbines), ``turbine_counts`` gives the counts per env, and each env's reward is its own
+    farm's (the mean over its n turbines).  Not available with ``multi_agent``."""
 
     metadata = {"name": "vectorized-windfarm"}
 
@@ -63,8 +71,10 @@ class VecWindFarmEnv:
                  start_iter: int = 0, auto_reset: bool = True, multi_agent: bool = False, env_id_offset: int = 0,
                  wind_time_series: Optional[Union[str, np.ndarray]] = None, exact_host_trig: Optional[bool] = None,
                  turbulence_intensity_range: Optional[tuple] = None, copy_outputs: bool = False,
-                 layout_assignment: str = "cycle"):
-        cases = layout_pool(layout)
+                 layout_assignment: str = "cycle", pad_turbines: bool = False):
+        if pad_turbines and multi_agent:
+            raise ValueError("pad_turbines is not supported by the multi-agent (Dec_) envs: their agents are the turbines")
+        cases = layout_pool(layout, pad_turbines)
         if layout_assignment not in ("cycle", "sample"):
             raise ValueError(f"layout_assignment must be 'cycle' or 'sample', got {layout_assignment!r}")
         if layout_assignment == "sample" and wind_time_series is not None:
@@ -76,6 +86,9 @@ class VecWindFarmEnv:
         self.farm_cases = cases
         self.layout_assignment = layout_assignment
         self.num_envs = int(num_envs)
+        self.pad_turbines = bool(pad_turbines)
+        if self.pad_turbines:
+            case = max(cases, key=lambda c: c["num_turbines"])  # the handle is created with the largest farm
         self.num_turbines = case["num_turbines"]
         self.dt = case.get("dt", 60)
         controls = dict(controls or {"yaw": (-40, 40, 5)})
@@ -108,7 +121,10 @@ class VecWindFarmEnv:
                                    continuous_control=continuous_control, multi_agent=multi_agent)
         self.device = self.backend.device
         if len(cases) > 1:
-            self.backend.set_layouts([c["xcoords"] for c in cases], [c["ycoords"] for c in cases])
+            if self.pad_turbines:
+                self.backend.set_mixed_layouts([c["xcoords"] for c in cases], [c["ycoords"] for c in cases])
+            else:
+                self.backend.set_layouts([c["xcoords"] for c in cases], [c["ycoords"] for c in cases])
             if layout_assignment == "cycle":
                 self.backend.assign_layouts(None, (self.env_id_offset + np.arange(self.num_envs)) % len(cases))
         if layout_assignment == "sample":
@@ -120,9 +136,10 @@ class VecWindFarmEnv:
         self.single_observation_space = spaces.Dict(OrderedDict([
             ("yaw", spaces.Box(ones * lo, ones * hi, shape=(T,))),
             ("freewind_measurements", spaces.Box(np.array([3, 0], np.float32), np.array([28, 360], np.float32), shape=(2,))),
-            ("wind_speed", spaces.Box(ones * 3, ones * 28, shape=(T,))),
+            # padding columns read 0
+            ("wind_speed", spaces.Box(ones * (0 if self.pad_turbines else 3), ones * 28, shape=(T,))),
             ("wind_direction", spaces.Box(ones * 0, ones * 360, shape=(T,))),
-        ]))
+        ] + ([("turbine_mask", spaces.MultiDiscrete([2] * T))] if self.pad_turbines else [])))
         self.action_space = self.single_action_space
         self.observation_space = self.single_observation_space
         self._gen = torch.Generator(device=self.device)  # time-series start offsets of in-loop resets only
@@ -146,6 +163,15 @@ class VecWindFarmEnv:
         self._arm_autoreset()
         self._zeros_bool = torch.zeros(self.num_envs, dtype=torch.bool, device=self.device)
         self._needs_reset = True
+        self._turbine_mask = None
+        if self.pad_turbines:
+            self._refresh_turbine_mask()
+
+    def _refresh_turbine_mask(self):
+        """Rebuild ``"turbine_mask"`` from the envs' turbine counts; called where layouts can change (construction, reset,
+        and auto-resets that draw layouts), so that a plain step costs no host round trip."""
+        counts = torch.as_tensor(self.backend.get_state("turbine_count"), device=self.device)
+        self._turbine_mask = torch.arange(self.num_turbines, device=self.device)[None, :] < counts[:, None]
 
     def _arm_autoreset(self):
         """In-kernel auto-reset (wf_set_autoreset): the truncating step itself zeroes the env's state and marks it; one
@@ -188,8 +214,11 @@ class VecWindFarmEnv:
     # -- API ------------------------------------------------------------------------------------------------------
     def _obs(self, out):
         c = (lambda t: t.clone()) if self.copy_outputs else (lambda t: t)
-        return OrderedDict([("yaw", c(out["yaw"])), ("freewind_measurements", c(out["freewind"])),
-                            ("wind_speed", c(out["wind_speed"])), ("wind_direction", c(out["wind_direction"]))])
+        obs = OrderedDict([("yaw", c(out["yaw"])), ("freewind_measurements", c(out["freewind"])),
+                           ("wind_speed", c(out["wind_speed"])), ("wind_direction", c(out["wind_direction"]))])
+        if self.pad_turbines:
+            obs["turbine_mask"] = self._turbine_mask  # replaced, never written in place, by _refresh_turbine_mask
+        return obs
 
     def reset(self, seed: Optional[int] = None, options: Optional[dict] = None, env_ids=None):
         """Reset all (or ``env_ids``) envs.  ``options`` may carry ``wind_speed`` / ``wind_direction`` (scalars or
@@ -253,6 +282,8 @@ class VecWindFarmEnv:
             self._countdowns = []
         self._countdowns = sorted(set(self._countdowns) | {self.max_num_steps - 1})
         self._needs_reset = False
+        if self.pad_turbines:
+            self._refresh_turbine_mask()
         return self._obs(out)
 
     def step(self, action):
@@ -288,6 +319,8 @@ class VecWindFarmEnv:
                 # the step kernel has already reset the truncated envs' state and marked them: wind draw + geometry +
                 # warm-up solve of the marked envs, no host round trip
                 out = self.backend.autoreset_finish(self.start_iter + 1)
+                if self.pad_turbines and self.layout_assignment == "sample":
+                    self._refresh_turbine_mask()
             else:  # time series: the wind generator restarts at a random row (interface.py:517)
                 start = torch.randint(0, self._series.shape[0], (self.num_envs,), device=self.device, generator=self._gen)
                 self._series_pos = torch.where(truncated, start, self._series_pos)
@@ -302,6 +335,11 @@ class VecWindFarmEnv:
     def layout_ids(self):
         """Index into the layout list of the layout every env currently runs (int32 [B], device copy)."""
         return torch.as_tensor(self.backend.get_state("layout_id"), device=self.device)
+
+    @property
+    def turbine_counts(self):
+        """Turbine count of the layout every env currently runs (int32 [B], device copy)."""
+        return torch.as_tensor(self.backend.get_state("turbine_count"), device=self.device)
 
     @property
     def episode_returns(self):
