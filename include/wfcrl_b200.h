@@ -225,6 +225,30 @@ int wf_autoreset_finish(WfHandle h, int32_t warmup_solves, const WfStepOut* out,
 int wf_update_command(WfHandle h, const double* d_yaw, const WfStepOut* out, void* stream);
 
 /*
+ * CANDIDATE EVALUATION.  Solve K candidate yaw settings per env in its CURRENT wind, TI, layout and geometry, without
+ * changing the handle's state ("what would the farm produce with these yaws?": yaw optimisation, model-based control).
+ *   d_yaw:       DEVICE double [B][K][T] absolute yaw in degrees (used as given, like wf_update_command: no clipping)
+ *   d_power:     DEVICE real   [B][K][T] per-turbine power in W (interface-mode units, interface.py:623)
+ *   d_ambiguous: DEVICE uint8  [B][K] or NULL: 1 = this candidate was re-solved by the FP64 kernel (strict FP32 handle;
+ *                always 0 on other handles)
+ * WF_KERNEL_FAST handles only.  Asynchronous on `stream`.
+ *  - State: no state array changes -- none of the names wf_get_state accepts (yaw, "ambiguous", num_iter, the episode sums,
+ *    nonfinite, ...), nor the re-solve list of the step path.  The next wf_step gives the same result bit for bit as if the
+ *    evaluation had not happened.
+ *  - Results: candidate (b, k) gives, bit for bit, the `power` row that wf_update_command with that yaw would write on this
+ *    handle in its current state, including candidates that a strict FP32 handle flags and re-solves in FP64.
+ *  - Layout pools of mixed counts: an env of n < T turbines ignores columns n..T-1 of its candidates (they may hold NaN)
+ *    and writes 0 there.  Multi-agent handles evaluate like any other (there is no transition).
+ *  - Launches: one per call, plus one FP64 re-solve launch on a strict FP32 handle (counted in wf_launch_count).
+ *  - Scratch: the first call with a larger B*K than before allocates the evaluation scratch, synchronously; later calls
+ *    with no larger K allocate nothing.
+ *  - Envs marked by the in-kernel auto-reset must be finished (wf_autoreset_finish) first.
+ * Refused with WF_ERR_INVALID before any work: WF_KERNEL_BASIC handles (and so the 5x5 grid), K < 1, NULL d_yaw or
+ * d_power, and B*K > 2^31 - 1 (the kernels' index type).
+ */
+int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, uint8_t* d_ambiguous, void* stream);
+
+/*
  * End-to-end convenience for hosts without device buffers: `h_action` (float [B][T]) in, wf_step, every non-NULL
  * member of `h_out` out, synchronous.  Two routes, same results bit for bit:
  *   - staged: cudaMemcpyAsync into device staging owned by the handle, 6 env chunks on 6 streams so the copies of one

@@ -96,6 +96,7 @@ class FlorisBatch:
                                             ("yaw", "wind_speed", "wind_direction", "power", "load", "reward",
                                              "freewind", "truncated")])
         self._host = None
+        self.eval_capacity = 0  # largest K evaluate_yaw has run with (its output buffers and the library scratch hold that)
 
     # ------------------------------------------------------------------------------------------------------
     def close(self):
@@ -231,6 +232,28 @@ class FlorisBatch:
                 raise ValueError(f"yaw must have shape ({self.B}, {self.T}), got {tuple(yaw.shape)}")
         _lib.check(self.lib.wf_update_command(self.handle, _ptr(yaw), C.byref(self._out_struct), self._stream()))
         return self.out
+
+    def evaluate_yaw(self, yaw: torch.Tensor) -> Dict[str, torch.Tensor]:
+        """Per-turbine power (W) of K candidate yaw settings per env, in each env's current wind, TI and layout, without
+        changing any state (``wf_evaluate_yaw``).  ``yaw``: contiguous float64 CUDA tensor [B, K, T], absolute degrees, not
+        clipped; padding columns of a mixed-count pool are ignored.  Returns ``{"power": [B, K, T], "ambiguous": bool [B, K]}``
+        (1 = re-solved in FP64 on a strict FP32 handle), views of buffers owned by the batch that the next call overwrites.
+        Asynchronous; the first call with a larger K than before allocates, synchronously."""
+        if not (torch.is_tensor(yaw) and yaw.dtype == torch.float64 and yaw.is_cuda and yaw.is_contiguous()):
+            raise TypeError("yaw must be a contiguous float64 CUDA tensor of shape [B, K, T]")
+        if yaw.dim() != 3 or yaw.shape[0] != self.B or yaw.shape[2] != self.T or yaw.shape[1] < 1:
+            raise ValueError(f"yaw must have shape ({self.B}, K, {self.T}) with K >= 1, got {tuple(yaw.shape)}")
+        K = int(yaw.shape[1])
+        power_buf, amb_buf = getattr(self, "_eval_power", None), getattr(self, "_eval_amb", None)
+        if K > self.eval_capacity:
+            power_buf = torch.zeros(self.B * K * self.T, dtype=self.real, device=self.device)
+            amb_buf = torch.zeros(self.B * K, dtype=torch.uint8, device=self.device)
+        power = power_buf[: self.B * K * self.T].view(self.B, K, self.T)
+        amb = amb_buf[: self.B * K].view(self.B, K)
+        _lib.check(self.lib.wf_evaluate_yaw(self.handle, _ptr(yaw), K, _ptr(power), _ptr(amb), self._stream()))
+        if K > self.eval_capacity:  # the library holds scratch for this K now
+            self._eval_power, self._eval_amb, self.eval_capacity = power_buf, amb_buf, K
+        return {"power": power, "ambiguous": amb.view(torch.bool)}
 
     def step_host(self, action_host: torch.Tensor, fields=("yaw", "wind_speed", "wind_direction", "reward",
                                                            "truncated", "power", "load", "freewind")):

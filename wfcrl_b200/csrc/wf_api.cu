@@ -70,6 +70,11 @@ struct WfHandle_t {
     double* d_pool = nullptr;  // the layout pool in one allocation: [L][T] x, [L][T] y, [L][2] centres, [L] int32 turbine
                                // counts (WfModel.layout_*)
     std::vector<int> layout_n;  // host copy of the pool's turbine counts
+    // wf_evaluate_yaw scratch, sized for the largest B*K evaluated so far: the evaluation fix list [eval_cap] and its 4
+    // counters in one allocation, and on a gathering FP64 handle one (v, w) scratch row per candidate [eval_cap][9T]
+    int eval_cap = 0;
+    int* d_eval_fix = nullptr;
+    double2* d_eval_vwg = nullptr;
 };
 
 template <typename T> static int dev_alloc(WfHandle_t* h, T** p, size_t n) {
@@ -193,6 +198,8 @@ int wf_destroy(WfHandle h) {
         if (ev) cudaEventDestroy(ev);
     if (h->h_fix_rec) cudaFreeHost(h->h_fix_rec);
     if (h->h_fix_n) cudaFreeHost(h->h_fix_n);
+    if (h->d_eval_fix) cudaFree(h->d_eval_fix);
+    if (h->d_eval_vwg) cudaFree(h->d_eval_vwg);
     delete h;
     return WF_OK;
 }
@@ -594,6 +601,66 @@ int wf_update_command(WfHandle h, const double* d_yaw, const WfStepOut* out, voi
     CUDA_TRY(cudaSetDevice(h->device));
     TRY(launch_step(h, WF_MODE_INTERFACE, nullptr, nullptr, d_yaw, to_ptrs(out), (cudaStream_t)stream));
     return mark_async(h, (cudaStream_t)stream);
+}
+
+// (Re)allocate the evaluation scratch for `cap` candidates.  Synchronous on both sides: no queued evaluation may still use the
+// old scratch, and the zeroing of the new one (cudaMemset runs on the legacy default stream, which a caller's non-blocking
+// stream does not wait for) is complete before the first evaluation kernel reads the counters.
+static int eval_reserve(WfHandle h, int cap) {
+    CUDA_TRY(cudaDeviceSynchronize());
+    if (h->d_eval_fix) cudaFree(h->d_eval_fix);
+    if (h->d_eval_vwg) cudaFree(h->d_eval_vwg);
+    h->d_eval_fix = nullptr;
+    h->d_eval_vwg = nullptr;
+    h->eval_cap = 0;
+    const size_t fix_bytes = sizeof(int) * ((size_t)cap + 4);
+    cudaError_t e = cudaMalloc(&h->d_eval_fix, fix_bytes);
+    if (e == cudaSuccess) e = cudaMemset(h->d_eval_fix, 0, fix_bytes);
+    if (e == cudaSuccess && wf_fast64_gathers(h->model, h->st)) {
+        const size_t vwg_bytes = sizeof(double2) * 9 * (size_t)h->model.T * (size_t)cap;
+        e = cudaMalloc(&h->d_eval_vwg, vwg_bytes);
+        if (e == cudaSuccess) e = cudaMemset(h->d_eval_vwg, 0, vwg_bytes);
+    }
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return set_err(e == cudaErrorMemoryAllocation ? WF_ERR_NOMEM : WF_ERR_CUDA,
+                       std::string("evaluation scratch: ") + cudaGetErrorString(e));
+    }
+    h->eval_cap = cap;
+    return WF_OK;
+}
+
+int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, uint8_t* d_ambiguous, void* stream) {
+    if (!h) return set_err(WF_ERR_INVALID, "NULL handle");
+    if (h->cfg.kernel != WF_KERNEL_FAST)
+        return set_err(WF_ERR_INVALID, "wf_evaluate_yaw needs the warp-per-env kernels (WF_KERNEL_FAST)");
+    if (K < 1) return set_err(WF_ERR_INVALID, "K (candidates per env) must be >= 1");
+    if (!d_yaw || !d_power) return set_err(WF_ERR_INVALID, "NULL argument");
+    const int64_t BK = (int64_t)h->model.B * K;
+    if (BK > (int64_t)INT32_MAX)
+        return set_err(WF_ERR_INVALID, "num_envs * K = " + std::to_string(BK) + " candidates exceed the kernels' 32-bit index "
+                                       "(at most 2^31 - 1 per call)");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (BK > h->eval_cap) TRY(eval_reserve(h, (int)BK));
+    const WfEvalArgs ev = {K, h->d_eval_fix, h->d_eval_fix + h->eval_cap, d_ambiguous, h->d_eval_vwg};
+    // the route of a step in the handle's current state: a stale vortex table is not read
+    const bool use_vtab = !h->vtab_stale;
+    cudaError_t e;
+    if (h->cfg.precision == WF_PREC_F64) {
+        e = wf_launch_eval_fast64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_power, st);
+        h->launches += 1;
+    } else {
+        e = wf_launch_eval_fast(h->fast_baked, h->model, h->fast, h->st, ev, d_yaw, d_power, st);
+        h->launches += 1;
+        if (e == cudaSuccess && is_strict_f32(h)) {
+            e = wf_launch_eval_fixup64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_power, st);
+            h->launches += 1;
+        }
+    }
+    if (e != cudaSuccess) return set_err(WF_ERR_CUDA, std::string("evaluation kernel launch: ") + cudaGetErrorString(e));
+    return mark_async(h, st);
 }
 
 // Device alias of a host pointer when it is page-locked memory the GPU can address (cudaHostAlloc / cudaHostRegister

@@ -124,16 +124,21 @@ struct wf_true_tag { static constexpr bool value = true; };
 struct wf_false_tag { static constexpr bool value = false; };
 
 // generic instantiation: 12 is a lower bound for the register allocator; 16 envs per SM are reached
-template <bool BAKED>
+// EVAL (wf_evaluate_yaw): CTA c solves candidate c of env c / K in interface mode with the yaw row c of `yaw_cmd`, writes power
+// row c of `out.power` and nothing else, and hands a flagged candidate to the evaluation fix list (wf_device.cuh: WfEvalArgs)
+template <bool BAKED, bool EVAL = false>
 __global__ void __launch_bounds__(32, BAKED ? 16 : 12)
-wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
+wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
                     const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
-                    const double* __restrict__ yaw_cmd, const WfOutPtrs out) {
-    const int b = blockIdx.x + env_begin;
+                    const double* __restrict__ yaw_cmd, const WfOutPtrs out, const WfEvalArgs ev) {
+    int b;
+    if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
+    const int mode = EVAL ? (int)WF_MODE_INTERFACE : mode_;
     if (mask && !mask[b]) return;
     const int T = m.T;
     const int lane = threadIdx.x;
     const size_t row = (size_t)b * T;
+    const size_t orow = EVAL ? (size_t)blockIdx.x * T : row;  // row of the yaw command and of the outputs
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const SmemView sm = carve(smem_raw, T);  // sized by T: every env of the handle reserves the same shared memory
     // the env's turbine count: the one loop bound below.  Columns n..T-1 of its rows are padding (wf_device.cuh)
@@ -158,8 +163,8 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
             s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
             s.yaw[row + tt] = (double)ynew;
         } else if (mode == WF_MODE_INTERFACE && yaw_cmd) {
-            const double y = yaw_cmd[row + tt];
-            s.yaw[row + tt] = y;
+            const double y = yaw_cmd[orow + tt];
+            if (!EVAL) s.yaw[row + tt] = y;
             ynew = (float)y;
         } else {
             ynew = (float)s.yaw[row + tt];
@@ -543,6 +548,10 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
             for (int q = 0; q < 4; ++q) loads[q] *= 1e7f;
         }
         const int orig = sm.ordr[tt];
+        if (EVAL) {  // the power is written once the candidate is known not to be flagged (below)
+            sm.tifin[tt] = p_out;
+            continue;
+        }
         float yv = sm.ynew[orig];
         if (mode == WF_MODE_WARMUP) {  // start state is clipped to the observation space (mdp.py:263-266)
             wsl = fclamp(wsl, 3.f, 28.f);
@@ -562,6 +571,17 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
         rsum_l += __shfl_xor_sync(0xffffffffu, rsum_l, sft);
     }
     const bool any_flag = __any_sync(0xffffffffu, flagged);
+    if constexpr (EVAL) {  // no state is written: the flag and the power row of the candidate only
+        if (lane == 0 && ev.amb) ev.amb[blockIdx.x] = (uint8_t)any_flag;
+        if (any_flag && strict) {  // re-solved by the evaluation instantiation of wf_fixup64_kernel
+            if (lane == 0) ev.fix_list[atomicAdd(&ev.fix_count[0], 1)] = blockIdx.x;
+            return;
+        }
+        float* const pw_out = (float*)out.power + orow;
+        for (int tt = lane; tt < n; tt += 32) pw_out[sm.ordr[tt]] = sm.tifin[tt];
+        for (int tt = n + lane; tt < T; tt += 32) pw_out[tt] = 0.f;
+        return;
+    }
     if (lane == 0 && s.amb) s.amb[b] = (uint8_t)any_flag;
     if (any_flag && strict) {
         // the FP64 re-solve (wf_fixup64_kernel, next launch on this stream) redoes this env from the committed yaw state and
@@ -619,7 +639,8 @@ wf_step_fast_kernel(const int mode, const int env_begin, const WfModel m, const 
 }  // namespace
 
 cudaError_t wf_configure_fast_kernels() {
-    for (auto k : {wf_step_fast_kernel<true>, wf_step_fast_kernel<false>}) {
+    for (auto k : {wf_step_fast_kernel<true>, wf_step_fast_kernel<false>, wf_step_fast_kernel<true, true>,
+                   wf_step_fast_kernel<false, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -633,8 +654,24 @@ static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& 
                                  const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
                                  const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
     wf_step_fast_kernel<BAKED><<<env_count, 32, fast_smem_bytes(m.T), stream>>>(mode, env_begin, m, fc, s, d_mask, d_action,
-                                                                               d_yaw_cmd, out);
+                                                                               d_yaw_cmd, out, WfEvalArgs{});
     return cudaGetLastError();
+}
+
+template <bool BAKED>
+static cudaError_t launch_eval_t(const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
+                                 const double* d_yaw, void* d_power, cudaStream_t stream) {
+    WfOutPtrs out = {};
+    out.power = d_power;
+    wf_step_fast_kernel<BAKED, true><<<(unsigned)m.B * (unsigned)ev.K, 32, fast_smem_bytes(m.T), stream>>>(
+        WF_MODE_INTERFACE, 0, m, fc, s, nullptr, nullptr, d_yaw, out, ev);
+    return cudaGetLastError();
+}
+
+cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
+                                const double* d_yaw, void* d_power, cudaStream_t stream) {
+    return baked ? launch_eval_t<true>(m, fc, s, ev, d_yaw, d_power, stream)
+                 : launch_eval_t<false>(m, fc, s, ev, d_yaw, d_power, stream);
 }
 
 cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,

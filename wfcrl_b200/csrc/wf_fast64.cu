@@ -8,6 +8,7 @@
 //                                 deficit queue) for handles without a vortex table;
 //   wf_fixup64_kernel<W>          W warps per env, built for latency: a chain warp evaluates the sources' scalar chains back to
 //                                 back while W-1 worker warps apply the previous source to its targets (named barriers).
+// and their candidate-evaluation forms (wf_evaluate_yaw): wf_step_fast64_kernel<GATHER, true> and wf_fixup64_eval_kernel<W>.
 //
 // Everything is evaluated in double precision and every simplification of wf_fast.cu that would be visible at the 1e-9 level
 // is dropped:
@@ -187,16 +188,19 @@ __device__ __forceinline__ void load_row12(const double* __restrict__ p, double*
 //          12 envs share an SM instead of 9.
 // OutT = type of the caller's output buffers (double for an FP64 handle, float for the re-solve on an FP32 handle).  FIX = re-solve: the FP32 kernel has already applied the action (yaw and
 // accumulators are committed) but none of the per-env epilogue state, which is committed here.
-template <int W, typename OutT, bool FIX, bool GATHER = false>
+// EVAL = candidate evaluation (wf_evaluate_yaw): candidate `cand` of env b, solved in interface mode with the yaw row `cand` of
+// `yaw_cmd`; its power goes to row `cand` of out.power, its flag to ev.amb[cand] (FIX: 1, else 0), and no state is written.
+template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false>
 __device__ __forceinline__ void solve_env64(const int b, const int mode, const bool use_vtab, const WfModel& m,
                                             const WfFastConst64& fc, const WfState& s, const float* __restrict__ action,
                                             const double* __restrict__ yaw_cmd, const WfOutPtrs& out,
-                                            float* __restrict__ rec = nullptr) {
+                                            float* __restrict__ rec, const WfEvalArgs& ev, const int cand) {
     const int T = m.T;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NT = 32 * W;
     auto csync = [] { if (W == 1) __syncwarp(); else __syncthreads(); };
     const size_t row = (size_t)b * T;
+    const size_t orow = EVAL ? (size_t)cand * T : row;  // row of the yaw command and of the outputs
     // the env's turbine count, the bound of every loop below; columns n..T-1 of its rows are padding (wf_device.cuh).
     // Shared memory and the table's row strides stay those of T.
     const int n = s.turbine_count[b];
@@ -204,8 +208,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     static_assert(!GATHER || W == 1, "the gather form is the one-warp throughput kernel");
     const SmemView64 sm = carve64(smem_raw64, T, GATHER);
     // (v, w) per rotor point: shared memory, or the env's global scratch (cache-global accesses: lanes exchange values
-    // through it between __syncwarp()s)
-    double2* const vwp = GATHER ? s.vwg + (size_t)b * 9 * T : sm.vw;
+    // through it between __syncwarp()s); an evaluation has a row per candidate, as the K candidates of an env run at once
+    double2* const vwp = GATHER ? (EVAL ? ev.vwg + (size_t)cand * 9 * T : s.vwg + (size_t)b * 9 * T) : sm.vw;
     auto vw_ld = [&](const int q) -> double2 { return GATHER ? __ldcg(vwp + q) : vwp[q]; };
     auto vw_st = [&](const int q, const double2 v) { if (GATHER) __stcg(vwp + q, v); else vwp[q] = v; };
     // vortex table of this env (wf_device.cuh), or NULL: evaluate every pair directly
@@ -217,7 +221,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     if (mode == WF_MODE_ENV) nm = s.num_moves[b] + 1;
     for (int tt = tid; tt < n; tt += NT) {
         double ynew;
-        if (!FIX && mode == WF_MODE_ENV) {
+        if (!FIX && !EVAL && mode == WF_MODE_ENV) {
             float a = action[row + tt];
             const float acc = s.acc[row + tt];
             const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
@@ -231,9 +235,9 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
             ynew = (double)y1;
             s.yaw[row + tt] = ynew;
-        } else if (!FIX && mode == WF_MODE_INTERFACE && yaw_cmd) {
-            ynew = yaw_cmd[row + tt];
-            s.yaw[row + tt] = ynew;
+        } else if ((!FIX || EVAL) && mode == WF_MODE_INTERFACE && yaw_cmd) {
+            ynew = yaw_cmd[orow + tt];
+            if (!EVAL) s.yaw[row + tt] = ynew;
         } else {
             ynew = s.yaw[row + tt];
         }
@@ -796,7 +800,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             wdl = dclamp(wdl, 0.0, 360.0);
             yv = dclamp(yv, (double)m.yaw_lo_f, (double)m.yaw_hi_f);
         }
-        const size_t o = row + orig;
+        const size_t o = orow + orig;
         if (out.yaw) ((OutT*)out.yaw)[o] = (OutT)yv;
         if (out.wind_speed) ((OutT*)out.wind_speed)[o] = (OutT)wsl;
         if (out.wind_direction) ((OutT*)out.wind_direction)[o] = (OutT)wdl;
@@ -814,7 +818,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     }
 #pragma unroll 1
     for (int tt = n + lane; tt < T; tt += 32) {  // padding columns: no stale value of an earlier layout shows
-        const size_t o = row + tt;
+        const size_t o = orow + tt;
         if (out.yaw) ((OutT*)out.yaw)[o] = (OutT)0;
         if (out.wind_speed) ((OutT*)out.wind_speed)[o] = (OutT)0;
         if (out.wind_direction) ((OutT*)out.wind_direction)[o] = (OutT)0;
@@ -828,6 +832,15 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             r[tt] = 0.f; r[T + tt] = 0.f; r[2 * T + tt] = 0.f; r[3 * T + tt] = 0.f;
             r[4 * T + 4 * tt] = 0.f; r[4 * T + 4 * tt + 1] = 0.f; r[4 * T + 4 * tt + 2] = 0.f; r[4 * T + 4 * tt + 3] = 0.f;
         }
+    }
+    // nothing of the epilogue state: no counters, no reward, no auto-reset.  The test of K (always > 0) keeps the code below
+    // alive in the evaluation instantiation, so that the compiler makes the same floating-point contractions above as in the
+    // step instantiation and a candidate's power equals the step's bit for bit.  With a plain `return` the sums of the power
+    // chain fused differently (1e-15 off the step, DESIGN.md section 5b).  This rests on the compiler's choices:
+    // tests/test_evaluate_yaw_gpu.py::test_equals_interface_mode (f64 modes) catches a compiler that makes others.
+    if (EVAL && ev.K > 0) {
+        if (lane == 0 && ev.amb) ev.amb[cand] = FIX ? 1 : 0;
+        return;
     }
 #pragma unroll
     for (int sft = 16; sft > 0; sft >>= 1) {
@@ -874,14 +887,16 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
 // sub-partition with two others (12 per SM), one of 128 registers with three (16 per SM; 12-48 bytes of spills).  The kernels
 // are latency-bound, throughput grows with the resident envs (measured on Turb32_Row5: 6 per SM 4.9 M env-steps/s, 9: 6.2 M,
 // 12: 7.6 M, 16: 8.2 M); at 80 turbines shared memory holds 14 envs of the gather kernel per SM (9 of the scatter kernel).
-template <bool GATHER>
+// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw)
+template <bool GATHER, bool EVAL = false>
 __global__ void __launch_bounds__(32, 16)
 wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                       const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
-                      const double* __restrict__ yaw_cmd, const WfOutPtrs out) {
-    const int b = blockIdx.x + env_begin;
+                      const double* __restrict__ yaw_cmd, const WfOutPtrs out, const WfEvalArgs ev) {
+    int b;
+    if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
     if (mask && !mask[b]) return;
-    solve_env64<1, double, false, GATHER>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out);
+    solve_env64<1, double, false, GATHER, EVAL>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
 }
 
 // Re-solve, in FP64, of the envs an FP32 launch flagged (their ids sit in s.fix_list[0, n), n in s.fix_count[0]); launched
@@ -895,7 +910,7 @@ wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __
     const int rec_len = WF_FIX_REC_HDR + 8 * m.T;  // header (env id, reward, freewind x2, truncated) + yaw, ws, wd, power, load x4
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
         solve_env64<W, float, true>(s.fix_list[k], mode, use_vtab, m, fc, s, nullptr, nullptr, out,
-                                    (rec && k < rec_cap) ? rec + (size_t)k * rec_len : nullptr);
+                                    (rec && k < rec_cap) ? rec + (size_t)k * rec_len : nullptr, WfEvalArgs{}, 0);
         __syncthreads();
     }
     if (threadIdx.x == 0) {
@@ -908,11 +923,35 @@ wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __
     }
 }
 
+// Evaluation instantiation of the re-solve (wf_evaluate_yaw): the candidates an evaluation launch flagged (ev.fix_list /
+// ev.fix_count, candidate c = env c / K), with the yaw rows of `yaw_cmd`; they write their power row and flag and commit
+// nothing.  A kernel of its own rather than a flag of wf_fixup64_kernel, whose parameter list (and so code) stays as it was.
+template <int W>
+__global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
+wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc, const WfState s,
+                       const WfOutPtrs out, const double* __restrict__ yaw_cmd, const WfEvalArgs ev) {
+    const int n = *(volatile int*)&ev.fix_count[0];
+    for (int k = blockIdx.x; k < n; k += gridDim.x) {
+        const int c = ev.fix_list[k];
+        solve_env64<W, float, true, false, true>(c / ev.K, mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {  // the last CTA to leave re-arms the evaluation counters
+        __threadfence();
+        if (atomicAdd(&ev.fix_count[1], 1) == (int)gridDim.x - 1) {
+            ev.fix_count[2] = n;
+            ev.fix_count[0] = 0;
+            ev.fix_count[1] = 0;
+        }
+    }
+}
+
 }  // namespace
 
 // Dynamic shared memory up to 100 KB for every FP64 kernel; the step kernels also prefer the largest shared-memory carveout.
 cudaError_t wf_configure_fast64_kernels() {
-    for (auto k : {wf_step_fast64_kernel<false>, wf_step_fast64_kernel<true>}) {
+    for (auto k : {wf_step_fast64_kernel<false>, wf_step_fast64_kernel<true>, wf_step_fast64_kernel<false, true>,
+                   wf_step_fast64_kernel<true, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -922,54 +961,97 @@ cudaError_t wf_configure_fast64_kernels() {
         const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e != cudaSuccess) return e;
     }
+    for (auto k : {wf_fixup64_eval_kernel<1>, wf_fixup64_eval_kernel<2>, wf_fixup64_eval_kernel<4>, wf_fixup64_eval_kernel<8>}) {
+        const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+        if (e != cudaSuccess) return e;
+    }
     return cudaSuccess;
 }
 
-template <int W>
+template <int W, bool EVAL>
 static cudaError_t launch_fixup_t(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                  const WfOutPtrs& out, int grid, float* d_rec, int rec_cap, cudaStream_t stream) {
-    wf_fixup64_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_rec, rec_cap);
+                                  const WfOutPtrs& out, int grid, float* d_rec, int rec_cap, const double* d_yaw,
+                                  const WfEvalArgs& ev, cudaStream_t stream) {
+    if (EVAL)
+        wf_fixup64_eval_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_yaw, ev);
+    else
+        wf_fixup64_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_rec, rec_cap);
     return cudaGetLastError();
 }
 
-cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                              const WfOutPtrs& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream) {
+// W and the grid of a re-solve launch behind a step (or evaluation) launch of `count` CTAs
+template <bool EVAL>
+static cudaError_t launch_fixup_sized(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
+                                      const WfOutPtrs& out, int count, float* d_rec, int rec_cap, const double* d_yaw,
+                                      const WfEvalArgs& ev, cudaStream_t stream) {
     // The launch is latency-bound while the flagged envs (1-2 % of the batch) are fewer than the CTAs the GPU holds at once,
     // and each env is a sequential sweep over its turbines: W warps per env cover 10 W targets in one fused pass per source.
     // So: as many warps as the farm can use (T / 10), fewer when the batch is large enough for the flagged envs to outnumber
     // the resident CTAs (148 at W = 8, 296 at W = 4, 592 at W = 2, 1184 at W = 1 on a B200: 8 warps of ~196 registers per SM).
     int w = m.T > 40 ? 8 : (m.T > 20 ? 4 : (m.T > 10 ? 2 : 1));
-    const int expected = env_count / 64 + 1;  // ~1.5 % of the envs
+    const int expected = count / 64 + 1;  // ~1.5 % of the envs
     while (w > 1 && expected > 148 * 8 / w) w >>= 1;
     const int resident = 148 * 8 / w;  // two ~196-register warps per SM sub-partition = 8 warps per SM
-    const int grid = env_count < resident ? env_count : resident;
+    const int grid = count < resident ? count : resident;
     switch (w) {
-        case 8: return launch_fixup_t<8>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
-        case 4: return launch_fixup_t<4>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
-        case 2: return launch_fixup_t<2>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
-        default: return launch_fixup_t<1>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, stream);
+        case 8: return launch_fixup_t<8, EVAL>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, d_yaw, ev, stream);
+        case 4: return launch_fixup_t<4, EVAL>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, d_yaw, ev, stream);
+        case 2: return launch_fixup_t<2, EVAL>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, d_yaw, ev, stream);
+        default: return launch_fixup_t<1, EVAL>(mode, use_vtab, m, fc, s, out, grid, d_rec, rec_cap, d_yaw, ev, stream);
     }
 }
 
-static bool fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
+cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
+                              const WfOutPtrs& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream) {
+    return launch_fixup_sized<false>(mode, use_vtab, m, fc, s, out, env_count, d_rec, rec_cap, nullptr, WfEvalArgs{}, stream);
+}
+
+// W is chosen from the B*K CTAs of the evaluation launch by the step's rule
+cudaError_t wf_launch_eval_fixup64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
+                                   const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream) {
+    WfOutPtrs out = {};
+    out.power = d_power;
+    return launch_fixup_sized<true>(WF_MODE_INTERFACE, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0, d_yaw, ev, stream);
+}
+
+bool wf_fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
 
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
                                   const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
     // a target-major table (and its scratch) belongs to the gather kernel; the scatter kernel evaluates every pair directly
-    const bool gather = fast64_gathers(m, s) && use_vtab;
+    const bool gather = wf_fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
     if (gather)
-        wf_step_fast64_kernel<true><<<env_count, 32, smem, stream>>>(mode, env_begin, true, m, fc, s, d_mask, d_action, d_yaw_cmd, out);
+        wf_step_fast64_kernel<true><<<env_count, 32, smem, stream>>>(mode, env_begin, true, m, fc, s, d_mask, d_action, d_yaw_cmd, out,
+                                                                     WfEvalArgs{});
     else
-        wf_step_fast64_kernel<false><<<env_count, 32, smem, stream>>>(mode, env_begin, use_vtab, m, fc, s, d_mask, d_action, d_yaw_cmd, out);
+        wf_step_fast64_kernel<false><<<env_count, 32, smem, stream>>>(mode, env_begin, use_vtab, m, fc, s, d_mask, d_action, d_yaw_cmd,
+                                                                      out, WfEvalArgs{});
+    return cudaGetLastError();
+}
+
+cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
+                                  const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream) {
+    // the same form as the step kernel of this handle in its current state (a stale table: the scatter form, pairs direct)
+    const bool gather = wf_fast64_gathers(m, s) && use_vtab;
+    const size_t smem = fast64_smem_bytes(m.T, gather);
+    const unsigned grid = (unsigned)m.B * (unsigned)ev.K;
+    WfOutPtrs out = {};
+    out.power = d_power;
+    if (gather)
+        wf_step_fast64_kernel<true, true><<<grid, 32, smem, stream>>>(WF_MODE_INTERFACE, 0, true, m, fc, s, nullptr, nullptr, d_yaw,
+                                                                      out, ev);
+    else
+        wf_step_fast64_kernel<false, true><<<grid, 32, smem, stream>>>(WF_MODE_INTERFACE, 0, use_vtab, m, fc, s, nullptr, nullptr,
+                                                                       d_yaw, out, ev);
     return cudaGetLastError();
 }
 
 cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                       int* smem) {
     *threads = 32;
-    const bool gather = fast64_gathers(m, s);
+    const bool gather = wf_fast64_gathers(m, s);
     *smem = (int)fast64_smem_bytes(m.T, gather);
     cudaError_t e = gather ? cudaFuncGetAttributes(attr, wf_step_fast64_kernel<true>) : cudaFuncGetAttributes(attr, wf_step_fast64_kernel<false>);
     if (e != cudaSuccess) return e;
