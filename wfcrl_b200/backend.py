@@ -28,6 +28,9 @@ _STATE_DTYPES = {
     "yi": (np.float64, "BT"), "cs": (np.float64, "B2"), "layout_id": (np.int32, "B"),
     "turbine_count": (np.int32, "B"),
 }
+# the step outputs (WfStepOut) and their shapes; each is "real" (the handle's precision) but the uint8 truncation flag
+_OUTPUTS = {"yaw": "BT", "wind_speed": "BT", "wind_direction": "BT", "power": "BT", "load": "BT4", "reward": "B",
+            "freewind": "B2", "truncated": "B"}
 
 
 def default_config() -> _lib.WfConfig:
@@ -38,6 +41,11 @@ def default_config() -> _lib.WfConfig:
 
 def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def _out_struct(bufs: Dict[str, torch.Tensor]) -> _lib.WfStepOut:
+    """The WfStepOut of the output buffers ``bufs`` (name -> tensor); the outputs it does not name are not written."""
+    return _lib.WfStepOut(**{k: t.data_ptr() for k, t in bufs.items()})
 
 
 class FlorisBatch:
@@ -81,20 +89,9 @@ class FlorisBatch:
         _lib.check(self.lib.wf_create(C.byref(cfg), lx.ctypes.data_as(C.c_void_p), ly.ctypes.data_as(C.c_void_p),
                                       C.byref(handle)))
         self.handle = handle
-        B, T, dev, r = self.B, self.T, self.device, self.real
-        self.out = {
-            "yaw": torch.zeros(B, T, dtype=r, device=dev),
-            "wind_speed": torch.zeros(B, T, dtype=r, device=dev),
-            "wind_direction": torch.zeros(B, T, dtype=r, device=dev),
-            "power": torch.zeros(B, T, dtype=r, device=dev),
-            "load": torch.zeros(B, T, 4, dtype=r, device=dev),
-            "reward": torch.zeros(B, dtype=r, device=dev),
-            "freewind": torch.zeros(B, 2, dtype=r, device=dev),
-            "truncated": torch.zeros(B, dtype=torch.uint8, device=dev),
-        }
-        self._out_struct = _lib.WfStepOut(*[self.out[k].data_ptr() for k in
-                                            ("yaw", "wind_speed", "wind_direction", "power", "load", "reward",
-                                             "freewind", "truncated")])
+        self.out = {k: torch.zeros(self._shape(kind), dtype=torch.uint8 if k == "truncated" else self.real,
+                                   device=self.device) for k, kind in _OUTPUTS.items()}
+        self._out_struct = _out_struct(self.out)
         self._host = None
         self.eval_capacity = 0  # largest K evaluate_yaw has run with (its output buffers and the library scratch hold that)
 
@@ -255,32 +252,33 @@ class FlorisBatch:
             self._eval_power, self._eval_amb, self.eval_capacity = power_buf, amb_buf, K
         return {"power": power, "ambiguous": amb.view(torch.bool)}
 
-    def step_host(self, action_host: torch.Tensor, fields=("yaw", "wind_speed", "wind_direction", "reward",
-                                                           "truncated", "power", "load", "freewind")):
+    def _host_out(self) -> Dict[str, torch.Tensor]:
+        """Pinned host mirror of ``self.out`` for the host-buffer entry points (allocated on first use)."""
+        if self._host is None:
+            self._host = {k: torch.empty(v.shape, dtype=v.dtype).pin_memory() for k, v in self.out.items()}
+        return self._host
+
+    def step_host(self, action_host: torch.Tensor, fields=tuple(_OUTPUTS)):
         """End-to-end step from HOST memory (pinned recommended): H2D action, step, D2H of ``fields``, sync."""
         if not (action_host.dtype == torch.float32 and not action_host.is_cuda and action_host.is_contiguous()):
             raise TypeError("action_host must be a contiguous float32 HOST tensor (pinned recommended)")
         if tuple(action_host.shape) != (self.B, self.T):
             raise ValueError(f"action_host must have shape ({self.B}, {self.T})")
-        if self._host is None:
-            self._host = {k: torch.empty(v.shape, dtype=v.dtype).pin_memory() for k, v in self.out.items()}
-        names = ("yaw", "wind_speed", "wind_direction", "power", "load", "reward", "freewind", "truncated")
-        st = _lib.WfStepOut(*[(self._host[k].data_ptr() if k in fields else None) for k in names])
+        host = self._host_out()
+        st = _out_struct({k: host[k] for k in fields})
         up, down = C.c_uint64(), C.c_uint64()
         _lib.check(self.lib.wf_step_host(self.handle, C.c_void_p(action_host.data_ptr()), C.byref(st), C.byref(up),
                                          C.byref(down)))
         self.last_h2d_bytes, self.last_d2h_bytes = up.value, down.value
-        return {k: self._host[k] for k in fields}
+        return {k: host[k] for k in fields}
 
     def update_command_host(self, yaw_host: Optional[np.ndarray] = None):
         """FlorisInterface.update_command from HOST memory in one library call (wf_update_command_host): float64 [B, T]
         yaw command in (or None), measures out as numpy views of pinned buffers (overwritten by the next call)."""
-        if self._host is None:
-            self._host = {k: torch.empty(v.shape, dtype=v.dtype).pin_memory() for k, v in self.out.items()}
         if getattr(self, "_host_np", None) is None:
-            self._host_np = {k: v.numpy() for k, v in self._host.items()}
-            names = ("yaw", "wind_speed", "wind_direction", "power", "load", "reward", "freewind", "truncated")
-            self._host_struct = _lib.WfStepOut(*[(self._host[k].data_ptr() if k != "reward" else None) for k in names])
+            host = self._host_out()
+            self._host_np = {k: v.numpy() for k, v in host.items()}
+            self._host_struct = _out_struct({k: v for k, v in host.items() if k != "reward"})
             self._yaw_pin = torch.empty(self.B, self.T, dtype=torch.float64).pin_memory()
             self._yaw_pin_np = self._yaw_pin.numpy()
         ptr = None
@@ -314,7 +312,7 @@ class FlorisBatch:
 
     # ------------------------------------------------------------------------------------------------------
     def _shape(self, kind):
-        return {"BT": (self.B, self.T), "B": (self.B,), "B2": (self.B, 2)}[kind]
+        return {"BT": (self.B, self.T), "BT4": (self.B, self.T, 4), "B": (self.B,), "B2": (self.B, 2)}[kind]
 
     def get_state(self, name: str) -> np.ndarray:
         dt, kind = _STATE_DTYPES[name]

@@ -47,7 +47,7 @@ struct WfHandle_t {
     // staging for wf_step_host
     float* d_action = nullptr;
     double* d_yaw_cmd = nullptr;
-    WfOutPtrs d_out = {};
+    WfStepOut d_out = {};
     static constexpr int kHostStreams = 6;
     cudaStream_t host_streams[kHostStreams] = {};  // one per chunk of the wf_step_host pipeline
     uint64_t launches = 0;
@@ -92,6 +92,47 @@ template <typename T> static int dev_alloc(WfHandle_t* h, T** p, size_t n) {
         int _r = (expr);          \
         if (_r != WF_OK) return _r; \
     } while (0)
+
+// A row of the tables below: a pointer member of WfStepOut or WfState, named by its byte offset (the members differ in
+// type), and the array it points to: element size (0 = "real") and extent, n elements per env (kB), per env and turbine
+// (kBT) or in all (kAll).
+enum Extent { kB, kBT, kAll };
+struct Array {
+    const char* name;  // of an exported state array (wf_get_state / wf_set_state), else NULL
+    size_t off, elem;
+    int n;
+    Extent ext;
+    size_t elems(size_t B, size_t T) const { return n * (ext == kBT ? B * T : ext == kB ? B : 1); }
+    size_t bytes(size_t B, size_t T, size_t es) const { return elems(B, T) * (elem ? elem : es); }
+};
+static void* ptr_at(const void* s, const Array& a) { void* p; memcpy(&p, (const char*)s + a.off, sizeof p); return p; }
+static void set_ptr_at(void* s, const Array& a, void* p) { memcpy((char*)s + a.off, &p, sizeof p); }
+
+// The eight step outputs in WfStepOut field order.  A strict FP32 handle's compact record (wf_fixup64_kernel) holds the
+// env id, then the per-env outputs, then the per-turbine outputs, each part in this order.
+static constexpr Array kOut[] = {
+    {nullptr, offsetof(WfStepOut, yaw), 0, 1, kBT}, {nullptr, offsetof(WfStepOut, wind_speed), 0, 1, kBT},
+    {nullptr, offsetof(WfStepOut, wind_direction), 0, 1, kBT}, {nullptr, offsetof(WfStepOut, power), 0, 1, kBT},
+    {nullptr, offsetof(WfStepOut, load), 0, 4, kBT}, {nullptr, offsetof(WfStepOut, reward), 0, 1, kB},
+    {nullptr, offsetof(WfStepOut, freewind), 0, 2, kB}, {nullptr, offsetof(WfStepOut, truncated), 1, 1, kB}};
+static constexpr int out_elems(Extent ext) { int n = 0; for (const Array& f : kOut) n += f.ext == ext ? f.n : 0; return n; }
+static_assert(WF_FIX_REC_HDR == 1 + out_elems(kB), "a fix-up record starts with the env id and the per-env outputs");
+
+// The state arrays wf_create always allocates.  Names and byte sizes are part of the ABI.
+#define MEMBER(m) offsetof(WfState, m), sizeof(*WfState::m)
+static constexpr Array kState[] = {
+    {"yaw", MEMBER(yaw), 1, kBT}, {"acc", MEMBER(acc), 1, kBT}, {"acc_prev", MEMBER(acc_prev), 1, kBT},
+    {"num_iter", MEMBER(num_iter), 1, kB}, {"num_moves", MEMBER(num_moves), 1, kB}, {"nonfinite", MEMBER(nonfinite), 1, kB},
+    {"episode", MEMBER(episode), 1, kB}, {"ambiguous", MEMBER(amb), 1, kB}, {"ep_return", MEMBER(ep_return), 1, kB},
+    {"ep_len", MEMBER(ep_len), 1, kB}, {"fin_sum", MEMBER(fin_sum), 1, kB}, {"fin_sumsq", MEMBER(fin_sumsq), 1, kB},
+    {"fin_n", MEMBER(fin_n), 1, kB}, {"fin_len", MEMBER(fin_len), 1, kB}, {nullptr, MEMBER(reset_mask), 1, kB},
+    {nullptr, MEMBER(fix_list), 1, kB}, {nullptr, MEMBER(fix_count), 4, kAll}, {"ws", MEMBER(ws), 1, kB},
+    {"wd", MEMBER(wd), 1, kB}, {"ws_norm", MEMBER(ws_norm), 1, kB}, {"shaper_ref", MEMBER(shaper_ref), 1, kB},
+    {"ti_ambient", MEMBER(ti_amb), 1, kB}, {"xs", MEMBER(xs), 1, kBT}, {"ys", MEMBER(ys), 1, kBT}, {"xi", MEMBER(xi), 1, kBT},
+    {"yi", MEMBER(yi), 1, kBT}, {"order", MEMBER(order), 1, kBT}, {"cs", MEMBER(cs), 2, kB}, {nullptr, MEMBER(xhl), 1, kBT},
+    {nullptr, MEMBER(yhl), 1, kBT}, {nullptr, MEMBER(idx), 1, kBT}, {nullptr, MEMBER(tab_lo), 1, kBT},
+    {nullptr, MEMBER(tab_glo), 1, kBT}, {"layout_id", MEMBER(layout_id), 1, kB}, {"turbine_count", MEMBER(turbine_count), 1, kB}};
+#undef MEMBER
 
 // called at the end of every asynchronous entry point: later host-buffer calls must run after the work queued here
 static int mark_async(WfHandle h, cudaStream_t st) {
@@ -287,24 +328,14 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
 
     WfState& s = h->st;
     const size_t BT = (size_t)B * T;
-    if ((rc = dev_alloc(h, &s.yaw, BT)) || (rc = dev_alloc(h, &s.acc, BT)) || (rc = dev_alloc(h, &s.acc_prev, BT)) ||
-        (rc = dev_alloc(h, &s.num_iter, (size_t)B)) || (rc = dev_alloc(h, &s.num_moves, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.nonfinite, (size_t)B)) || (rc = dev_alloc(h, &s.episode, (size_t)B)) || (rc = dev_alloc(h, &s.amb, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.reset_mask, (size_t)B)) || (rc = dev_alloc(h, &s.ep_return, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.ep_len, (size_t)B)) || (rc = dev_alloc(h, &s.fin_sum, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.fin_sumsq, (size_t)B)) || (rc = dev_alloc(h, &s.fin_n, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.fin_len, (size_t)B)) || (rc = dev_alloc(h, &s.fix_list, (size_t)B)) || (rc = dev_alloc(h, &s.fix_count, (size_t)4)) ||
-        (rc = dev_alloc(h, &s.ws, (size_t)B)) || (rc = dev_alloc(h, &s.wd, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.ws_norm, (size_t)B)) || (rc = dev_alloc(h, &s.shaper_ref, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.ti_amb, (size_t)B)) || (rc = dev_alloc(h, &s.xs, BT)) || (rc = dev_alloc(h, &s.ys, BT)) ||
-        (rc = dev_alloc(h, &s.xi, BT)) || (rc = dev_alloc(h, &s.yi, BT)) || (rc = dev_alloc(h, &s.order, BT)) ||
-        (rc = dev_alloc(h, &s.cs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.xhl, BT)) ||
-        (rc = dev_alloc(h, &s.yhl, BT)) || (rc = dev_alloc(h, &s.idx, BT)) || (rc = dev_alloc(h, &h->d_mask, (size_t)B)) ||
-        (rc = dev_alloc(h, &h->d_rws, (size_t)B)) || (rc = dev_alloc(h, &h->d_rwd, (size_t)B)) ||
-        (rc = dev_alloc(h, &h->d_rcs, (size_t)2 * B)) || (rc = dev_alloc(h, &s.layout_id, (size_t)B)) ||
-        (rc = dev_alloc(h, &s.turbine_count, (size_t)B)))
+    for (const Array& a : kState) {
+        char* p;
+        if ((rc = dev_alloc(h, &p, a.bytes(B, T, h->es)))) return fail(rc);
+        set_ptr_at(&s, a, p);
+    }
+    if ((rc = dev_alloc(h, &h->d_mask, (size_t)B)) || (rc = dev_alloc(h, &h->d_rws, (size_t)B)) ||
+        (rc = dev_alloc(h, &h->d_rwd, (size_t)B)) || (rc = dev_alloc(h, &h->d_rcs, (size_t)2 * B)))
         return fail(rc);
-    if ((rc = dev_alloc(h, &s.tab_lo, BT)) || (rc = dev_alloc(h, &s.tab_glo, BT))) return fail(rc);
     // The vortex table trades the V sweep's arithmetic for one streamed read of 36 reals per turbine pair.  Measured on B200
     // (profiles/r2_vortex_table.md): it pays in the FP64 kernels (whose sweep is 3x more expensive), but not in the FP32 kernel,
     // where the instructions that remain are latency-bound and the direct evaluation wins by 6 % -- so the FP32 step kernel
@@ -369,22 +400,13 @@ int wf_create(const WfConfig* cfg, const double* lx, const double* ly, WfHandle*
     return WF_OK;
 }
 
-static WfOutPtrs to_ptrs(const WfStepOut* o) {
-    WfOutPtrs p = {};
-    if (o) {
-        p.yaw = o->yaw; p.wind_speed = o->wind_speed; p.wind_direction = o->wind_direction; p.power = o->power;
-        p.load = o->load; p.reward = o->reward; p.freewind = o->freewind; p.truncated = o->truncated;
-    }
-    return p;
-}
-
 static bool is_strict_f32(WfHandle h) {
     return h->cfg.kernel == WF_KERNEL_FAST && h->cfg.precision == WF_PREC_F32 && h->model.amb_eps > 0.f;
 }
 
 // FP64 re-solve of the envs flagged by the FP32 launches issued since the previous fix-up (all of them must precede this launch
 // in stream order); d_rec / rec_cap: optional compact copies of the re-solved envs' results (host path)
-static int launch_fixup(WfHandle h, int mode, const WfOutPtrs& out, cudaStream_t st, float* d_rec = nullptr, int rec_cap = 0) {
+static int launch_fixup(WfHandle h, int mode, const WfStepOut& out, cudaStream_t st, float* d_rec = nullptr, int rec_cap = 0) {
     cudaError_t e = wf_launch_fixup64(mode, !h->vtab_stale, h->model, h->fast64, h->st, out, h->model.B, d_rec, rec_cap, st);
     h->launches += 1;
     if (e != cudaSuccess) return set_err(WF_ERR_CUDA, std::string("fix-up kernel launch: ") + cudaGetErrorString(e));
@@ -406,9 +428,11 @@ static void timing_collect(WfHandle h) {
     h->t_calls += 1;
 }
 
+// out == NULL: no outputs are written
 static int launch_step(WfHandle h, int mode, const uint8_t* d_mask, const float* d_action, const double* d_yaw,
-                       const WfOutPtrs& out, cudaStream_t st, int env_begin = 0, int env_count = -1,
+                       const WfStepOut* outp, cudaStream_t st, int env_begin = 0, int env_count = -1,
                        bool defer_fixup = false) {
+    const WfStepOut out = outp ? *outp : WfStepOut{};
     if (env_count < 0) env_count = h->model.B;
     const bool timed = h->timing && !defer_fixup && env_begin == 0 && env_count == h->model.B;
     if (timed) {
@@ -455,7 +479,7 @@ int wf_reset_masked(WfHandle h, const uint8_t* d_mask, const double* d_ws, const
     CUDA_TRY(wf_launch_reset_state(h->model, h->st, d_mask, d_ws, d_wd, st));
     CUDA_TRY(launch_geometry(h, d_mask, nullptr, st));
     h->launches += 1;
-    for (int k = 0; k < warmup; ++k) TRY(launch_step(h, WF_MODE_WARMUP, d_mask, nullptr, nullptr, to_ptrs(out), st));
+    for (int k = 0; k < warmup; ++k) TRY(launch_step(h, WF_MODE_WARMUP, d_mask, nullptr, nullptr, out, st));
     return mark_async(h, st);
 }
 
@@ -497,7 +521,7 @@ int wf_reset(WfHandle h, const int32_t* ids, int32_t n, const double* ws, const 
     CUDA_TRY(launch_geometry(h, h->d_mask, hc ? h->d_rcs : nullptr, st));
     h->launches += 1;
     for (int k = 0; k < warmup; ++k)
-        TRY(launch_step(h, WF_MODE_WARMUP, h->d_mask, nullptr, nullptr, to_ptrs(out), st));
+        TRY(launch_step(h, WF_MODE_WARMUP, h->d_mask, nullptr, nullptr, out, st));
     CUDA_TRY(cudaStreamSynchronize(st));  // the handle-owned pinned staging is reusable when this call returns
     return WF_OK;
 }
@@ -584,7 +608,7 @@ int wf_autoreset_finish(WfHandle h, int32_t warmup, const WfStepOut* out, void* 
     cudaStream_t st = (cudaStream_t)stream;
     const uint8_t* mask = h->st.reset_mask;
     CUDA_TRY(launch_geometry(h, mask, nullptr, st, true, /*autoreset_draw=*/true));
-    for (int k = 0; k < warmup; ++k) TRY(launch_step(h, WF_MODE_WARMUP, mask, nullptr, nullptr, to_ptrs(out), st));
+    for (int k = 0; k < warmup; ++k) TRY(launch_step(h, WF_MODE_WARMUP, mask, nullptr, nullptr, out, st));
     CUDA_TRY(cudaMemsetAsync(h->st.reset_mask, 0, (size_t)h->model.B, st));
     return mark_async(h, st);
 }
@@ -592,14 +616,14 @@ int wf_autoreset_finish(WfHandle h, int32_t warmup, const WfStepOut* out, void* 
 int wf_step(WfHandle h, const float* d_action, const WfStepOut* out, void* stream) {
     if (!h || !d_action) return set_err(WF_ERR_INVALID, "NULL argument");
     CUDA_TRY(cudaSetDevice(h->device));
-    TRY(launch_step(h, WF_MODE_ENV, nullptr, d_action, nullptr, to_ptrs(out), (cudaStream_t)stream));
+    TRY(launch_step(h, WF_MODE_ENV, nullptr, d_action, nullptr, out, (cudaStream_t)stream));
     return mark_async(h, (cudaStream_t)stream);
 }
 
 int wf_update_command(WfHandle h, const double* d_yaw, const WfStepOut* out, void* stream) {
     if (!h) return set_err(WF_ERR_INVALID, "NULL handle");
     CUDA_TRY(cudaSetDevice(h->device));
-    TRY(launch_step(h, WF_MODE_INTERFACE, nullptr, nullptr, d_yaw, to_ptrs(out), (cudaStream_t)stream));
+    TRY(launch_step(h, WF_MODE_INTERFACE, nullptr, nullptr, d_yaw, out, (cudaStream_t)stream));
     return mark_async(h, (cudaStream_t)stream);
 }
 
@@ -664,17 +688,28 @@ int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, u
 }
 
 // Device alias of a host pointer when it is page-locked memory the GPU can address (cudaHostAlloc / cudaHostRegister
-// under unified addressing, e.g. a torch pinned tensor); NULL for pageable memory.
-static void* mapped_alias(const void* p) {
+// under unified addressing, e.g. a torch pinned tensor); NULL for NULL, and for pageable memory, which clears *all.
+static void* mapped_alias(const void* p, bool* all) {
     cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-        cudaGetLastError();
-        return nullptr;
-    }
-    return a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
+    if (!p) return nullptr;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) cudaGetLastError();
+    else if (a.type == cudaMemoryTypeHost && a.devicePointer) return a.devicePointer;
+    *all = false;
+    return nullptr;
 }
 
 static constexpr size_t kZeroCopyMaxElems = 163840;  // envs x turbines up to which wf_step_host maps the host buffers
+
+// device -> host copies of env rows [b0, b0 + nb) of the outputs the caller asked for, from the staging buffers
+static int copy_out_rows(WfHandle h, const WfHostOut* ho, size_t b0, size_t nb, cudaStream_t st) {
+    for (const Array& f : kOut)
+        if (void* dst = ptr_at(ho, f)) {
+            const size_t row = f.bytes(1, h->model.T, h->es);
+            CUDA_TRY(cudaMemcpyAsync((char*)dst + b0 * row, (const char*)ptr_at(&h->d_out, f) + b0 * row, nb * row,
+                                     cudaMemcpyDeviceToHost, st));
+        }
+    return WF_OK;
+}
 
 // shared implementation of the two host-buffer entry points
 static int step_host_impl(WfHandle h, int mode, const float* h_action, const double* h_yaw, const WfHostOut* ho,
@@ -682,9 +717,9 @@ static int step_host_impl(WfHandle h, int mode, const float* h_action, const dou
     CUDA_TRY(cudaSetDevice(h->device));
     const size_t B = h->model.B, T = h->model.T, BT = B * T, es = h->es;
     const uint64_t up = (h_action ? sizeof(float) * BT : 0) + (h_yaw ? sizeof(double) * BT : 0);
-    const uint64_t down = ((ho->yaw ? BT : 0) + (ho->wind_speed ? BT : 0) + (ho->wind_direction ? BT : 0) +
-                           (ho->power ? BT : 0) + (ho->load ? 4 * BT : 0) + (ho->reward ? B : 0) +
-                           (ho->freewind ? 2 * B : 0)) * es + (ho->truncated ? B : 0);
+    uint64_t down = 0;
+    for (const Array& f : kOut)
+        if (ptr_at(ho, f)) down += f.bytes(B, T, es);
     if (h2d) *h2d = up;
     if (d2h) *d2h = down;
     // run after whatever the caller queued asynchronously on its own stream (resets, wind updates, device-side steps)
@@ -701,22 +736,13 @@ static int step_host_impl(WfHandle h, int mode, const float* h_action, const dou
     const bool want_zero = force ? !strcmp(force, "zero_copy") : BT <= kZeroCopyMaxElems;
     if (want_zero) {
         bool all = true;
-        WfOutPtrs z = {};
-        const float* za = nullptr;
-        const double* zy = nullptr;
-#define ALIAS(dst, src)                                   \
-    if (src) {                                            \
-        void* q = mapped_alias(src);                      \
-        all = all && q != nullptr;                        \
-        dst = static_cast<decltype(dst)>(q);              \
-    }
-        ALIAS(za, h_action) ALIAS(zy, h_yaw) ALIAS(z.yaw, ho->yaw) ALIAS(z.wind_speed, ho->wind_speed)
-        ALIAS(z.wind_direction, ho->wind_direction) ALIAS(z.power, ho->power) ALIAS(z.load, ho->load)
-        ALIAS(z.reward, ho->reward) ALIAS(z.freewind, ho->freewind) ALIAS(z.truncated, ho->truncated)
-#undef ALIAS
+        const float* za = (const float*)mapped_alias(h_action, &all);
+        const double* zy = (const double*)mapped_alias(h_yaw, &all);
+        WfStepOut z = {};
+        for (const Array& f : kOut) set_ptr_at(&z, f, mapped_alias(ptr_at(ho, f), &all));
         if (all) {
             if (wait_async) CUDA_TRY(cudaStreamWaitEvent(h->host_streams[0], h->ev_async, 0));
-            TRY(launch_step(h, mode, nullptr, za, zy, z, h->host_streams[0]));
+            TRY(launch_step(h, mode, nullptr, za, zy, &z, h->host_streams[0]));
             CUDA_TRY(cudaStreamSynchronize(h->host_streams[0]));
             return WF_OK;
         }
@@ -727,31 +753,21 @@ static int step_host_impl(WfHandle h, int mode, const float* h_action, const dou
     if (!h->d_action) {
         TRY(dev_alloc(h, &h->d_action, BT));
         TRY(dev_alloc(h, &h->d_yaw_cmd, BT));
-        char* p;
-        TRY(dev_alloc(h, &p, BT * es)); h->d_out.yaw = p;
-        TRY(dev_alloc(h, &p, BT * es)); h->d_out.wind_speed = p;
-        TRY(dev_alloc(h, &p, BT * es)); h->d_out.wind_direction = p;
-        TRY(dev_alloc(h, &p, BT * es)); h->d_out.power = p;
-        TRY(dev_alloc(h, &p, 4 * BT * es)); h->d_out.load = p;
-        TRY(dev_alloc(h, &p, B * es)); h->d_out.reward = p;
-        TRY(dev_alloc(h, &p, 2 * B * es)); h->d_out.freewind = p;
-        TRY(dev_alloc(h, &h->d_out.truncated, B));
+        for (const Array& f : kOut) {
+            char* p;
+            TRY(dev_alloc(h, &p, f.bytes(B, T, es)));
+            set_ptr_at(&h->d_out, f, p);
+        }
     }
-    WfOutPtrs o = {};
-    if (ho->yaw) o.yaw = h->d_out.yaw;
-    if (ho->wind_speed) o.wind_speed = h->d_out.wind_speed;
-    if (ho->wind_direction) o.wind_direction = h->d_out.wind_direction;
-    if (ho->power) o.power = h->d_out.power;
-    if (ho->load) o.load = h->d_out.load;
-    if (ho->reward) o.reward = h->d_out.reward;
-    if (ho->freewind) o.freewind = h->d_out.freewind;
-    if (ho->truncated) o.truncated = h->d_out.truncated;
+    WfStepOut o = {};  // the staging buffers of the outputs the caller asked for
+    for (const Array& f : kOut)
+        if (ptr_at(ho, f)) set_ptr_at(&o, f, ptr_at(&h->d_out, f));
     const int nchunk = (B >= 2048) ? WfHandle_t::kHostStreams : 1;
     // Strict FP32 handle: the chunks' FP32 launches share one fix-up list and ONE FP64 re-solve launch follows the last chunk,
     // so the chunks' device->host copies overlap the later chunks as before and only the re-solve of the few flagged envs
     // trails; their results come back as compact records that are scattered into the caller's arrays below.
     const bool strict = is_strict_f32(h);
-    const int rec_len = WF_FIX_REC_HDR + 8 * (int)T;
+    const int rec_len = WF_FIX_REC_HDR + out_elems(kBT) * (int)T;
     if (strict && !h->d_fix_rec) {
         h->fix_rec_cap = (int)(B < 1024 ? B : 1024);
         TRY(dev_alloc(h, &h->d_fix_rec, (size_t)h->fix_rec_cap * rec_len));
@@ -769,17 +785,10 @@ static int step_host_impl(WfHandle h, int mode, const float* h_action, const dou
             CUDA_TRY(cudaMemcpyAsync(h->d_action + b0 * T, h_action + b0 * T, sizeof(float) * nb * T, cudaMemcpyHostToDevice, st));
         if (h_yaw)
             CUDA_TRY(cudaMemcpyAsync(h->d_yaw_cmd + b0 * T, h_yaw + b0 * T, sizeof(double) * nb * T, cudaMemcpyHostToDevice, st));
-        TRY(launch_step(h, mode, nullptr, h_action ? h->d_action : nullptr, h_yaw ? h->d_yaw_cmd : nullptr, o, st,
+        TRY(launch_step(h, mode, nullptr, h_action ? h->d_action : nullptr, h_yaw ? h->d_yaw_cmd : nullptr, &o, st,
                         (int)b0, (int)nb, /*defer_fixup=*/true));
         if (strict) CUDA_TRY(cudaEventRecord(h->ev_chunk[c], st));
-#define D2H(field, per_env)                                                                                       \
-    if (ho->field) {                                                                                              \
-        const size_t off = b0 * (per_env), bytes = nb * (per_env);                                                \
-        CUDA_TRY(cudaMemcpyAsync((char*)ho->field + off, (char*)h->d_out.field + off, bytes, cudaMemcpyDeviceToHost, st)); \
-    }
-        D2H(load, 4 * T * es) D2H(yaw, T * es) D2H(wind_speed, T * es) D2H(wind_direction, T * es) D2H(power, T * es)
-        D2H(reward, es) D2H(freewind, 2 * es) D2H(truncated, 1)
-#undef D2H
+        TRY(copy_out_rows(h, ho, b0, nb, st));
     }
     if (strict) {
         cudaStream_t fs = h->host_streams[0];
@@ -801,23 +810,20 @@ static int step_host_impl(WfHandle h, int mode, const float* h_action, const dou
             const float* r = h->h_fix_rec + (size_t)k * rec_len;
             int b;
             memcpy(&b, r, sizeof(int));
-            const float* pt = r + WF_FIX_REC_HDR;
-            if (ho->reward) ((float*)ho->reward)[b] = r[1];
-            if (ho->freewind) { ((float*)ho->freewind)[2 * b] = r[2]; ((float*)ho->freewind)[2 * b + 1] = r[3]; }
-            if (ho->truncated) ho->truncated[b] = (uint8_t)(r[4] != 0.f);
-            if (ho->yaw) memcpy((float*)ho->yaw + (size_t)b * T, pt, sizeof(float) * T);
-            if (ho->wind_speed) memcpy((float*)ho->wind_speed + (size_t)b * T, pt + T, sizeof(float) * T);
-            if (ho->wind_direction) memcpy((float*)ho->wind_direction + (size_t)b * T, pt + 2 * T, sizeof(float) * T);
-            if (ho->power) memcpy((float*)ho->power + (size_t)b * T, pt + 3 * T, sizeof(float) * T);
-            if (ho->load) memcpy((float*)ho->load + (size_t)b * 4 * T, pt + 4 * T, sizeof(float) * 4 * T);
+            const float* part[2] = {r + 1, r + WF_FIX_REC_HDR};  // the per-env and the per-turbine outputs, in kOut order
+            for (const Array& f : kOut) {
+                const float* src = part[f.ext == kBT];
+                const size_t ne = f.elems(1, T);
+                part[f.ext == kBT] += ne;
+                uint8_t* dst = (uint8_t*)ptr_at(ho, f);
+                if (dst && f.elem == 1)  // truncated: stored as 1.f / 0.f
+                    for (size_t i = 0; i < ne; ++i) dst[b * ne + i] = (uint8_t)(src[i] != 0.f);
+                else if (dst)
+                    memcpy(dst + sizeof(float) * b * ne, src, sizeof(float) * ne);
+            }
         }
         if (n > have) {  // more re-solved envs than records (never in practice): copy their rows from the device arrays
-#define ROW(field, per_env)                                                                                      \
-    if (ho->field)                                                                                                \
-        CUDA_TRY(cudaMemcpyAsync((char*)ho->field, (char*)h->d_out.field, B * (per_env), cudaMemcpyDeviceToHost, fs));
-            ROW(load, 4 * T * es) ROW(yaw, T * es) ROW(wind_speed, T * es) ROW(wind_direction, T * es) ROW(power, T * es)
-            ROW(reward, es) ROW(freewind, 2 * es) ROW(truncated, 1)
-#undef ROW
+            TRY(copy_out_rows(h, ho, 0, B, fs));
             CUDA_TRY(cudaStreamSynchronize(fs));
         }
         return WF_OK;
@@ -859,31 +865,24 @@ int wf_set_turbulence_intensity(WfHandle h, const double* d_ti, void* stream) {
     return mark_async(h, (cudaStream_t)stream);
 }
 
-static int find_state(WfHandle h, const char* name, void** p, size_t* bytes) {
-    const size_t B = h->model.B, BT = B * h->model.T;
-    const WfState& s = h->st;
-    struct { const char* n; void* p; size_t b; } tab[] = {
-        {"yaw", s.yaw, BT * 8}, {"acc", s.acc, BT * 4}, {"acc_prev", s.acc_prev, BT * 4},
-        {"num_iter", s.num_iter, B * 4}, {"num_moves", s.num_moves, B * 4}, {"nonfinite", s.nonfinite, B * 4}, {"episode", s.episode, B * 4}, {"ambiguous", s.amb, B},
-        {"ep_return", s.ep_return, B * 8}, {"ep_len", s.ep_len, B * 4}, {"fin_sum", s.fin_sum, B * 8},
-        {"fin_sumsq", s.fin_sumsq, B * 8}, {"fin_n", s.fin_n, B * 4}, {"fin_len", s.fin_len, B * 8}, {"ws", s.ws, B * 8}, {"wd", s.wd, B * 8},
-        {"ws_norm", s.ws_norm, B * 8}, {"shaper_ref", s.shaper_ref, B * 8}, {"ti_ambient", s.ti_amb, B * 8},
-        {"order", s.order, BT * 4}, {"xs", s.xs, BT * 8}, {"ys", s.ys, BT * 8}, {"xi", s.xi, BT * 8},
-        {"yi", s.yi, BT * 8}, {"cs", s.cs, B * 16}, {"layout_id", s.layout_id, B * 4},
-        {"turbine_count", s.turbine_count, B * 4}};
-    for (auto& e : tab)
-        if (!strcmp(e.n, name)) { *p = e.p; *bytes = e.b; return WF_OK; }
+// the device array of an exported state array of `bytes` bytes
+static int find_state(WfHandle h, const char* name, size_t bytes, void** p) {
+    for (const Array& a : kState)
+        if (a.name && !strcmp(a.name, name)) {
+            if (a.bytes(h->model.B, h->model.T, h->es) != bytes) return set_err(WF_ERR_INVALID, "size mismatch for state array");
+            *p = ptr_at(&h->st, a);
+            return WF_OK;
+        }
     return set_err(WF_ERR_INVALID, std::string("unknown state array '") + name + "'");
 }
 
 int wf_get_state(WfHandle h, const char* name, void* dst, size_t bytes) {
     if (!h || !name || !dst) return set_err(WF_ERR_INVALID, "NULL argument");
-    void* p; size_t b;
-    TRY(find_state(h, name, &p, &b));
-    if (b != bytes) return set_err(WF_ERR_INVALID, "size mismatch for state array");
+    void* p;
+    TRY(find_state(h, name, bytes, &p));
     CUDA_TRY(cudaSetDevice(h->device));
     CUDA_TRY(cudaDeviceSynchronize());
-    CUDA_TRY(cudaMemcpy(dst, p, b, cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(dst, p, bytes, cudaMemcpyDeviceToHost));
     return WF_OK;
 }
 
@@ -894,9 +893,8 @@ int wf_set_state(WfHandle h, const char* name, const void* src, size_t bytes) {
                                        "rebuilds the geometry");
     if (!strcmp(name, "turbine_count"))
         return set_err(WF_ERR_INVALID, "\"turbine_count\" is read-only: it follows from the env's layout id");
-    void* p; size_t b;
-    TRY(find_state(h, name, &p, &b));
-    if (b != bytes) return set_err(WF_ERR_INVALID, "size mismatch for state array");
+    void* p;
+    TRY(find_state(h, name, bytes, &p));
     CUDA_TRY(cudaSetDevice(h->device));
     CUDA_TRY(cudaDeviceSynchronize());
     const bool yaw = !strcmp(name, "yaw");
@@ -911,7 +909,7 @@ int wf_set_state(WfHandle h, const char* name, const void* src, size_t bytes) {
                                                        std::to_string(cnt[e]) + " turbines, but column " + std::to_string(t) +
                                                        " (padding) is nonzero");
     }
-    CUDA_TRY(cudaMemcpy(p, src, b, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(p, src, bytes, cudaMemcpyHostToDevice));
     return WF_OK;
 }
 

@@ -1,5 +1,7 @@
 // Internal device-side structures shared by the kernels and the C-ABI layer (not part of the public ABI).
 #pragma once
+#include "../../include/wfcrl_b200.h"  // WfStepOut: the step kernels write the caller's output pointers
+
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -137,17 +139,6 @@ template <typename R> struct WfFastConstT {
 typedef WfFastConstT<float> WfFastConst;
 typedef WfFastConstT<double> WfFastConst64;
 
-struct WfOutPtrs {
-    void* yaw;
-    void* wind_speed;
-    void* wind_direction;
-    void* power;
-    void* load;
-    void* reward;
-    void* freewind;
-    uint8_t* truncated;
-};
-
 enum WfMode { WF_MODE_INTERFACE = 0, WF_MODE_ENV = 1, WF_MODE_WARMUP = 2 };
 
 // Candidate evaluation (wf_evaluate_yaw): the EVAL instantiations of the fast kernels solve K candidate yaw settings per env,
@@ -166,7 +157,7 @@ struct WfEvalArgs {
 cudaError_t wf_launch_geometry(const WfModel& m, const WfState& s, const uint8_t* d_mask, const double* d_cs_override,
                                cudaStream_t stream, bool autoreset_draw = false);
 cudaError_t wf_launch_step_basic(int precision, int mode, const WfModel& m, const WfState& s, const uint8_t* d_mask,
-                                 const float* d_action, const double* d_yaw_cmd, const WfOutPtrs& out,
+                                 const float* d_action, const double* d_yaw_cmd, const WfStepOut& out,
                                  int env_begin, int env_count, cudaStream_t stream);
 cudaError_t wf_launch_vortex_table(const WfModel& m, const WfFastConst64& fc, const WfState& s, const uint8_t* d_mask,
                                    cudaStream_t stream);
@@ -184,14 +175,14 @@ cudaError_t wf_configure_fast_kernels();    // wf_fast.cu
 cudaError_t wf_configure_fast64_kernels();  // wf_fast64.cu
 cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                 const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream);
+                                const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream);
 cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                              const WfOutPtrs& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream);
+                              const WfStepOut& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream);
 cudaError_t wf_step_fast_attributes(bool baked, const WfModel& m, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                     int* smem);
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                  const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream);
+                                  const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream);
 cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                       int* smem);
 // candidate evaluation: one launch of B*K CTAs (d_yaw [B*K][T], d_power real [B*K][T]); on a strict FP32 handle

@@ -130,7 +130,7 @@ template <bool BAKED, bool EVAL = false>
 __global__ void __launch_bounds__(32, BAKED ? 16 : 12)
 wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
                     const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
-                    const double* __restrict__ yaw_cmd, const WfOutPtrs out, const WfEvalArgs ev) {
+                    const double* __restrict__ yaw_cmd, const WfStepOut out, const WfEvalArgs ev) {
     int b;
     if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
     const int mode = EVAL ? (int)WF_MODE_INTERFACE : mode_;
@@ -652,7 +652,7 @@ cudaError_t wf_configure_fast_kernels() {
 template <bool BAKED>
 static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                  const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                 const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
+                                 const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream) {
     wf_step_fast_kernel<BAKED><<<env_count, 32, fast_smem_bytes(m.T), stream>>>(mode, env_begin, m, fc, s, d_mask, d_action,
                                                                                d_yaw_cmd, out, WfEvalArgs{});
     return cudaGetLastError();
@@ -661,7 +661,7 @@ static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& 
 template <bool BAKED>
 static cudaError_t launch_eval_t(const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
                                  const double* d_yaw, void* d_power, cudaStream_t stream) {
-    WfOutPtrs out = {};
+    WfStepOut out = {};
     out.power = d_power;
     wf_step_fast_kernel<BAKED, true><<<(unsigned)m.B * (unsigned)ev.K, 32, fast_smem_bytes(m.T), stream>>>(
         WF_MODE_INTERFACE, 0, m, fc, s, nullptr, nullptr, d_yaw, out, ev);
@@ -676,7 +676,7 @@ cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst&
 
 cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,
                                 const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
+                                const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream) {
     return baked ? launch_fast_t<true>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, stream)
                  : launch_fast_t<false>(mode, m, fc, s, d_mask, d_action, d_yaw_cmd, out, env_begin, env_count, stream);
 }

@@ -193,7 +193,7 @@ __device__ __forceinline__ void load_row12(const double* __restrict__ p, double*
 template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false>
 __device__ __forceinline__ void solve_env64(const int b, const int mode, const bool use_vtab, const WfModel& m,
                                             const WfFastConst64& fc, const WfState& s, const float* __restrict__ action,
-                                            const double* __restrict__ yaw_cmd, const WfOutPtrs& out,
+                                            const double* __restrict__ yaw_cmd, const WfStepOut& out,
                                             float* __restrict__ rec, const WfEvalArgs& ev, const int cand) {
     const int T = m.T;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -892,7 +892,7 @@ template <bool GATHER, bool EVAL = false>
 __global__ void __launch_bounds__(32, 16)
 wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                       const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
-                      const double* __restrict__ yaw_cmd, const WfOutPtrs out, const WfEvalArgs ev) {
+                      const double* __restrict__ yaw_cmd, const WfStepOut out, const WfEvalArgs ev) {
     int b;
     if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
     if (mask && !mask[b]) return;
@@ -905,7 +905,7 @@ wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, 
 template <int W>
 __global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
 wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
-                  const WfState s, const WfOutPtrs out, float* __restrict__ rec, const int rec_cap) {
+                  const WfState s, const WfStepOut out, float* __restrict__ rec, const int rec_cap) {
     const int n = *(volatile int*)&s.fix_count[0];
     const int rec_len = WF_FIX_REC_HDR + 8 * m.T;  // header (env id, reward, freewind x2, truncated) + yaw, ws, wd, power, load x4
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
@@ -929,7 +929,7 @@ wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __
 template <int W>
 __global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
 wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc, const WfState s,
-                       const WfOutPtrs out, const double* __restrict__ yaw_cmd, const WfEvalArgs ev) {
+                       const WfStepOut out, const double* __restrict__ yaw_cmd, const WfEvalArgs ev) {
     const int n = *(volatile int*)&ev.fix_count[0];
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
         const int c = ev.fix_list[k];
@@ -970,7 +970,7 @@ cudaError_t wf_configure_fast64_kernels() {
 
 template <int W, bool EVAL>
 static cudaError_t launch_fixup_t(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                  const WfOutPtrs& out, int grid, float* d_rec, int rec_cap, const double* d_yaw,
+                                  const WfStepOut& out, int grid, float* d_rec, int rec_cap, const double* d_yaw,
                                   const WfEvalArgs& ev, cudaStream_t stream) {
     if (EVAL)
         wf_fixup64_eval_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_yaw, ev);
@@ -982,7 +982,7 @@ static cudaError_t launch_fixup_t(int mode, bool use_vtab, const WfModel& m, con
 // W and the grid of a re-solve launch behind a step (or evaluation) launch of `count` CTAs
 template <bool EVAL>
 static cudaError_t launch_fixup_sized(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                      const WfOutPtrs& out, int count, float* d_rec, int rec_cap, const double* d_yaw,
+                                      const WfStepOut& out, int count, float* d_rec, int rec_cap, const double* d_yaw,
                                       const WfEvalArgs& ev, cudaStream_t stream) {
     // The launch is latency-bound while the flagged envs (1-2 % of the batch) are fewer than the CTAs the GPU holds at once,
     // and each env is a sequential sweep over its turbines: W warps per env cover 10 W targets in one fused pass per source.
@@ -1002,14 +1002,14 @@ static cudaError_t launch_fixup_sized(int mode, bool use_vtab, const WfModel& m,
 }
 
 cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                              const WfOutPtrs& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream) {
+                              const WfStepOut& out, int env_count, float* d_rec, int rec_cap, cudaStream_t stream) {
     return launch_fixup_sized<false>(mode, use_vtab, m, fc, s, out, env_count, d_rec, rec_cap, nullptr, WfEvalArgs{}, stream);
 }
 
 // W is chosen from the B*K CTAs of the evaluation launch by the step's rule
 cudaError_t wf_launch_eval_fixup64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                    const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream) {
-    WfOutPtrs out = {};
+    WfStepOut out = {};
     out.power = d_power;
     return launch_fixup_sized<true>(WF_MODE_INTERFACE, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0, d_yaw, ev, stream);
 }
@@ -1018,7 +1018,7 @@ bool wf_fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajo
 
 cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const uint8_t* d_mask, const float* d_action, const double* d_yaw_cmd,
-                                  const WfOutPtrs& out, int env_begin, int env_count, cudaStream_t stream) {
+                                  const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream) {
     // a target-major table (and its scratch) belongs to the gather kernel; the scatter kernel evaluates every pair directly
     const bool gather = wf_fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
@@ -1037,7 +1037,7 @@ cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastC
     const bool gather = wf_fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
     const unsigned grid = (unsigned)m.B * (unsigned)ev.K;
-    WfOutPtrs out = {};
+    WfStepOut out = {};
     out.power = d_power;
     if (gather)
         wf_step_fast64_kernel<true, true><<<grid, 32, smem, stream>>>(WF_MODE_INTERFACE, 0, true, m, fc, s, nullptr, nullptr, d_yaw,

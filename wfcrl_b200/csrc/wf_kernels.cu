@@ -394,7 +394,7 @@ template <typename R, int G>
 __global__ void __launch_bounds__(WF_MAX_TURBINES_K)
 wf_step_basic_kernel(const int mode, const int env_begin, const WfModel m, const WfState s,
                      const uint8_t* __restrict__ mask, const float* __restrict__ action,
-                     const double* __restrict__ yaw_cmd, const WfOutPtrs out) {
+                     const double* __restrict__ yaw_cmd, const WfStepOut out) {
     const int b = blockIdx.x + env_begin;
     if (mask && !mask[b]) return;
     const int T = m.T;
@@ -848,7 +848,7 @@ cudaError_t wf_launch_reset_state(const WfModel& m, const WfState& s, const uint
 }
 
 cudaError_t wf_launch_step_basic(int precision, int mode, const WfModel& m, const WfState& s, const uint8_t* d_mask,
-                                 const float* d_action, const double* d_yaw_cmd, const WfOutPtrs& out,
+                                 const float* d_action, const double* d_yaw_cmd, const WfStepOut& out,
                                  int env_begin, int env_count, cudaStream_t stream) {
     const int threads = round_up_warp(m.T);
 #define WF_GO(R_, G_) wf_step_basic_kernel<R_, G_><<<env_count, threads, 0, stream>>>(mode, env_begin, m, s, d_mask, d_action, d_yaw_cmd, out)
