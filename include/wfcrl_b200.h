@@ -249,6 +249,34 @@ int wf_update_command(WfHandle h, const double* d_yaw, const WfStepOut* out, voi
 int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, uint8_t* d_ambiguous, void* stream);
 
 /*
+ * ACTION EVALUATION (one-step lookahead).  What wf_step would return for each of K candidate actions per env, from where
+ * each env is now, without stepping: the batched one-step model query of model-based RL, MPC and planning baselines.
+ *   d_action:    DEVICE float [B][K][T], each [T] row interpreted exactly as wf_step interprets d_action (continuous:
+ *                increments clipped to +-step; discrete: values in {0, 1, 2})
+ *   out:         a WfStepOut whose buffers have B*K rows, i.e. the shapes of a handle of B*K envs: real [B][K][T] yaw,
+ *                wind_speed, wind_direction, power, real [B][K][T][4] load, real [B][K] reward, uint8 [B][K] truncated,
+ *                real [B][K][2] freewind.  Any member may be NULL, as for wf_step.  Env-mode units (MW, loads / 1e7).
+ *   d_ambiguous: DEVICE uint8 [B][K] or NULL, as for wf_evaluate_yaw
+ * WF_KERNEL_FAST handles only.  Asynchronous on `stream`.
+ *  - Results: row (b, k) of every output equals, bit for bit, row b of what wf_step would write on this handle in its
+ *    current state with candidate k as env b's action: the actuation constraint with acc / num_moves (acc_prev on
+ *    multi-agent handles), the clip, the float32 yaw transition, the loads, the reward normalised by ws_norm with its load
+ *    term and shaper (StepPercentage reads shaper_ref and does not write it), truncated = (num_iter + 1 == max_iter), and
+ *    candidates that a strict FP32 handle flags and re-solves in FP64.
+ *  - State: as wf_evaluate_yaw, nothing changes -- yaw, acc, acc_prev, num_iter, num_moves, nonfinite, episode,
+ *    "ambiguous", the episode sums, shaper_ref, ws_norm, the step path's re-solve list -- and the in-kernel auto-reset never
+ *    fires or marks an env.  The next wf_step gives the same result bit for bit as if the evaluation had not happened.
+ *  - Layout pools of mixed counts: actions in columns n..T-1 of an env of n < T turbines are ignored (they may hold NaN);
+ *    those columns of every per-turbine output are written as 0.
+ *  - Launches, scratch, auto-reset precondition: as wf_evaluate_yaw, with which it shares the scratch (calls of the two
+ *    with different K may be interleaved).
+ * Refused with WF_ERR_INVALID before any work: WF_KERNEL_BASIC handles, K < 1, NULL d_action or out, and
+ * B*K > 2^31 - 1.
+ */
+int wf_evaluate_actions(WfHandle h, const float* d_action, int32_t K, const WfStepOut* out, uint8_t* d_ambiguous,
+                        void* stream);
+
+/*
  * End-to-end convenience for hosts without device buffers: `h_action` (float [B][T]) in, wf_step, every non-NULL
  * member of `h_out` out, synchronous.  Two routes, same results bit for bit:
  *   - staged: cudaMemcpyAsync into device staging owned by the handle, 6 env chunks on 6 streams so the copies of one

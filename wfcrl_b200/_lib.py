@@ -65,6 +65,7 @@ SYMBOLS = {
     "wf_step": (C.c_int, [_P, _P, C.POINTER(WfStepOut), _P]),
     "wf_update_command": (C.c_int, [_P, _P, C.POINTER(WfStepOut), _P]),
     "wf_evaluate_yaw": (C.c_int, [_P, _P, C.c_int32, _P, _P, _P]),
+    "wf_evaluate_actions": (C.c_int, [_P, _P, C.c_int32, C.POINTER(WfStepOut), _P, _P]),
     "wf_step_host": (C.c_int, [_P, _P, C.POINTER(WfStepOut), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "wf_update_command_host": (C.c_int, [_P, _P, C.POINTER(WfStepOut)]),
     "wf_update_wind": (C.c_int, [_P, _P, _P, _P, _P, _P]),

@@ -94,6 +94,7 @@ class FlorisBatch:
         self._out_struct = _out_struct(self.out)
         self._host = None
         self.eval_capacity = 0  # largest K evaluate_yaw has run with (its output buffers and the library scratch hold that)
+        self.act_capacity, self._act_bufs = 0, None  # the same for evaluate_actions
 
     # ------------------------------------------------------------------------------------------------------
     def close(self):
@@ -251,6 +252,35 @@ class FlorisBatch:
         if K > self.eval_capacity:  # the library holds scratch for this K now
             self._eval_power, self._eval_amb, self.eval_capacity = power_buf, amb_buf, K
         return {"power": power, "ambiguous": amb.view(torch.bool)}
+
+    def evaluate_actions(self, action: torch.Tensor) -> Dict[str, torch.Tensor]:
+        """What ``step`` would return for each of K candidate actions per env, from the current state, without stepping
+        (``wf_evaluate_actions``).  ``action``: contiguous float32 CUDA tensor [B, K, T], each [T] row interpreted as
+        ``step`` interprets one; padding columns of a mixed-count pool are ignored.  Returns the eight step outputs with a K
+        axis after the batch axis (``yaw`` [B, K, T], ..., ``load`` [B, K, T, 4], ``reward`` / ``truncated`` [B, K],
+        ``freewind`` [B, K, 2]; env-mode units) and ``"ambiguous"`` bool [B, K], views of buffers owned by the batch that
+        the next call overwrites.  No state changes.  Asynchronous; the first call with a larger K than before allocates,
+        synchronously."""
+        if not (torch.is_tensor(action) and action.dtype == torch.float32 and action.is_cuda and action.is_contiguous()):
+            raise TypeError("action must be a contiguous float32 CUDA tensor of shape [B, K, T]")
+        if action.dim() != 3 or action.shape[0] != self.B or action.shape[2] != self.T or action.shape[1] < 1:
+            raise ValueError(f"action must have shape ({self.B}, K, {self.T}) with K >= 1, got {tuple(action.shape)}")
+        K = int(action.shape[1])
+        kinds = dict(_OUTPUTS, ambiguous="B")
+        bufs = self._act_bufs
+        if K > self.act_capacity:
+            bufs = {k: torch.zeros((self.B, K) + self._shape(kind)[1:], device=self.device,
+                                   dtype=torch.uint8 if k in ("truncated", "ambiguous") else self.real)
+                    for k, kind in kinds.items()}
+        res = {k: bufs[k].view(-1)[: self.B * K * bufs[k][0, 0].numel()].view((self.B, K) + bufs[k].shape[2:])
+               for k in kinds}
+        amb = res.pop("ambiguous")
+        _lib.check(self.lib.wf_evaluate_actions(self.handle, _ptr(action), K, C.byref(_out_struct(res)), _ptr(amb),
+                                                self._stream()))
+        if K > self.act_capacity:
+            self._act_bufs, self.act_capacity = bufs, K
+        res["ambiguous"] = amb.view(torch.bool)
+        return res
 
     def _host_out(self) -> Dict[str, torch.Tensor]:
         """Pinned host mirror of ``self.out`` for the host-buffer entry points (allocated on first use)."""

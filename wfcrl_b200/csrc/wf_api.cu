@@ -70,11 +70,13 @@ struct WfHandle_t {
     double* d_pool = nullptr;  // the layout pool in one allocation: [L][T] x, [L][T] y, [L][2] centres, [L] int32 turbine
                                // counts (WfModel.layout_*)
     std::vector<int> layout_n;  // host copy of the pool's turbine counts
-    // wf_evaluate_yaw scratch, sized for the largest B*K evaluated so far: the evaluation fix list [eval_cap] and its 4
-    // counters in one allocation, and on a gathering FP64 handle one (v, w) scratch row per candidate [eval_cap][9T]
+    // wf_evaluate_yaw / wf_evaluate_actions scratch, sized for the largest B*K either has evaluated so far: the evaluation fix
+    // list [eval_cap] and its 4 counters in one allocation, on a gathering FP64 handle one (v, w) scratch row per candidate
+    // [eval_cap][9T], on a strict FP32 handle one transitioned-yaw row per candidate [eval_cap][T]
     int eval_cap = 0;
     int* d_eval_fix = nullptr;
     double2* d_eval_vwg = nullptr;
+    double* d_eval_yaw = nullptr;
 };
 
 template <typename T> static int dev_alloc(WfHandle_t* h, T** p, size_t n) {
@@ -241,6 +243,7 @@ int wf_destroy(WfHandle h) {
     if (h->h_fix_n) cudaFreeHost(h->h_fix_n);
     if (h->d_eval_fix) cudaFree(h->d_eval_fix);
     if (h->d_eval_vwg) cudaFree(h->d_eval_vwg);
+    if (h->d_eval_yaw) cudaFree(h->d_eval_yaw);
     delete h;
     return WF_OK;
 }
@@ -634,8 +637,10 @@ static int eval_reserve(WfHandle h, int cap) {
     CUDA_TRY(cudaDeviceSynchronize());
     if (h->d_eval_fix) cudaFree(h->d_eval_fix);
     if (h->d_eval_vwg) cudaFree(h->d_eval_vwg);
+    if (h->d_eval_yaw) cudaFree(h->d_eval_yaw);
     h->d_eval_fix = nullptr;
     h->d_eval_vwg = nullptr;
+    h->d_eval_yaw = nullptr;
     h->eval_cap = 0;
     const size_t fix_bytes = sizeof(int) * ((size_t)cap + 4);
     cudaError_t e = cudaMalloc(&h->d_eval_fix, fix_bytes);
@@ -645,6 +650,8 @@ static int eval_reserve(WfHandle h, int cap) {
         e = cudaMalloc(&h->d_eval_vwg, vwg_bytes);
         if (e == cudaSuccess) e = cudaMemset(h->d_eval_vwg, 0, vwg_bytes);
     }
+    if (e == cudaSuccess && is_strict_f32(h))
+        e = cudaMalloc(&h->d_eval_yaw, sizeof(double) * (size_t)h->model.T * (size_t)cap);  // written before it is read
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -655,36 +662,52 @@ static int eval_reserve(WfHandle h, int cap) {
     return WF_OK;
 }
 
-int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, uint8_t* d_ambiguous, void* stream) {
+// The two evaluation entry points: yaw candidates d_yaw (interface mode, out.power only) or action candidates d_action (env
+// mode, every output of out), K per env, outputs in rows of B*K
+static int evaluate(WfHandle h, const char* fn, const double* d_yaw, const float* d_action, int32_t K, const WfStepOut* outp,
+                    uint8_t* d_ambiguous, cudaStream_t st) {
     if (!h) return set_err(WF_ERR_INVALID, "NULL handle");
     if (h->cfg.kernel != WF_KERNEL_FAST)
-        return set_err(WF_ERR_INVALID, "wf_evaluate_yaw needs the warp-per-env kernels (WF_KERNEL_FAST)");
+        return set_err(WF_ERR_INVALID, std::string(fn) + " needs the warp-per-env kernels (WF_KERNEL_FAST)");
+    // K >= 1 is also what keeps the evaluation kernels from writing state: the FP64 ones skip their commits on a run-time
+    // test of K (wf_fast64.cu: solve_env64), so this refusal must stay ahead of every launch below
     if (K < 1) return set_err(WF_ERR_INVALID, "K (candidates per env) must be >= 1");
-    if (!d_yaw || !d_power) return set_err(WF_ERR_INVALID, "NULL argument");
+    if ((!d_yaw && !d_action) || !outp) return set_err(WF_ERR_INVALID, "NULL argument");
+    const WfStepOut out = *outp;
     const int64_t BK = (int64_t)h->model.B * K;
     if (BK > (int64_t)INT32_MAX)
         return set_err(WF_ERR_INVALID, "num_envs * K = " + std::to_string(BK) + " candidates exceed the kernels' 32-bit index "
                                        "(at most 2^31 - 1 per call)");
     CUDA_TRY(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
     if (BK > h->eval_cap) TRY(eval_reserve(h, (int)BK));
-    const WfEvalArgs ev = {K, h->d_eval_fix, h->d_eval_fix + h->eval_cap, d_ambiguous, h->d_eval_vwg};
+    const WfEvalArgs ev = {K, h->d_eval_fix, h->d_eval_fix + h->eval_cap, d_ambiguous, h->d_eval_vwg, h->d_eval_yaw};
     // the route of a step in the handle's current state: a stale vortex table is not read
     const bool use_vtab = !h->vtab_stale;
     cudaError_t e;
     if (h->cfg.precision == WF_PREC_F64) {
-        e = wf_launch_eval_fast64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_power, st);
+        e = wf_launch_eval_fast64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_action, out, st);
         h->launches += 1;
     } else {
-        e = wf_launch_eval_fast(h->fast_baked, h->model, h->fast, h->st, ev, d_yaw, d_power, st);
+        e = wf_launch_eval_fast(h->fast_baked, h->model, h->fast, h->st, ev, d_yaw, d_action, out, st);
         h->launches += 1;
         if (e == cudaSuccess && is_strict_f32(h)) {
-            e = wf_launch_eval_fixup64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_power, st);
+            e = wf_launch_eval_fixup64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_action != nullptr, out, st);
             h->launches += 1;
         }
     }
     if (e != cudaSuccess) return set_err(WF_ERR_CUDA, std::string("evaluation kernel launch: ") + cudaGetErrorString(e));
     return mark_async(h, st);
+}
+
+int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, uint8_t* d_ambiguous, void* stream) {
+    WfStepOut out = {};
+    out.power = d_power;
+    return evaluate(h, "wf_evaluate_yaw", d_yaw, nullptr, K, d_power ? &out : nullptr, d_ambiguous, (cudaStream_t)stream);
+}
+
+int wf_evaluate_actions(WfHandle h, const float* d_action, int32_t K, const WfStepOut* out, uint8_t* d_ambiguous,
+                        void* stream) {
+    return evaluate(h, "wf_evaluate_actions", nullptr, d_action, K, out, d_ambiguous, (cudaStream_t)stream);
 }
 
 // Device alias of a host pointer when it is page-locked memory the GPU can address (cudaHostAlloc / cudaHostRegister

@@ -141,16 +141,18 @@ typedef WfFastConstT<double> WfFastConst64;
 
 enum WfMode { WF_MODE_INTERFACE = 0, WF_MODE_ENV = 1, WF_MODE_WARMUP = 2 };
 
-// Candidate evaluation (wf_evaluate_yaw): the EVAL instantiations of the fast kernels solve K candidate yaw settings per env,
-// CTA c = candidate c = env c / K, candidate c % K (the K candidates of an env are adjacent, so that its geometry and table
-// rows are shared in L2).  They read the candidate's yaw from the caller's [B*K][T] array, write its power row c and touch
-// no WfState array.  The scratch below belongs to the handle's evaluation path alone.
+// Candidate evaluation (wf_evaluate_yaw, wf_evaluate_actions): the EVAL instantiations of the fast kernels solve K candidates
+// per env, CTA c = candidate c = env c / K, candidate c % K (the K candidates of an env are adjacent, so that its geometry and
+// table rows are shared in L2).  They read the candidate's yaw (or action) from the caller's [B*K][T] array, write its output
+// rows c and write no WfState array.  The scratch below belongs to the handle's evaluation path alone.
 struct WfEvalArgs {
     int K;             // candidates per env
     int* fix_list;     // [B*K] strict FP32: ids of the candidates the FP32 launch flagged (never the step path's fix_list)
     int* fix_count;    // [4] as WfState.fix_count, for fix_list
     uint8_t* amb;      // [B*K] or NULL: 1 = the candidate was re-solved by the FP64 kernel
     double2* vwg;      // [B*K][9T] FP64 gather form: the (v, w) scratch, one row per candidate (WfState.vwg is per env)
+    double* yaw;       // [B*K][T] strict FP32, actions: the transitioned yaw of a flagged candidate, which its re-solve
+                       //     reads where the step's re-solve reads the committed WfState.yaw
 };
 
 // launchers implemented in wf_kernels.cu
@@ -185,12 +187,15 @@ cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, con
                                   const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream);
 cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                       int* smem);
-// candidate evaluation: one launch of B*K CTAs (d_yaw [B*K][T], d_power real [B*K][T]); on a strict FP32 handle
-// wf_launch_eval_fixup64 re-solves the flagged candidates (ev.fix_list) in FP64
+// candidate evaluation: one launch of B*K CTAs with out's buffers of B*K rows; on a strict FP32 handle wf_launch_eval_fixup64
+// re-solves the flagged candidates (ev.fix_list) in FP64.  d_action == NULL: yaw candidates d_yaw [B*K][T] in interface mode,
+// out.power only (wf_evaluate_yaw); else action candidates d_action [B*K][T] in env mode, every output (wf_evaluate_actions)
 cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
-                                const double* d_yaw, void* d_power, cudaStream_t stream);
+                                const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream);
 cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                  const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream);
+                                  const WfEvalArgs& ev, const double* d_yaw, const float* d_action, const WfStepOut& out,
+                                  cudaStream_t stream);
 cudaError_t wf_launch_eval_fixup64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                   const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream);
+                                   const WfEvalArgs& ev, const double* d_yaw, bool actions, const WfStepOut& out,
+                                   cudaStream_t stream);
 bool wf_fast64_gathers(const WfModel& m, const WfState& s);  // an FP64 handle's step kernel runs the gather form

@@ -126,19 +126,22 @@ struct wf_false_tag { static constexpr bool value = false; };
 // generic instantiation: 12 is a lower bound for the register allocator; 16 envs per SM are reached
 // EVAL (wf_evaluate_yaw): CTA c solves candidate c of env c / K in interface mode with the yaw row c of `yaw_cmd`, writes power
 // row c of `out.power` and nothing else, and hands a flagged candidate to the evaluation fix list (wf_device.cuh: WfEvalArgs)
-template <bool BAKED, bool EVAL = false>
+// EVAL + ACT (wf_evaluate_actions): CTA c runs env b = c / K's step with action row c in the run-time mode (env) of the step --
+// transition, solve, epilogue and reward -- against b's state, which it reads and never writes; every output goes to row c.
+// A flagged candidate leaves its transitioned yaw in ev.yaw row c for the re-solve
+template <bool BAKED, bool EVAL = false, bool ACT = false>
 __global__ void __launch_bounds__(32, BAKED ? 16 : 12)
 wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
                     const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
                     const double* __restrict__ yaw_cmd, const WfStepOut out, const WfEvalArgs ev) {
     int b;
     if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
-    const int mode = EVAL ? (int)WF_MODE_INTERFACE : mode_;
+    const int mode = (EVAL && !ACT) ? (int)WF_MODE_INTERFACE : mode_;
     if (mask && !mask[b]) return;
     const int T = m.T;
     const int lane = threadIdx.x;
     const size_t row = (size_t)b * T;
-    const size_t orow = EVAL ? (size_t)blockIdx.x * T : row;  // row of the yaw command and of the outputs
+    const size_t orow = EVAL ? (size_t)blockIdx.x * T : row;  // row of the yaw command / action and of the outputs
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const SmemView sm = carve(smem_raw, T);  // sized by T: every env of the handle reserves the same shared memory
     // the env's turbine count: the one loop bound below.  Columns n..T-1 of its rows are padding (wf_device.cuh)
@@ -150,7 +153,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
     for (int tt = lane; tt < n; tt += 32) {
         float ynew;
         if (mode == WF_MODE_ENV) {
-            float a = action[row + tt];
+            float a = action[orow + tt];
             const float acc = s.acc[row + tt];
             const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
             const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
@@ -159,9 +162,11 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
             else a = __fmul_rn(__fsub_rn(a, 1.0f), m.yaw_step_f);
             const float y0 = fminf(fmaxf((float)s.yaw[row + tt], m.yaw_lo_f), m.yaw_hi_f);
             ynew = fminf(fmaxf(__fadd_rn(y0, a), m.yaw_lo_f), m.yaw_hi_f);
-            s.acc_prev[row + tt] = acc;
-            s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
-            s.yaw[row + tt] = (double)ynew;
+            if (!ACT) {
+                s.acc_prev[row + tt] = acc;
+                s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
+                s.yaw[row + tt] = (double)ynew;
+            }
         } else if (mode == WF_MODE_INTERFACE && yaw_cmd) {
             const double y = yaw_cmd[orow + tt];
             if (!EVAL) s.yaw[row + tt] = y;
@@ -548,7 +553,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
             for (int q = 0; q < 4; ++q) loads[q] *= 1e7f;
         }
         const int orig = sm.ordr[tt];
-        if (EVAL) {  // the power is written once the candidate is known not to be flagged (below)
+        if (EVAL && !ACT) {  // the power is written once the candidate is known not to be flagged (below)
             sm.tifin[tt] = p_out;
             continue;
         }
@@ -558,7 +563,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
             wdl = fclamp(wdl, 0.f, 360.f);
             yv = fclamp(yv, m.yaw_lo_f, m.yaw_hi_f);
         }
-        const size_t o = row + orig;
+        const size_t o = orow + orig;
         if (out.yaw) ((float*)out.yaw)[o] = yv;
         if (out.wind_speed) ((float*)out.wind_speed)[o] = wsl;
         if (out.wind_direction) ((float*)out.wind_direction)[o] = wdl;
@@ -571,7 +576,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
         rsum_l += __shfl_xor_sync(0xffffffffu, rsum_l, sft);
     }
     const bool any_flag = __any_sync(0xffffffffu, flagged);
-    if constexpr (EVAL) {  // no state is written: the flag and the power row of the candidate only
+    if constexpr (EVAL && !ACT) {  // no state is written: the flag and the power row of the candidate only
         if (lane == 0 && ev.amb) ev.amb[blockIdx.x] = (uint8_t)any_flag;
         if (any_flag && strict) {  // re-solved by the evaluation instantiation of wf_fixup64_kernel
             if (lane == 0) ev.fix_list[atomicAdd(&ev.fix_count[0], 1)] = blockIdx.x;
@@ -582,23 +587,34 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
         for (int tt = n + lane; tt < T; tt += 32) pw_out[tt] = 0.f;
         return;
     }
-    if (lane == 0 && s.amb) s.amb[b] = (uint8_t)any_flag;
-    if (any_flag && strict) {
+    if constexpr (ACT) {
+        if (lane == 0 && ev.amb) ev.amb[blockIdx.x] = (uint8_t)any_flag;
+        if (any_flag && strict) {  // re-solved by wf_fixup64_eval_kernel<W, true> from this transitioned yaw
+            for (int tt = lane; tt < n; tt += 32) ev.yaw[orow + tt] = (double)sm.ynew[tt];
+            if (lane == 0) ev.fix_list[atomicAdd(&ev.fix_count[0], 1)] = blockIdx.x;
+            return;
+        }
+    } else if (lane == 0 && s.amb) {
+        s.amb[b] = (uint8_t)any_flag;
+    }
+    if (!ACT && any_flag && strict) {
         // the FP64 re-solve (wf_fixup64_kernel, next launch on this stream) redoes this env from the committed yaw state and
         // commits the per-env epilogue state itself
         if (lane == 0) s.fix_list[atomicAdd(&s.fix_count[0], 1)] = b;
         return;
     }
+    // the per-env outputs go to row ob; an evaluation commits none of the state below
+    const int ob = ACT ? (int)blockIdx.x : b;
     int it = 0;
     if (lane == 0) {
         it = s.num_iter[b] + 1;
-        s.num_iter[b] = it;
-        if (out.truncated) out.truncated[b] = (uint8_t)(it == m.max_iter);
+        if (!ACT) s.num_iter[b] = it;
+        if (out.truncated) out.truncated[ob] = (uint8_t)(it == m.max_iter);
         float fw0 = ws, fw1 = wd;
         if (mode == WF_MODE_WARMUP) { fw0 = fclamp(fw0, 3.f, 28.f); fw1 = fclamp(fw1, 0.f, 360.f); }
-        if (out.freewind) ((float2*)out.freewind)[b] = make_float2(fw0, fw1);
+        if (out.freewind) ((float2*)out.freewind)[ob] = make_float2(fw0, fw1);
         if (mode == WF_MODE_ENV) {
-            s.num_moves[b] = nm;
+            if (!ACT) s.num_moves[b] = nm;
             const float wn = (float)s.ws_norm[b];
             const float invT = 1.f / (float)n;  // the mean over the env's own turbines
             float reward = rsum_p * 1e3f / (wn * wn * wn) * invT - fc.load_coef * rsum_l * (0.25f * invT);
@@ -607,18 +623,20 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
             } else if (m.shaper == 2) {
                 const double ref = s.shaper_ref[b];
                 const float shaped = (ref == 0.0) ? 0.f : (float)(((double)reward - ref) / ref);
-                s.shaper_ref[b] = (double)reward;
+                if (!ACT) s.shaper_ref[b] = (double)reward;
                 reward = shaped;
             }
-            if (!isfinite(reward)) s.nonfinite[b] += 1;
-            if (out.reward) ((float*)out.reward)[b] = reward;
-            wfreset::episode_account(s, b, (double)reward, it == m.max_iter);
-            s.ws_norm[b] = ws_d;
+            if (!ACT && !isfinite(reward)) s.nonfinite[b] += 1;
+            if (out.reward) ((float*)out.reward)[ob] = reward;
+            if (!ACT) {
+                wfreset::episode_account(s, b, (double)reward, it == m.max_iter);
+                s.ws_norm[b] = ws_d;
+            }
         }
     }
     // in-kernel auto-reset (wf_set_autoreset): the step that truncates also starts the env's next episode -- zero yaw /
     // accumulators / counters -- and marks the env for wf_autoreset_finish (wind draw + geometry + warm-up solve); the outputs written above remain the FINAL observation of the finished episode
-    if (mode == WF_MODE_ENV && m.autoreset && __shfl_sync(0xffffffffu, (int)(it == m.max_iter), 0)) {
+    if (!ACT && mode == WF_MODE_ENV && m.autoreset && __shfl_sync(0xffffffffu, (int)(it == m.max_iter), 0)) {
         for (int tt = lane; tt < T; tt += 32) { s.yaw[row + tt] = 0.0; s.acc[row + tt] = 0.f; s.acc_prev[row + tt] = 0.f; }
         if (lane == 0) wfreset::autoreset_mark(s, b);
     }
@@ -627,7 +645,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
     auto zero_padding = [&](void* p, const int w) {
         if (p)
 #pragma unroll 1
-            for (int q = n * w + lane; q < T * w; q += 32) ((float*)p)[row * w + q] = 0.f;
+            for (int q = n * w + lane; q < T * w; q += 32) ((float*)p)[orow * w + q] = 0.f;
     };
     zero_padding(out.yaw, 1);
     zero_padding(out.wind_speed, 1);
@@ -640,7 +658,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
 
 cudaError_t wf_configure_fast_kernels() {
     for (auto k : {wf_step_fast_kernel<true>, wf_step_fast_kernel<false>, wf_step_fast_kernel<true, true>,
-                   wf_step_fast_kernel<false, true>}) {
+                   wf_step_fast_kernel<false, true>, wf_step_fast_kernel<true, true, true>, wf_step_fast_kernel<false, true, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -658,20 +676,21 @@ static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& 
     return cudaGetLastError();
 }
 
-template <bool BAKED>
+template <bool BAKED, bool ACT>
 static cudaError_t launch_eval_t(const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
-                                 const double* d_yaw, void* d_power, cudaStream_t stream) {
-    WfStepOut out = {};
-    out.power = d_power;
-    wf_step_fast_kernel<BAKED, true><<<(unsigned)m.B * (unsigned)ev.K, 32, fast_smem_bytes(m.T), stream>>>(
-        WF_MODE_INTERFACE, 0, m, fc, s, nullptr, nullptr, d_yaw, out, ev);
+                                 const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream) {
+    wf_step_fast_kernel<BAKED, true, ACT><<<(unsigned)m.B * (unsigned)ev.K, 32, fast_smem_bytes(m.T), stream>>>(
+        ACT ? WF_MODE_ENV : WF_MODE_INTERFACE, 0, m, fc, s, nullptr, d_action, d_yaw, out, ev);
     return cudaGetLastError();
 }
 
 cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
-                                const double* d_yaw, void* d_power, cudaStream_t stream) {
-    return baked ? launch_eval_t<true>(m, fc, s, ev, d_yaw, d_power, stream)
-                 : launch_eval_t<false>(m, fc, s, ev, d_yaw, d_power, stream);
+                                const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream) {
+    if (d_action)
+        return baked ? launch_eval_t<true, true>(m, fc, s, ev, nullptr, d_action, out, stream)
+                     : launch_eval_t<false, true>(m, fc, s, ev, nullptr, d_action, out, stream);
+    return baked ? launch_eval_t<true, false>(m, fc, s, ev, d_yaw, nullptr, out, stream)
+                 : launch_eval_t<false, false>(m, fc, s, ev, d_yaw, nullptr, out, stream);
 }
 
 cudaError_t wf_launch_step_fast(int mode, bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s,

@@ -8,7 +8,8 @@
 //                                 deficit queue) for handles without a vortex table;
 //   wf_fixup64_kernel<W>          W warps per env, built for latency: a chain warp evaluates the sources' scalar chains back to
 //                                 back while W-1 worker warps apply the previous source to its targets (named barriers).
-// and their candidate-evaluation forms (wf_evaluate_yaw): wf_step_fast64_kernel<GATHER, true> and wf_fixup64_eval_kernel<W>.
+// and their candidate-evaluation forms: wf_step_fast64_kernel<GATHER, true> and wf_fixup64_eval_kernel<W> (wf_evaluate_yaw),
+// wf_step_fast64_kernel<GATHER, true, true> and wf_fixup64_eval_kernel<W, true> (wf_evaluate_actions).
 //
 // Everything is evaluated in double precision and every simplification of wf_fast.cu that would be visible at the 1e-9 level
 // is dropped:
@@ -190,7 +191,9 @@ __device__ __forceinline__ void load_row12(const double* __restrict__ p, double*
 // accumulators are committed) but none of the per-env epilogue state, which is committed here.
 // EVAL = candidate evaluation (wf_evaluate_yaw): candidate `cand` of env b, solved in interface mode with the yaw row `cand` of
 // `yaw_cmd`; its power goes to row `cand` of out.power, its flag to ev.amb[cand] (FIX: 1, else 0), and no state is written.
-template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false>
+// EVAL + ACT (wf_evaluate_actions): env b's step with the action row `cand` (FIX: from the transitioned yaw row `cand` of
+// ev.yaw), in the run-time mode of the step; every output goes to row `cand`, and the state is read and never written.
+template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false, bool ACT = false>
 __device__ __forceinline__ void solve_env64(const int b, const int mode, const bool use_vtab, const WfModel& m,
                                             const WfFastConst64& fc, const WfState& s, const float* __restrict__ action,
                                             const double* __restrict__ yaw_cmd, const WfStepOut& out,
@@ -201,6 +204,9 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     auto csync = [] { if (W == 1) __syncwarp(); else __syncthreads(); };
     const size_t row = (size_t)b * T;
     const size_t orow = EVAL ? (size_t)cand * T : row;  // row of the yaw command and of the outputs
+    // ACT: no state is committed, on a test of K (always > 0) the compiler cannot fold, for the reason given at the end of the
+    // interface-mode evaluation below: the commits stay in the code, and the floating-point contractions those of the step
+    const bool commit = !ACT || ev.K < 1;
     // the env's turbine count, the bound of every loop below; columns n..T-1 of its rows are padding (wf_device.cuh).
     // Shared memory and the table's row strides stay those of T.
     const int n = s.turbine_count[b];
@@ -221,8 +227,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     if (mode == WF_MODE_ENV) nm = s.num_moves[b] + 1;
     for (int tt = tid; tt < n; tt += NT) {
         double ynew;
-        if (!FIX && !EVAL && mode == WF_MODE_ENV) {
-            float a = action[row + tt];
+        if (!FIX && (!EVAL || ACT) && mode == WF_MODE_ENV) {
+            float a = action[orow + tt];
             const float acc = s.acc[row + tt];
             const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
             const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
@@ -231,10 +237,14 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             else a = __fmul_rn(__fsub_rn(a, 1.0f), m.yaw_step_f);
             const float y0 = fminf(fmaxf((float)s.yaw[row + tt], m.yaw_lo_f), m.yaw_hi_f);
             const float y1 = fminf(fmaxf(__fadd_rn(y0, a), m.yaw_lo_f), m.yaw_hi_f);
-            s.acc_prev[row + tt] = acc;
-            s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
+            if (commit) {
+                s.acc_prev[row + tt] = acc;
+                s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
+            }
             ynew = (double)y1;
-            s.yaw[row + tt] = ynew;
+            if (commit) s.yaw[row + tt] = ynew;
+        } else if (FIX && ACT) {
+            ynew = ev.yaw[orow + tt];
         } else if ((!FIX || EVAL) && mode == WF_MODE_INTERFACE && yaw_cmd) {
             ynew = yaw_cmd[orow + tt];
             if (!EVAL) s.yaw[row + tt] = ynew;
@@ -838,7 +848,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     // step instantiation and a candidate's power equals the step's bit for bit.  With a plain `return` the sums of the power
     // chain fused differently (1e-15 off the step, DESIGN.md section 5b).  This rests on the compiler's choices:
     // tests/test_evaluate_yaw_gpu.py::test_equals_interface_mode (f64 modes) catches a compiler that makes others.
-    if (EVAL && ev.K > 0) {
+    if (EVAL && !ACT && ev.K > 0) {
         if (lane == 0 && ev.amb) ev.amb[cand] = FIX ? 1 : 0;
         return;
     }
@@ -847,17 +857,19 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         rsum_p += __shfl_xor_sync(0xffffffffu, rsum_p, sft);
         rsum_l += __shfl_xor_sync(0xffffffffu, rsum_l, sft);
     }
+    // the per-env outputs go to row ob; an evaluation commits none of the state below
+    const int ob = ACT ? cand : b;
     int it = 0;
     if (lane == 0) {
         it = s.num_iter[b] + 1;
-        s.num_iter[b] = it;
-        if (out.truncated) out.truncated[b] = (uint8_t)(it == m.max_iter);
+        if (commit) s.num_iter[b] = it;
+        if (out.truncated) out.truncated[ob] = (uint8_t)(it == m.max_iter);
         double fw0 = ws, fw1 = wd;
         if (mode == WF_MODE_WARMUP) { fw0 = dclamp(fw0, 3.0, 28.0); fw1 = dclamp(fw1, 0.0, 360.0); }
-        if (out.freewind) { ((OutT*)out.freewind)[2 * b] = (OutT)fw0; ((OutT*)out.freewind)[2 * b + 1] = (OutT)fw1; }
+        if (out.freewind) { ((OutT*)out.freewind)[2 * ob] = (OutT)fw0; ((OutT*)out.freewind)[2 * ob + 1] = (OutT)fw1; }
         if (FIX && rec) { rec[0] = __int_as_float(b); rec[1] = 0.f; rec[2] = (float)fw0; rec[3] = (float)fw1; rec[4] = (it == m.max_iter) ? 1.f : 0.f; }
         if (mode == WF_MODE_ENV) {
-            s.num_moves[b] = nm;
+            if (commit) s.num_moves[b] = nm;
             const double wn = s.ws_norm[b];
             double reward = rsum_p * 1e3 / (wn * wn * wn) / n - m.load_coef * (rsum_l / (4.0 * n));  // mean over the env's turbines
             if (m.shaper == 1) {
@@ -865,19 +877,22 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             } else if (m.shaper == 2) {
                 const double ref = s.shaper_ref[b];
                 const double shaped = (ref == 0.0) ? 0.0 : (reward - ref) / ref;
-                s.shaper_ref[b] = reward;
+                if (commit) s.shaper_ref[b] = reward;
                 reward = shaped;
             }
-            if (!isfinite(reward)) s.nonfinite[b] += 1;
-            if (out.reward) ((OutT*)out.reward)[b] = (OutT)reward;
+            if (commit && !isfinite(reward)) s.nonfinite[b] += 1;
+            if (out.reward) ((OutT*)out.reward)[ob] = (OutT)reward;
             if (FIX && rec) rec[1] = (float)reward;
-            wfreset::episode_account(s, b, FIX ? (double)(float)reward : reward, it == m.max_iter);  // FIX: what the caller sees
-            s.ws_norm[b] = ws;
+            if (commit) {
+                wfreset::episode_account(s, b, FIX ? (double)(float)reward : reward, it == m.max_iter);  // FIX: what the caller sees
+                s.ws_norm[b] = ws;
+            }
         }
+        if (ACT && ev.amb) ev.amb[cand] = FIX ? 1 : 0;
     }
     // in-kernel auto-reset (see wf_fast.cu): the truncating step starts the env's next episode and marks it for
     // wf_autoreset_finish; the outputs above remain the final observation
-    if (mode == WF_MODE_ENV && m.autoreset && __shfl_sync(0xffffffffu, (int)(it == m.max_iter), 0)) {
+    if (commit && mode == WF_MODE_ENV && m.autoreset && __shfl_sync(0xffffffffu, (int)(it == m.max_iter), 0)) {
         for (int tt = lane; tt < T; tt += 32) { s.yaw[row + tt] = 0.0; s.acc[row + tt] = 0.f; s.acc_prev[row + tt] = 0.f; }
         if (lane == 0) wfreset::autoreset_mark(s, b);
     }
@@ -887,8 +902,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
 // sub-partition with two others (12 per SM), one of 128 registers with three (16 per SM; 12-48 bytes of spills).  The kernels
 // are latency-bound, throughput grows with the resident envs (measured on Turb32_Row5: 6 per SM 4.9 M env-steps/s, 9: 6.2 M,
 // 12: 7.6 M, 16: 8.2 M); at 80 turbines shared memory holds 14 envs of the gather kernel per SM (9 of the scatter kernel).
-// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw)
-template <bool GATHER, bool EVAL = false>
+// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw; ACT: wf_evaluate_actions)
+template <bool GATHER, bool EVAL = false, bool ACT = false>
 __global__ void __launch_bounds__(32, 16)
 wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                       const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
@@ -896,7 +911,7 @@ wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, 
     int b;
     if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
     if (mask && !mask[b]) return;
-    solve_env64<1, double, false, GATHER, EVAL>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
+    solve_env64<1, double, false, GATHER, EVAL, ACT>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
 }
 
 // Re-solve, in FP64, of the envs an FP32 launch flagged (their ids sit in s.fix_list[0, n), n in s.fix_count[0]); launched
@@ -926,14 +941,16 @@ wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __
 // Evaluation instantiation of the re-solve (wf_evaluate_yaw): the candidates an evaluation launch flagged (ev.fix_list /
 // ev.fix_count, candidate c = env c / K), with the yaw rows of `yaw_cmd`; they write their power row and flag and commit
 // nothing.  A kernel of its own rather than a flag of wf_fixup64_kernel, whose parameter list (and so code) stays as it was.
-template <int W>
+// ACT (wf_evaluate_actions): the candidates' transitioned yaw rows are in ev.yaw; the env-mode epilogue writes every output
+// row of the candidate, reward included, and commits nothing.
+template <int W, bool ACT = false>
 __global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
 wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc, const WfState s,
                        const WfStepOut out, const double* __restrict__ yaw_cmd, const WfEvalArgs ev) {
     const int n = *(volatile int*)&ev.fix_count[0];
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
         const int c = ev.fix_list[k];
-        solve_env64<W, float, true, false, true>(c / ev.K, mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
+        solve_env64<W, float, true, false, true, ACT>(c / ev.K, mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
         __syncthreads();
     }
     if (threadIdx.x == 0) {  // the last CTA to leave re-arms the evaluation counters
@@ -951,7 +968,8 @@ wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, con
 // Dynamic shared memory up to 100 KB for every FP64 kernel; the step kernels also prefer the largest shared-memory carveout.
 cudaError_t wf_configure_fast64_kernels() {
     for (auto k : {wf_step_fast64_kernel<false>, wf_step_fast64_kernel<true>, wf_step_fast64_kernel<false, true>,
-                   wf_step_fast64_kernel<true, true>}) {
+                   wf_step_fast64_kernel<true, true>, wf_step_fast64_kernel<false, true, true>,
+                   wf_step_fast64_kernel<true, true, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -961,7 +979,9 @@ cudaError_t wf_configure_fast64_kernels() {
         const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e != cudaSuccess) return e;
     }
-    for (auto k : {wf_fixup64_eval_kernel<1>, wf_fixup64_eval_kernel<2>, wf_fixup64_eval_kernel<4>, wf_fixup64_eval_kernel<8>}) {
+    for (auto k : {wf_fixup64_eval_kernel<1>, wf_fixup64_eval_kernel<2>, wf_fixup64_eval_kernel<4>, wf_fixup64_eval_kernel<8>,
+                   wf_fixup64_eval_kernel<1, true>, wf_fixup64_eval_kernel<2, true>, wf_fixup64_eval_kernel<4, true>,
+                   wf_fixup64_eval_kernel<8, true>}) {
         const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e != cudaSuccess) return e;
     }
@@ -972,7 +992,9 @@ template <int W, bool EVAL>
 static cudaError_t launch_fixup_t(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const WfStepOut& out, int grid, float* d_rec, int rec_cap, const double* d_yaw,
                                   const WfEvalArgs& ev, cudaStream_t stream) {
-    if (EVAL)
+    if (EVAL && mode == WF_MODE_ENV)
+        wf_fixup64_eval_kernel<W, true><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_yaw, ev);
+    else if (EVAL)
         wf_fixup64_eval_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_yaw, ev);
     else
         wf_fixup64_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_rec, rec_cap);
@@ -1008,10 +1030,10 @@ cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const W
 
 // W is chosen from the B*K CTAs of the evaluation launch by the step's rule
 cudaError_t wf_launch_eval_fixup64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                   const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream) {
-    WfStepOut out = {};
-    out.power = d_power;
-    return launch_fixup_sized<true>(WF_MODE_INTERFACE, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0, d_yaw, ev, stream);
+                                   const WfEvalArgs& ev, const double* d_yaw, bool actions, const WfStepOut& out,
+                                   cudaStream_t stream) {
+    return launch_fixup_sized<true>(actions ? WF_MODE_ENV : WF_MODE_INTERFACE, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0,
+                                    d_yaw, ev, stream);
 }
 
 bool wf_fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
@@ -1032,14 +1054,19 @@ cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, con
 }
 
 cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                  const WfEvalArgs& ev, const double* d_yaw, void* d_power, cudaStream_t stream) {
+                                  const WfEvalArgs& ev, const double* d_yaw, const float* d_action, const WfStepOut& out,
+                                  cudaStream_t stream) {
     // the same form as the step kernel of this handle in its current state (a stale table: the scatter form, pairs direct)
     const bool gather = wf_fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
     const unsigned grid = (unsigned)m.B * (unsigned)ev.K;
-    WfStepOut out = {};
-    out.power = d_power;
-    if (gather)
+    if (d_action && gather)  // the mode stays a run-time argument, as in the step (DESIGN.md section 5b)
+        wf_step_fast64_kernel<true, true, true><<<grid, 32, smem, stream>>>(WF_MODE_ENV, 0, true, m, fc, s, nullptr, d_action,
+                                                                            nullptr, out, ev);
+    else if (d_action)
+        wf_step_fast64_kernel<false, true, true><<<grid, 32, smem, stream>>>(WF_MODE_ENV, 0, use_vtab, m, fc, s, nullptr, d_action,
+                                                                             nullptr, out, ev);
+    else if (gather)
         wf_step_fast64_kernel<true, true><<<grid, 32, smem, stream>>>(WF_MODE_INTERFACE, 0, true, m, fc, s, nullptr, nullptr, d_yaw,
                                                                       out, ev);
     else

@@ -331,6 +331,33 @@ class VecWindFarmEnv:
         self.last_info = info  # joint (un-split) info of this step, incl. final_observation on auto-reset steps
         return obs, reward, self._zeros_bool, truncated, info
 
+    def evaluate_actions(self, action):
+        """One-step lookahead: what ``step`` would return for each of K candidate actions per env, from where each env is
+        now, without stepping (``FlorisBatch.evaluate_actions``).  ``action``: [B, K, T] (or ``{"yaw": ...}``).  Returns
+        ``(obs, reward, terminated, truncated, info)`` with a K axis after the batch axis, exactly as ``step`` would return
+        them for each candidate, without the auto-reset handling: a candidate that truncates reports ``truncated`` and its
+        final observation, and nothing is reset.  The env's state, its cohort countdowns included, does not change.
+        Views of buffers the next call overwrites unless ``copy_outputs``.  Not available in wind-time-series mode, where a
+        step moves the wind before it solves."""
+        assert not self._needs_reset, "Call reset before `evaluate_actions`"
+        if self._series is not None:
+            raise ValueError("evaluate_actions is not available in wind-time-series mode: a step there moves the wind (and "
+                             "the geometry) before it solves, which an evaluation cannot do without changing the state")
+        if isinstance(action, dict):
+            action = action["yaw"]
+        if not torch.is_tensor(action):
+            action = torch.as_tensor(np.asarray(action, dtype=np.float32), device=self.device)
+        out = self.backend.evaluate_actions(action.to(device=self.device, dtype=torch.float32).contiguous())
+        c = (lambda t: t.clone()) if self.copy_outputs else (lambda t: t)
+        obs = OrderedDict([("yaw", c(out["yaw"])), ("freewind_measurements", c(out["freewind"])),
+                           ("wind_speed", c(out["wind_speed"])), ("wind_direction", c(out["wind_direction"]))])
+        K = out["reward"].shape[1]
+        if self.pad_turbines:
+            obs["turbine_mask"] = self._turbine_mask[:, None, :].expand(-1, K, -1)
+        terminated = torch.zeros(self.num_envs, K, dtype=torch.bool, device=self.device)
+        info = {"power": c(out["power"]), "load": c(out["load"])}
+        return obs, c(out["reward"]), terminated, c(out["truncated"].view(torch.bool)), info
+
     @property
     def layout_ids(self):
         """Index into the layout list of the layout every env currently runs (int32 [B], device copy)."""
@@ -401,4 +428,17 @@ class VecMAWindFarmEnv(VecWindFarmEnv):
         per_agent_info = {a: {"power": info["power"][:, i], "load": info["load"][:, i]}
                           for a, i in self.agent_name_mapping.items()}
         return (self._split(obs), {a: reward for a in self.possible_agents}, {a: terminated for a in self.possible_agents},
+                {a: truncated for a in self.possible_agents}, per_agent_info)
+
+    def evaluate_actions(self, actions):
+        """``VecWindFarmEnv.evaluate_actions`` for the agents: ``actions`` is the joint float32 [B, K, T] tensor (column
+        k = agent k) or ``{agent: {"yaw": tensor[B, K]}}``; returns per-agent dicts as ``step`` does, with the K axis."""
+        if isinstance(actions, dict) and actions and next(iter(actions)) in self.agent_name_mapping:
+            actions = torch.stack([torch.as_tensor(actions[a]["yaw"], device=self.device) for a in self.possible_agents], 2)
+        obs, reward, terminated, truncated, info = super().evaluate_actions(actions)
+        split = {a: OrderedDict((k, v[:, :, i]) for k, v in obs.items() if k != "freewind_measurements")
+                 for a, i in self.agent_name_mapping.items()}
+        per_agent_info = {a: {"power": info["power"][:, :, i], "load": info["load"][:, :, i]}
+                          for a, i in self.agent_name_mapping.items()}
+        return (split, {a: reward for a in self.possible_agents}, {a: terminated for a in self.possible_agents},
                 {a: truncated for a in self.possible_agents}, per_agent_info)
