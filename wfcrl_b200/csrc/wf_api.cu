@@ -691,7 +691,8 @@ static int evaluate(WfHandle h, const char* fn, const double* d_yaw, const float
         e = wf_launch_eval_fast(h->fast_baked, h->model, h->fast, h->st, ev, d_yaw, d_action, out, st);
         h->launches += 1;
         if (e == cudaSuccess && is_strict_f32(h)) {
-            e = wf_launch_eval_fixup64(use_vtab, h->model, h->fast64, h->st, ev, d_yaw, d_action != nullptr, out, st);
+            e = wf_launch_eval_fixup64(d_action ? WF_MODE_ENV : WF_MODE_INTERFACE, use_vtab, h->model, h->fast64, h->st, ev,
+                                       d_yaw, out, st);
             h->launches += 1;
         }
     }

@@ -188,14 +188,14 @@ cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, con
 cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                       int* smem);
 // candidate evaluation: one launch of B*K CTAs with out's buffers of B*K rows; on a strict FP32 handle wf_launch_eval_fixup64
-// re-solves the flagged candidates (ev.fix_list) in FP64.  d_action == NULL: yaw candidates d_yaw [B*K][T] in interface mode,
-// out.power only (wf_evaluate_yaw); else action candidates d_action [B*K][T] in env mode, every output (wf_evaluate_actions)
+// re-solves the flagged candidates (ev.fix_list) in FP64, in the evaluation's mode.  d_action == NULL: yaw candidates d_yaw
+// [B*K][T] in interface mode, out.power only (wf_evaluate_yaw); else action candidates d_action [B*K][T] in env mode, every
+// output (wf_evaluate_actions)
 cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
                                 const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream);
 cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const WfEvalArgs& ev, const double* d_yaw, const float* d_action, const WfStepOut& out,
                                   cudaStream_t stream);
-cudaError_t wf_launch_eval_fixup64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                   const WfEvalArgs& ev, const double* d_yaw, bool actions, const WfStepOut& out,
-                                   cudaStream_t stream);
+cudaError_t wf_launch_eval_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
+                                   const WfEvalArgs& ev, const double* d_yaw, const WfStepOut& out, cudaStream_t stream);
 bool wf_fast64_gathers(const WfModel& m, const WfState& s);  // an FP64 handle's step kernel runs the gather form

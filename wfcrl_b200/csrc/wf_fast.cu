@@ -128,7 +128,10 @@ struct wf_false_tag { static constexpr bool value = false; };
 // row c of `out.power` and nothing else, and hands a flagged candidate to the evaluation fix list (wf_device.cuh: WfEvalArgs)
 // EVAL + ACT (wf_evaluate_actions): CTA c runs env b = c / K's step with action row c in the run-time mode (env) of the step --
 // transition, solve, epilogue and reward -- against b's state, which it reads and never writes; every output goes to row c.
-// A flagged candidate leaves its transitioned yaw in ev.yaw row c for the re-solve
+// A flagged candidate leaves its transitioned yaw in ev.yaw row c for the re-solve.
+// Unlike the FP64 kernels, this kernel keeps yaw evaluation an instantiation of its own (EVAL without ACT), with the mode a
+// compile-time constant: with the env-mode epilogue (wind direction, loads, reward) compiled in, FP32 yaw evaluation ran
+// 1-3 % slower (DESIGN.md section 5b)
 template <bool BAKED, bool EVAL = false, bool ACT = false>
 __global__ void __launch_bounds__(32, BAKED ? 16 : 12)
 wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
@@ -578,7 +581,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
     const bool any_flag = __any_sync(0xffffffffu, flagged);
     if constexpr (EVAL && !ACT) {  // no state is written: the flag and the power row of the candidate only
         if (lane == 0 && ev.amb) ev.amb[blockIdx.x] = (uint8_t)any_flag;
-        if (any_flag && strict) {  // re-solved by the evaluation instantiation of wf_fixup64_kernel
+        if (any_flag && strict) {  // re-solved in interface mode by wf_fixup64_eval_kernel, from the caller's yaw_cmd row
             if (lane == 0) ev.fix_list[atomicAdd(&ev.fix_count[0], 1)] = blockIdx.x;
             return;
         }
@@ -589,7 +592,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
     }
     if constexpr (ACT) {
         if (lane == 0 && ev.amb) ev.amb[blockIdx.x] = (uint8_t)any_flag;
-        if (any_flag && strict) {  // re-solved by wf_fixup64_eval_kernel<W, true> from this transitioned yaw
+        if (any_flag && strict) {  // re-solved in env mode by wf_fixup64_eval_kernel, from this transitioned yaw
             for (int tt = lane; tt < n; tt += 32) ev.yaw[orow + tt] = (double)sm.ynew[tt];
             if (lane == 0) ev.fix_list[atomicAdd(&ev.fix_count[0], 1)] = blockIdx.x;
             return;

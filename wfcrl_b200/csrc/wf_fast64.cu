@@ -8,8 +8,8 @@
 //                                 deficit queue) for handles without a vortex table;
 //   wf_fixup64_kernel<W>          W warps per env, built for latency: a chain warp evaluates the sources' scalar chains back to
 //                                 back while W-1 worker warps apply the previous source to its targets (named barriers).
-// and their candidate-evaluation forms: wf_step_fast64_kernel<GATHER, true> and wf_fixup64_eval_kernel<W> (wf_evaluate_yaw),
-// wf_step_fast64_kernel<GATHER, true, true> and wf_fixup64_eval_kernel<W, true> (wf_evaluate_actions).
+// and their candidate-evaluation forms wf_step_fast64_kernel<GATHER, true> and wf_fixup64_eval_kernel<W> (wf_evaluate_yaw in
+// interface mode, wf_evaluate_actions in env mode).
 //
 // Everything is evaluated in double precision and every simplification of wf_fast.cu that would be visible at the 1e-9 level
 // is dropped:
@@ -189,11 +189,11 @@ __device__ __forceinline__ void load_row12(const double* __restrict__ p, double*
 //          12 envs share an SM instead of 9.
 // OutT = type of the caller's output buffers (double for an FP64 handle, float for the re-solve on an FP32 handle).  FIX = re-solve: the FP32 kernel has already applied the action (yaw and
 // accumulators are committed) but none of the per-env epilogue state, which is committed here.
-// EVAL = candidate evaluation (wf_evaluate_yaw): candidate `cand` of env b, solved in interface mode with the yaw row `cand` of
-// `yaw_cmd`; its power goes to row `cand` of out.power, its flag to ev.amb[cand] (FIX: 1, else 0), and no state is written.
-// EVAL + ACT (wf_evaluate_actions): env b's step with the action row `cand` (FIX: from the transitioned yaw row `cand` of
-// ev.yaw), in the run-time mode of the step; every output goes to row `cand`, and the state is read and never written.
-template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false, bool ACT = false>
+// EVAL = candidate evaluation: env b's step for candidate `cand`, in the run-time mode of the step; every output goes to row
+// `cand`, its flag to ev.amb[cand] (FIX: 1, else 0), and the state is read and never written.  Env mode (wf_evaluate_actions):
+// the action row `cand` (FIX: the transitioned yaw row `cand` of ev.yaw).  Interface mode (wf_evaluate_yaw): the yaw row
+// `cand` of `yaw_cmd`.
+template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false>
 __device__ __forceinline__ void solve_env64(const int b, const int mode, const bool use_vtab, const WfModel& m,
                                             const WfFastConst64& fc, const WfState& s, const float* __restrict__ action,
                                             const double* __restrict__ yaw_cmd, const WfStepOut& out,
@@ -204,9 +204,12 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     auto csync = [] { if (W == 1) __syncwarp(); else __syncthreads(); };
     const size_t row = (size_t)b * T;
     const size_t orow = EVAL ? (size_t)cand * T : row;  // row of the yaw command and of the outputs
-    // ACT: no state is committed, on a test of K (always > 0) the compiler cannot fold, for the reason given at the end of the
-    // interface-mode evaluation below: the commits stay in the code, and the floating-point contractions those of the step
-    const bool commit = !ACT || ev.K < 1;
+    // EVAL: no state is committed, on a test of K (always > 0) the compiler cannot fold.  The commits stay in the code, so the
+    // compiler makes the same floating-point contractions as in the step and a candidate's outputs equal the step's bit for
+    // bit; with the commits compiled out, multiply-adds fused differently (1 ulp off the step, DESIGN.md section 5b).  This
+    // rests on the compiler's choices: the bit-equality tests of both evaluations (tests/test_evaluate_yaw_gpu.py,
+    // tests/test_evaluate_actions_gpu.py) catch a compiler that makes others
+    const bool commit = !EVAL || ev.K < 1;
     // the env's turbine count, the bound of every loop below; columns n..T-1 of its rows are padding (wf_device.cuh).
     // Shared memory and the table's row strides stay those of T.
     const int n = s.turbine_count[b];
@@ -227,7 +230,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     if (mode == WF_MODE_ENV) nm = s.num_moves[b] + 1;
     for (int tt = tid; tt < n; tt += NT) {
         double ynew;
-        if (!FIX && (!EVAL || ACT) && mode == WF_MODE_ENV) {
+        if (!FIX && mode == WF_MODE_ENV) {
             float a = action[orow + tt];
             const float acc = s.acc[row + tt];
             const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
@@ -243,7 +246,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             }
             ynew = (double)y1;
             if (commit) s.yaw[row + tt] = ynew;
-        } else if (FIX && ACT) {
+        } else if (FIX && EVAL && mode == WF_MODE_ENV) {
+            // the FP32 launch's transitioned yaw; an interface-mode candidate reads the caller's yaw_cmd below
             ynew = ev.yaw[orow + tt];
         } else if ((!FIX || EVAL) && mode == WF_MODE_INTERFACE && yaw_cmd) {
             ynew = yaw_cmd[orow + tt];
@@ -843,22 +847,13 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
             r[4 * T + 4 * tt] = 0.f; r[4 * T + 4 * tt + 1] = 0.f; r[4 * T + 4 * tt + 2] = 0.f; r[4 * T + 4 * tt + 3] = 0.f;
         }
     }
-    // nothing of the epilogue state: no counters, no reward, no auto-reset.  The test of K (always > 0) keeps the code below
-    // alive in the evaluation instantiation, so that the compiler makes the same floating-point contractions above as in the
-    // step instantiation and a candidate's power equals the step's bit for bit.  With a plain `return` the sums of the power
-    // chain fused differently (1e-15 off the step, DESIGN.md section 5b).  This rests on the compiler's choices:
-    // tests/test_evaluate_yaw_gpu.py::test_equals_interface_mode (f64 modes) catches a compiler that makes others.
-    if (EVAL && !ACT && ev.K > 0) {
-        if (lane == 0 && ev.amb) ev.amb[cand] = FIX ? 1 : 0;
-        return;
-    }
 #pragma unroll
     for (int sft = 16; sft > 0; sft >>= 1) {
         rsum_p += __shfl_xor_sync(0xffffffffu, rsum_p, sft);
         rsum_l += __shfl_xor_sync(0xffffffffu, rsum_l, sft);
     }
     // the per-env outputs go to row ob; an evaluation commits none of the state below
-    const int ob = ACT ? cand : b;
+    const int ob = EVAL ? cand : b;
     int it = 0;
     if (lane == 0) {
         it = s.num_iter[b] + 1;
@@ -888,7 +883,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
                 s.ws_norm[b] = ws;
             }
         }
-        if (ACT && ev.amb) ev.amb[cand] = FIX ? 1 : 0;
+        if (EVAL && ev.amb) ev.amb[cand] = FIX ? 1 : 0;
     }
     // in-kernel auto-reset (see wf_fast.cu): the truncating step starts the env's next episode and marks it for
     // wf_autoreset_finish; the outputs above remain the final observation
@@ -902,8 +897,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
 // sub-partition with two others (12 per SM), one of 128 registers with three (16 per SM; 12-48 bytes of spills).  The kernels
 // are latency-bound, throughput grows with the resident envs (measured on Turb32_Row5: 6 per SM 4.9 M env-steps/s, 9: 6.2 M,
 // 12: 7.6 M, 16: 8.2 M); at 80 turbines shared memory holds 14 envs of the gather kernel per SM (9 of the scatter kernel).
-// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw; ACT: wf_evaluate_actions)
-template <bool GATHER, bool EVAL = false, bool ACT = false>
+// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw in interface mode, wf_evaluate_actions in env mode)
+template <bool GATHER, bool EVAL = false>
 __global__ void __launch_bounds__(32, 16)
 wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                       const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
@@ -911,7 +906,7 @@ wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, 
     int b;
     if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
     if (mask && !mask[b]) return;
-    solve_env64<1, double, false, GATHER, EVAL, ACT>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
+    solve_env64<1, double, false, GATHER, EVAL>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
 }
 
 // Re-solve, in FP64, of the envs an FP32 launch flagged (their ids sit in s.fix_list[0, n), n in s.fix_count[0]); launched
@@ -938,19 +933,18 @@ wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __
     }
 }
 
-// Evaluation instantiation of the re-solve (wf_evaluate_yaw): the candidates an evaluation launch flagged (ev.fix_list /
-// ev.fix_count, candidate c = env c / K), with the yaw rows of `yaw_cmd`; they write their power row and flag and commit
-// nothing.  A kernel of its own rather than a flag of wf_fixup64_kernel, whose parameter list (and so code) stays as it was.
-// ACT (wf_evaluate_actions): the candidates' transitioned yaw rows are in ev.yaw; the env-mode epilogue writes every output
-// row of the candidate, reward included, and commits nothing.
-template <int W, bool ACT = false>
+// Evaluation instantiation of the re-solve: the candidates an evaluation launch flagged (ev.fix_list / ev.fix_count,
+// candidate c = env c / K), from the transitioned yaw rows in ev.yaw (env mode, wf_evaluate_actions) or the yaw rows of
+// `yaw_cmd` (interface mode, wf_evaluate_yaw); they write every output row of the candidate and its flag and commit nothing.
+// A kernel of its own rather than a flag of wf_fixup64_kernel, whose parameter list (and so code) stays as it was.
+template <int W>
 __global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
 wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc, const WfState s,
                        const WfStepOut out, const double* __restrict__ yaw_cmd, const WfEvalArgs ev) {
     const int n = *(volatile int*)&ev.fix_count[0];
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
         const int c = ev.fix_list[k];
-        solve_env64<W, float, true, false, true, ACT>(c / ev.K, mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
+        solve_env64<W, float, true, false, true>(c / ev.K, mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
         __syncthreads();
     }
     if (threadIdx.x == 0) {  // the last CTA to leave re-arms the evaluation counters
@@ -968,8 +962,7 @@ wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, con
 // Dynamic shared memory up to 100 KB for every FP64 kernel; the step kernels also prefer the largest shared-memory carveout.
 cudaError_t wf_configure_fast64_kernels() {
     for (auto k : {wf_step_fast64_kernel<false>, wf_step_fast64_kernel<true>, wf_step_fast64_kernel<false, true>,
-                   wf_step_fast64_kernel<true, true>, wf_step_fast64_kernel<false, true, true>,
-                   wf_step_fast64_kernel<true, true, true>}) {
+                   wf_step_fast64_kernel<true, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -979,9 +972,7 @@ cudaError_t wf_configure_fast64_kernels() {
         const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e != cudaSuccess) return e;
     }
-    for (auto k : {wf_fixup64_eval_kernel<1>, wf_fixup64_eval_kernel<2>, wf_fixup64_eval_kernel<4>, wf_fixup64_eval_kernel<8>,
-                   wf_fixup64_eval_kernel<1, true>, wf_fixup64_eval_kernel<2, true>, wf_fixup64_eval_kernel<4, true>,
-                   wf_fixup64_eval_kernel<8, true>}) {
+    for (auto k : {wf_fixup64_eval_kernel<1>, wf_fixup64_eval_kernel<2>, wf_fixup64_eval_kernel<4>, wf_fixup64_eval_kernel<8>}) {
         const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e != cudaSuccess) return e;
     }
@@ -992,9 +983,7 @@ template <int W, bool EVAL>
 static cudaError_t launch_fixup_t(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                   const WfStepOut& out, int grid, float* d_rec, int rec_cap, const double* d_yaw,
                                   const WfEvalArgs& ev, cudaStream_t stream) {
-    if (EVAL && mode == WF_MODE_ENV)
-        wf_fixup64_eval_kernel<W, true><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_yaw, ev);
-    else if (EVAL)
+    if (EVAL)
         wf_fixup64_eval_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_yaw, ev);
     else
         wf_fixup64_kernel<W><<<grid, 32 * W, fast64_smem_bytes(m.T), stream>>>(mode, use_vtab, m, fc, s, out, d_rec, rec_cap);
@@ -1029,11 +1018,9 @@ cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const W
 }
 
 // W is chosen from the B*K CTAs of the evaluation launch by the step's rule
-cudaError_t wf_launch_eval_fixup64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
-                                   const WfEvalArgs& ev, const double* d_yaw, bool actions, const WfStepOut& out,
-                                   cudaStream_t stream) {
-    return launch_fixup_sized<true>(actions ? WF_MODE_ENV : WF_MODE_INTERFACE, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0,
-                                    d_yaw, ev, stream);
+cudaError_t wf_launch_eval_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
+                                   const WfEvalArgs& ev, const double* d_yaw, const WfStepOut& out, cudaStream_t stream) {
+    return launch_fixup_sized<true>(mode, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0, d_yaw, ev, stream);
 }
 
 bool wf_fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
@@ -1060,18 +1047,11 @@ cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastC
     const bool gather = wf_fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
     const unsigned grid = (unsigned)m.B * (unsigned)ev.K;
-    if (d_action && gather)  // the mode stays a run-time argument, as in the step (DESIGN.md section 5b)
-        wf_step_fast64_kernel<true, true, true><<<grid, 32, smem, stream>>>(WF_MODE_ENV, 0, true, m, fc, s, nullptr, d_action,
-                                                                            nullptr, out, ev);
-    else if (d_action)
-        wf_step_fast64_kernel<false, true, true><<<grid, 32, smem, stream>>>(WF_MODE_ENV, 0, use_vtab, m, fc, s, nullptr, d_action,
-                                                                             nullptr, out, ev);
-    else if (gather)
-        wf_step_fast64_kernel<true, true><<<grid, 32, smem, stream>>>(WF_MODE_INTERFACE, 0, true, m, fc, s, nullptr, nullptr, d_yaw,
-                                                                      out, ev);
+    const int mode = d_action ? WF_MODE_ENV : WF_MODE_INTERFACE;
+    if (gather)
+        wf_step_fast64_kernel<true, true><<<grid, 32, smem, stream>>>(mode, 0, true, m, fc, s, nullptr, d_action, d_yaw, out, ev);
     else
-        wf_step_fast64_kernel<false, true><<<grid, 32, smem, stream>>>(WF_MODE_INTERFACE, 0, use_vtab, m, fc, s, nullptr, nullptr,
-                                                                       d_yaw, out, ev);
+        wf_step_fast64_kernel<false, true><<<grid, 32, smem, stream>>>(mode, 0, use_vtab, m, fc, s, nullptr, d_action, d_yaw, out, ev);
     return cudaGetLastError();
 }
 
