@@ -277,6 +277,39 @@ int wf_evaluate_actions(WfHandle h, const float* d_action, int32_t K, const WfSt
                         void* stream);
 
 /*
+ * ROLLOUT EVALUATION (open-loop H-step lookahead).  What H successive wf_step calls would return for each of K candidate
+ * action sequences per env, from where each env is now, without stepping: the model query of MPC, random shooting, the
+ * cross-entropy method and H-step model-based RL.  wf_evaluate_actions is the case H = 1.
+ *   d_action:    DEVICE float [B][K][H][T]: row (b, k, h) is env b's action at step h of candidate k, each [T] row
+ *                interpreted exactly as wf_step interprets d_action
+ *   out:         a WfStepOut whose buffers have B*K*H rows: real [B][K][H][T] yaw, wind_speed, wind_direction, power,
+ *                real [B][K][H][T][4] load, real [B][K][H] reward, uint8 [B][K][H] truncated, real [B][K][H][2] freewind.
+ *                Any member may be NULL (a planner needs reward and truncated only).  Env-mode units.
+ *   d_ambiguous: DEVICE uint8 [B][K][H] or NULL: 1 = the row was re-solved by the FP64 kernel (strict FP32 handle)
+ * WF_KERNEL_FAST handles only.  Asynchronous on `stream`.
+ *  - Results: row (b, k, h) of every output equals, bit for bit, row b of what the (h+1)-th of H successive wf_step calls
+ *    would write on this handle in its current state with env b's actions d_action[b][k][0..h]: the transition chain with
+ *    the actuation constraint (acc, num_moves, acc_prev on multi-agent handles) firing at any step, the reward normalised
+ *    by the stored ws_norm at h = 0 and by ws after, both shapers with StepPercentage chained through the rollout (its
+ *    reference at h >= 1 is the previous row's unshaped reward, as the step commits it), load_coef,
+ *    truncated = (num_iter + h + 1 == max_iter), and rows that a strict FP32 handle flags and re-solves in FP64.
+ *  - Truncation: a candidate's rollout ends with its first truncating step; every later row is not solved and all its
+ *    outputs (reward, truncated, freewind and d_ambiguous included) are written as 0.  An env already past max_iter never
+ *    truncates and all its rows are evaluated.  Nothing continues into a next episode.
+ *  - State, layout pools of mixed counts, multi-agent handles, auto-reset precondition: as wf_evaluate_actions.
+ *  - Launches (counted in wf_launch_count): one, plus one FP64 re-solve launch on a strict FP32 handle, plus one
+ *    reward-chaining launch with the StepPercentage shaper when H > 1 and out->reward is not NULL.
+ *  - Scratch: shared with wf_evaluate_yaw and wf_evaluate_actions and sized in rows (B*K*H; calls of the three may be
+ *    interleaved); the first call with more rows than before allocates, synchronously: 4 bytes per row, plus 9T*16 bytes
+ *    per row on an FP64 handle with the vortex table (11.5 KB at T = 80), plus 8T bytes per row on a strict FP32 handle,
+ *    plus 8 bytes per row with the StepPercentage shaper.  1024 HornsRev1 envs x K = 16 x H = 8 on an FP64 handle: 1.5 GB.
+ * Refused with WF_ERR_INVALID before any work: WF_KERNEL_BASIC handles, K < 1, H < 1, NULL d_action or out, and
+ * B*K*H > 2^31 - 1.
+ */
+int wf_evaluate_rollouts(WfHandle h, const float* d_action, int32_t K, int32_t H, const WfStepOut* out,
+                         uint8_t* d_ambiguous, void* stream);
+
+/*
  * End-to-end convenience for hosts without device buffers: `h_action` (float [B][T]) in, wf_step, every non-NULL
  * member of `h_out` out, synchronous.  Two routes, same results bit for bit:
  *   - staged: cudaMemcpyAsync into device staging owned by the handle, 6 env chunks on 6 streams so the copies of one

@@ -94,7 +94,8 @@ class FlorisBatch:
         self._out_struct = _out_struct(self.out)
         self._host = None
         self.eval_capacity = 0  # largest K evaluate_yaw has run with (its output buffers and the library scratch hold that)
-        self.act_capacity, self._act_bufs = 0, None  # the same for evaluate_actions
+        # output name -> flat buffer, grown on demand: one set for evaluate_actions, one for evaluate_rollouts
+        self._act_bufs, self._roll_bufs = {}, {}
 
     # ------------------------------------------------------------------------------------------------------
     def close(self):
@@ -255,30 +256,52 @@ class FlorisBatch:
 
     def evaluate_actions(self, action: torch.Tensor) -> Dict[str, torch.Tensor]:
         """What ``step`` would return for each of K candidate actions per env, from the current state, without stepping
-        (``wf_evaluate_actions``).  ``action``: contiguous float32 CUDA tensor [B, K, T], each [T] row interpreted as
-        ``step`` interprets one; padding columns of a mixed-count pool are ignored.  Returns the eight step outputs with a K
-        axis after the batch axis (``yaw`` [B, K, T], ..., ``load`` [B, K, T, 4], ``reward`` / ``truncated`` [B, K],
-        ``freewind`` [B, K, 2]; env-mode units) and ``"ambiguous"`` bool [B, K], views of buffers owned by the batch that
-        the next call overwrites.  No state changes.  Asynchronous; the first call with a larger K than before allocates,
-        synchronously."""
+        (``wf_evaluate_actions``; ``evaluate_rollouts`` with H = 1).  ``action``: contiguous float32 CUDA tensor [B, K, T],
+        each [T] row interpreted as ``step`` interprets one; padding columns of a mixed-count pool are ignored.  Returns the
+        eight step outputs with a K axis after the batch axis (``yaw`` [B, K, T], ..., ``load`` [B, K, T, 4], ``reward`` /
+        ``truncated`` [B, K], ``freewind`` [B, K, 2]; env-mode units) and ``"ambiguous"`` bool [B, K], views of buffers
+        owned by the batch that the next call overwrites.  No state changes.  Asynchronous; the first call with a larger K
+        than before allocates, synchronously."""
         if not (torch.is_tensor(action) and action.dtype == torch.float32 and action.is_cuda and action.is_contiguous()):
             raise TypeError("action must be a contiguous float32 CUDA tensor of shape [B, K, T]")
         if action.dim() != 3 or action.shape[0] != self.B or action.shape[2] != self.T or action.shape[1] < 1:
             raise ValueError(f"action must have shape ({self.B}, K, {self.T}) with K >= 1, got {tuple(action.shape)}")
-        K = int(action.shape[1])
-        kinds = dict(_OUTPUTS, ambiguous="B")
-        bufs = self._act_bufs
-        if K > self.act_capacity:
-            bufs = {k: torch.zeros((self.B, K) + self._shape(kind)[1:], device=self.device,
-                                   dtype=torch.uint8 if k in ("truncated", "ambiguous") else self.real)
-                    for k, kind in kinds.items()}
-        res = {k: bufs[k].view(-1)[: self.B * K * bufs[k][0, 0].numel()].view((self.B, K) + bufs[k].shape[2:])
-               for k in kinds}
+        return {k: v[:, :, 0] for k, v in self._evaluate(action[:, :, None], tuple(_OUTPUTS), self._act_bufs).items()}
+
+    def evaluate_rollouts(self, action: torch.Tensor, fields=tuple(_OUTPUTS)) -> Dict[str, torch.Tensor]:
+        """What H successive ``step`` calls would return for each of K candidate action sequences per env, from the
+        current state, without stepping (``wf_evaluate_rollouts``).  ``action``: contiguous float32 CUDA tensor
+        [B, K, H, T]; row [b, k, h] is env b's action at step h of candidate k.  Returns the step outputs named in
+        ``fields`` with K and H axes after the batch axis (``yaw`` [B, K, H, T], ..., ``reward`` / ``truncated`` [B, K, H])
+        and ``"ambiguous"`` bool [B, K, H]; outputs not in ``fields`` are neither computed into a buffer nor allocated.  A
+        candidate's rollout ends with its first truncating step: the rows after it read 0.  Views of buffers owned by the
+        batch that the next call overwrites (``evaluate_actions`` has buffers of its own).  No state changes.
+        Asynchronous; a call with more rows (B*K*H) than any evaluation before allocates, synchronously."""
+        if not (torch.is_tensor(action) and action.dtype == torch.float32 and action.is_cuda and action.is_contiguous()):
+            raise TypeError("action must be a contiguous float32 CUDA tensor of shape [B, K, H, T]")
+        if action.dim() != 4 or action.shape[0] != self.B or action.shape[3] != self.T or min(action.shape[1:3]) < 1:
+            raise ValueError(f"action must have shape ({self.B}, K, H, {self.T}) with K, H >= 1, got {tuple(action.shape)}")
+        unknown = set(fields) - set(_OUTPUTS)
+        if unknown:
+            raise ValueError(f"unknown output fields {sorted(unknown)}; the step outputs are {list(_OUTPUTS)}")
+        return self._evaluate(action, tuple(fields), self._roll_bufs)
+
+    def _evaluate(self, action: torch.Tensor, fields, bufs) -> Dict[str, torch.Tensor]:
+        """``wf_evaluate_rollouts`` of a checked [B, K, H, T] action into views of ``bufs`` (name -> flat buffer)."""
+        K, H = int(action.shape[1]), int(action.shape[2])
+        res = {}
+        for name in fields + ("ambiguous",):
+            shape = (self.B, K, H) + self._shape(_OUTPUTS.get(name, "B"))[1:]
+            n = int(np.prod(shape))
+            buf = bufs.get(name)
+            if buf is None or buf.numel() < n:
+                buf = torch.zeros(n, dtype=torch.uint8 if name in ("truncated", "ambiguous") else self.real,
+                                  device=self.device)
+                bufs[name] = buf
+            res[name] = buf[:n].view(shape)
         amb = res.pop("ambiguous")
-        _lib.check(self.lib.wf_evaluate_actions(self.handle, _ptr(action), K, C.byref(_out_struct(res)), _ptr(amb),
-                                                self._stream()))
-        if K > self.act_capacity:
-            self._act_bufs, self.act_capacity = bufs, K
+        _lib.check(self.lib.wf_evaluate_rollouts(self.handle, _ptr(action), K, H, C.byref(_out_struct(res)), _ptr(amb),
+                                                 self._stream()))
         res["ambiguous"] = amb.view(torch.bool)
         return res
 

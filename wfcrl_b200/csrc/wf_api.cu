@@ -70,13 +70,15 @@ struct WfHandle_t {
     double* d_pool = nullptr;  // the layout pool in one allocation: [L][T] x, [L][T] y, [L][2] centres, [L] int32 turbine
                                // counts (WfModel.layout_*)
     std::vector<int> layout_n;  // host copy of the pool's turbine counts
-    // wf_evaluate_yaw / wf_evaluate_actions scratch, sized for the largest B*K either has evaluated so far: the evaluation fix
-    // list [eval_cap] and its 4 counters in one allocation, on a gathering FP64 handle one (v, w) scratch row per candidate
-    // [eval_cap][9T], on a strict FP32 handle one transitioned-yaw row per candidate [eval_cap][T]
+    // wf_evaluate_yaw / wf_evaluate_actions / wf_evaluate_rollouts scratch, sized in rows (B*K*H) for the largest call of
+    // any of them so far: the evaluation fix list [eval_cap] and its 4 counters in one allocation, on a gathering FP64
+    // handle one (v, w) scratch row per row [eval_cap][9T], on a strict FP32 handle one transitioned-yaw row per row
+    // [eval_cap][T], with the StepPercentage shaper one unshaped reward per row [eval_cap] (the reference of the next row)
     int eval_cap = 0;
     int* d_eval_fix = nullptr;
     double2* d_eval_vwg = nullptr;
     double* d_eval_yaw = nullptr;
+    double* d_eval_rew = nullptr;
 };
 
 template <typename T> static int dev_alloc(WfHandle_t* h, T** p, size_t n) {
@@ -244,6 +246,7 @@ int wf_destroy(WfHandle h) {
     if (h->d_eval_fix) cudaFree(h->d_eval_fix);
     if (h->d_eval_vwg) cudaFree(h->d_eval_vwg);
     if (h->d_eval_yaw) cudaFree(h->d_eval_yaw);
+    if (h->d_eval_rew) cudaFree(h->d_eval_rew);
     delete h;
     return WF_OK;
 }
@@ -630,7 +633,7 @@ int wf_update_command(WfHandle h, const double* d_yaw, const WfStepOut* out, voi
     return mark_async(h, (cudaStream_t)stream);
 }
 
-// (Re)allocate the evaluation scratch for `cap` candidates.  Synchronous on both sides: no queued evaluation may still use the
+// (Re)allocate the evaluation scratch for `cap` rows.  Synchronous on both sides: no queued evaluation may still use the
 // old scratch, and the zeroing of the new one (cudaMemset runs on the legacy default stream, which a caller's non-blocking
 // stream does not wait for) is complete before the first evaluation kernel reads the counters.
 static int eval_reserve(WfHandle h, int cap) {
@@ -638,9 +641,11 @@ static int eval_reserve(WfHandle h, int cap) {
     if (h->d_eval_fix) cudaFree(h->d_eval_fix);
     if (h->d_eval_vwg) cudaFree(h->d_eval_vwg);
     if (h->d_eval_yaw) cudaFree(h->d_eval_yaw);
+    if (h->d_eval_rew) cudaFree(h->d_eval_rew);
     h->d_eval_fix = nullptr;
     h->d_eval_vwg = nullptr;
     h->d_eval_yaw = nullptr;
+    h->d_eval_rew = nullptr;
     h->eval_cap = 0;
     const size_t fix_bytes = sizeof(int) * ((size_t)cap + 4);
     cudaError_t e = cudaMalloc(&h->d_eval_fix, fix_bytes);
@@ -652,6 +657,8 @@ static int eval_reserve(WfHandle h, int cap) {
     }
     if (e == cudaSuccess && is_strict_f32(h))
         e = cudaMalloc(&h->d_eval_yaw, sizeof(double) * (size_t)h->model.T * (size_t)cap);  // written before it is read
+    if (e == cudaSuccess && h->model.shaper == WF_SHAPER_STEP_PCT)
+        e = cudaMalloc(&h->d_eval_rew, sizeof(double) * (size_t)cap);  // written before it is read
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -662,25 +669,30 @@ static int eval_reserve(WfHandle h, int cap) {
     return WF_OK;
 }
 
-// The two evaluation entry points: yaw candidates d_yaw (interface mode, out.power only) or action candidates d_action (env
-// mode, every output of out), K per env, outputs in rows of B*K
-static int evaluate(WfHandle h, const char* fn, const double* d_yaw, const float* d_action, int32_t K, const WfStepOut* outp,
-                    uint8_t* d_ambiguous, cudaStream_t st) {
+// The evaluation entry points: yaw candidates d_yaw (interface mode, out.power only, H = 1) or action sequences d_action
+// (env mode, every output of out; wf_evaluate_actions is H = 1), K per env of H steps each, outputs in rows of B*K*H
+static int evaluate(WfHandle h, const char* fn, const double* d_yaw, const float* d_action, int32_t K, int32_t H,
+                    const WfStepOut* outp, uint8_t* d_ambiguous, cudaStream_t st) {
     if (!h) return set_err(WF_ERR_INVALID, "NULL handle");
     if (h->cfg.kernel != WF_KERNEL_FAST)
         return set_err(WF_ERR_INVALID, std::string(fn) + " needs the warp-per-env kernels (WF_KERNEL_FAST)");
     // K >= 1 is also what keeps the evaluation kernels from writing state: the FP64 ones skip their commits on a run-time
     // test of K (wf_fast64.cu: solve_env64), so this refusal must stay ahead of every launch below
     if (K < 1) return set_err(WF_ERR_INVALID, "K (candidates per env) must be >= 1");
+    if (H < 1) return set_err(WF_ERR_INVALID, "H (steps per candidate) must be >= 1");
     if ((!d_yaw && !d_action) || !outp) return set_err(WF_ERR_INVALID, "NULL argument");
     const WfStepOut out = *outp;
-    const int64_t BK = (int64_t)h->model.B * K;
-    if (BK > (int64_t)INT32_MAX)
-        return set_err(WF_ERR_INVALID, "num_envs * K = " + std::to_string(BK) + " candidates exceed the kernels' 32-bit index "
-                                       "(at most 2^31 - 1 per call)");
+    const int64_t rows = (int64_t)h->model.B * K * H;
+    if (rows > (int64_t)INT32_MAX)
+        return set_err(WF_ERR_INVALID, "num_envs * K" + std::string(H > 1 ? " * H = " : " = ") + std::to_string(rows) +
+                                       (H > 1 ? " rows" : " candidates") + " exceed the kernels' 32-bit index (at most "
+                                       "2^31 - 1 per call)");
     CUDA_TRY(cudaSetDevice(h->device));
-    if (BK > h->eval_cap) TRY(eval_reserve(h, (int)BK));
-    const WfEvalArgs ev = {K, h->d_eval_fix, h->d_eval_fix + h->eval_cap, d_ambiguous, h->d_eval_vwg, h->d_eval_yaw};
+    if (rows > h->eval_cap) TRY(eval_reserve(h, (int)rows));
+    // StepPercentage chains the reward through the steps of a rollout: the kernels keep each row's unshaped reward
+    const bool chain = H > 1 && h->model.shaper == WF_SHAPER_STEP_PCT && out.reward;
+    const WfEvalArgs ev = {K, H, h->d_eval_fix, h->d_eval_fix + h->eval_cap, d_ambiguous, h->d_eval_vwg, h->d_eval_yaw,
+                           chain ? h->d_eval_rew : nullptr};
     // the route of a step in the handle's current state: a stale vortex table is not read
     const bool use_vtab = !h->vtab_stale;
     cudaError_t e;
@@ -696,6 +708,10 @@ static int evaluate(WfHandle h, const char* fn, const double* d_yaw, const float
             h->launches += 1;
         }
     }
+    if (e == cudaSuccess && chain) {
+        e = wf_launch_eval_step_pct(h->cfg.precision == WF_PREC_F64, h->model, h->st, ev, out.reward, st);
+        h->launches += 1;
+    }
     if (e != cudaSuccess) return set_err(WF_ERR_CUDA, std::string("evaluation kernel launch: ") + cudaGetErrorString(e));
     return mark_async(h, st);
 }
@@ -703,12 +719,17 @@ static int evaluate(WfHandle h, const char* fn, const double* d_yaw, const float
 int wf_evaluate_yaw(WfHandle h, const double* d_yaw, int32_t K, void* d_power, uint8_t* d_ambiguous, void* stream) {
     WfStepOut out = {};
     out.power = d_power;
-    return evaluate(h, "wf_evaluate_yaw", d_yaw, nullptr, K, d_power ? &out : nullptr, d_ambiguous, (cudaStream_t)stream);
+    return evaluate(h, "wf_evaluate_yaw", d_yaw, nullptr, K, 1, d_power ? &out : nullptr, d_ambiguous, (cudaStream_t)stream);
 }
 
 int wf_evaluate_actions(WfHandle h, const float* d_action, int32_t K, const WfStepOut* out, uint8_t* d_ambiguous,
                         void* stream) {
-    return evaluate(h, "wf_evaluate_actions", nullptr, d_action, K, out, d_ambiguous, (cudaStream_t)stream);
+    return evaluate(h, "wf_evaluate_actions", nullptr, d_action, K, 1, out, d_ambiguous, (cudaStream_t)stream);
+}
+
+int wf_evaluate_rollouts(WfHandle h, const float* d_action, int32_t K, int32_t H, const WfStepOut* out,
+                         uint8_t* d_ambiguous, void* stream) {
+    return evaluate(h, "wf_evaluate_rollouts", nullptr, d_action, K, H, out, d_ambiguous, (cudaStream_t)stream);
 }
 
 // Device alias of a host pointer when it is page-locked memory the GPU can address (cudaHostAlloc / cudaHostRegister

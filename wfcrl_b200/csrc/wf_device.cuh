@@ -141,19 +141,79 @@ typedef WfFastConstT<double> WfFastConst64;
 
 enum WfMode { WF_MODE_INTERFACE = 0, WF_MODE_ENV = 1, WF_MODE_WARMUP = 2 };
 
-// Candidate evaluation (wf_evaluate_yaw, wf_evaluate_actions): the EVAL instantiations of the fast kernels solve K candidates
-// per env, CTA c = candidate c = env c / K, candidate c % K (the K candidates of an env are adjacent, so that its geometry and
-// table rows are shared in L2).  They read the candidate's yaw (or action) from the caller's [B*K][T] array, write its output
-// rows c and write no WfState array.  The scratch below belongs to the handle's evaluation path alone.
+// Candidate evaluation (wf_evaluate_yaw, wf_evaluate_actions, wf_evaluate_rollouts): the EVAL instantiations of the fast
+// kernels solve K candidates per env, each an open-loop sequence of H steps (H = 1 but for rollouts).  CTA c = row c =
+// (b*K + k)*H + h: env b = c / (K*H), step h = c % H (the K*H rows of an env are adjacent, so that its geometry and table rows
+// are shared in L2).  They read the row's yaw (or actions 0..h of its sequence) from the caller's [B*K*H][T] array, write its
+// output rows c and write no WfState array.  The scratch below belongs to the handle's evaluation path alone.
 struct WfEvalArgs {
     int K;             // candidates per env
-    int* fix_list;     // [B*K] strict FP32: ids of the candidates the FP32 launch flagged (never the step path's fix_list)
+    int H;             // steps per candidate (in the padding after K: no field below moved)
+    int* fix_list;     // [B*K*H] strict FP32: ids of the rows the FP32 launch flagged (never the step path's fix_list)
     int* fix_count;    // [4] as WfState.fix_count, for fix_list
-    uint8_t* amb;      // [B*K] or NULL: 1 = the candidate was re-solved by the FP64 kernel
-    double2* vwg;      // [B*K][9T] FP64 gather form: the (v, w) scratch, one row per candidate (WfState.vwg is per env)
-    double* yaw;       // [B*K][T] strict FP32, actions: the transitioned yaw of a flagged candidate, which its re-solve
+    uint8_t* amb;      // [B*K*H] or NULL: 1 = the row was re-solved by the FP64 kernel
+    double2* vwg;      // [B*K*H][9T] FP64 gather form: the (v, w) scratch, one row per row (WfState.vwg is per env)
+    double* yaw;       // [B*K*H][T] strict FP32, actions: the transitioned yaw of a flagged row, which its re-solve
                        //     reads where the step's re-solve reads the committed WfState.yaw
+    double* rew;       // [B*K*H] or NULL: StepPercentage rollouts (H > 1): every row's unshaped reward, the reference of
+                       //     the next row (wf_launch_eval_step_pct shapes rows h >= 1; row 0 is shaped in the kernels)
 };
+
+// The applied yaw increment of one turbine's action a in the env step (mdp.py:291-319), in the step's float32 operations:
+// 0 when the actuation-rate constraint on acc_c (the accumulator the constraint sees) over nm moves fires, else the clip
+// (continuous control) or the map of {0, 1, 2} (discrete).  Shared by the step and evaluation kernels of both precisions.
+__device__ __forceinline__ float wf_applied_action(const WfModel& m, float a, const float acc_c, const int nm) {
+    const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
+    if (frac >= 0.1f) a = 0.0f;
+    if (m.continuous) a = fminf(fmaxf(a, -m.yaw_step_f), m.yaw_step_f);
+    else a = __fmul_rn(__fsub_rn(a, 1.0f), m.yaw_step_f);
+    return a;
+}
+// The new yaw of a step: the clipped sum of the clipped yaw y and the applied increment a
+__device__ __forceinline__ float wf_new_yaw(const WfModel& m, const float y, const float a) {
+    const float y0 = fminf(fmaxf(y, m.yaw_lo_f), m.yaw_hi_f);
+    return fminf(fmaxf(__fadd_rn(y0, a), m.yaw_lo_f), m.yaw_hi_f);
+}
+
+// Rollouts (wf_evaluate_rollouts): steps 0..h-1 of a row's action sequence (step j's action at row arow + j*T) replayed
+// for one turbine from its committed state (acc, acc_c, yaw y), in registers.  Returns the yaw step h starts from and
+// leaves acc, acc_c as step h sees them (each step commits acc_prev = acc, acc += |a|).  stale: multi-agent handle, not
+// the last turbine (the constraint sees acc_prev).  Rolled, and run only for h > 0: the one-step path keeps the step's code.
+__device__ __forceinline__ float wf_replay(const WfModel& m, const float* __restrict__ action, const size_t arow, const int T,
+                                           const int tt, const bool stale, const int nm, const int h, float& acc,
+                                           float& acc_c, float y) {
+#pragma unroll 1
+    for (int j = 0; j < h; ++j) {
+        const float a = wf_applied_action(m, action[arow + (size_t)j * T + tt], acc_c, nm + j);
+        y = wf_new_yaw(m, y, a);
+        const float acc_next = __fadd_rn(acc, fabsf(a));
+        acc_c = stale ? acc : acc_next;
+        acc = acc_next;
+    }
+    return y;
+}
+
+// A rollout row past its candidate's truncating step (wf_evaluate_rollouts): every output of row c and its flag read 0.
+// One warp; OutT = type of the caller's "real" buffers.
+template <typename OutT>
+__device__ __forceinline__ void wf_zero_eval_row(const WfStepOut& out, uint8_t* amb, const size_t c, const int T,
+                                                 const int lane) {
+    auto zero = [&](void* p, const int w) {
+        if (p)
+            for (int q = lane; q < T * w; q += 32) ((OutT*)p)[c * T * w + q] = (OutT)0;
+    };
+    zero(out.yaw, 1);
+    zero(out.wind_speed, 1);
+    zero(out.wind_direction, 1);
+    zero(out.power, 1);
+    zero(out.load, 4);
+    if (lane == 0) {
+        if (out.reward) ((OutT*)out.reward)[c] = (OutT)0;
+        if (out.freewind) { ((OutT*)out.freewind)[2 * c] = (OutT)0; ((OutT*)out.freewind)[2 * c + 1] = (OutT)0; }
+        if (out.truncated) out.truncated[c] = 0;
+        if (amb) amb[c] = 0;
+    }
+}
 
 // launchers implemented in wf_kernels.cu
 cudaError_t wf_launch_geometry(const WfModel& m, const WfState& s, const uint8_t* d_mask, const double* d_cs_override,
@@ -187,10 +247,11 @@ cudaError_t wf_launch_step_fast64(int mode, bool use_vtab, const WfModel& m, con
                                   const WfStepOut& out, int env_begin, int env_count, cudaStream_t stream);
 cudaError_t wf_step_fast64_attributes(const WfModel& m, const WfState& s, cudaFuncAttributes* attr, int* ctas_per_sm, int* threads,
                                       int* smem);
-// candidate evaluation: one launch of B*K CTAs with out's buffers of B*K rows; on a strict FP32 handle wf_launch_eval_fixup64
-// re-solves the flagged candidates (ev.fix_list) in FP64, in the evaluation's mode.  d_action == NULL: yaw candidates d_yaw
-// [B*K][T] in interface mode, out.power only (wf_evaluate_yaw); else action candidates d_action [B*K][T] in env mode, every
-// output (wf_evaluate_actions)
+// candidate evaluation: one launch of B*K*H CTAs with out's buffers of B*K*H rows; on a strict FP32 handle
+// wf_launch_eval_fixup64 re-solves the flagged rows (ev.fix_list) in FP64, in the evaluation's mode.  d_action == NULL: yaw
+// candidates d_yaw [B*K][T] (H = 1) in interface mode, out.power only (wf_evaluate_yaw); else action sequences d_action
+// [B*K*H][T] in env mode, every output (wf_evaluate_actions at H = 1, wf_evaluate_rollouts); then, for StepPercentage
+// rollouts, wf_launch_eval_step_pct chains the reward of rows h >= 1 through ev.rew
 cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
                                 const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream);
 cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
@@ -198,4 +259,6 @@ cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastC
                                   cudaStream_t stream);
 cudaError_t wf_launch_eval_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                    const WfEvalArgs& ev, const double* d_yaw, const WfStepOut& out, cudaStream_t stream);
+cudaError_t wf_launch_eval_step_pct(bool f64, const WfModel& m, const WfState& s, const WfEvalArgs& ev, void* d_reward,
+                                    cudaStream_t stream);
 bool wf_fast64_gathers(const WfModel& m, const WfState& s);  // an FP64 handle's step kernel runs the gather form

@@ -126,25 +126,34 @@ struct wf_false_tag { static constexpr bool value = false; };
 // generic instantiation: 12 is a lower bound for the register allocator; 16 envs per SM are reached
 // EVAL (wf_evaluate_yaw): CTA c solves candidate c of env c / K in interface mode with the yaw row c of `yaw_cmd`, writes power
 // row c of `out.power` and nothing else, and hands a flagged candidate to the evaluation fix list (wf_device.cuh: WfEvalArgs)
-// EVAL + ACT (wf_evaluate_actions): CTA c runs env b = c / K's step with action row c in the run-time mode (env) of the step --
-// transition, solve, epilogue and reward -- against b's state, which it reads and never writes; every output goes to row c.
-// A flagged candidate leaves its transitioned yaw in ev.yaw row c for the re-solve.
+// EVAL + ACT (wf_evaluate_actions): CTA c runs env b = c / K's step with action row c in the run-time mode (env) of the
+// step -- transition, solve, epilogue and reward -- against b's state, which it reads and never writes; every output goes
+// to row c.  A flagged candidate leaves its transitioned yaw in ev.yaw row c for the re-solve.
+// EVAL + ACT + ROLL (wf_evaluate_rollouts, H > 1): CTA c = row (b*K + k)*H + h runs step h of candidate k's action sequence
+// on env b: the transitions of steps 0..h-1 (wf_replay, action rows c - h .. c - 1), then step h as above.  A separate
+// instantiation, so that at H = 1 (h = 0 a compile-time constant) the action kernel is the one it was before rollouts.
 // Unlike the FP64 kernels, this kernel keeps yaw evaluation an instantiation of its own (EVAL without ACT), with the mode a
 // compile-time constant: with the env-mode epilogue (wind direction, loads, reward) compiled in, FP32 yaw evaluation ran
 // 1-3 % slower (DESIGN.md section 5b)
-template <bool BAKED, bool EVAL = false, bool ACT = false>
+template <bool BAKED, bool EVAL = false, bool ACT = false, bool ROLL = false>
 __global__ void __launch_bounds__(32, BAKED ? 16 : 12)
 wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const __grid_constant__ WfFastConst fc,
                     const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
                     const double* __restrict__ yaw_cmd, const WfStepOut out, const WfEvalArgs ev) {
-    int b;
-    if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
+    int b, h = 0;  // h: step of the row in its candidate's sequence (0 but for rollouts)
+    if constexpr (ROLL) { b = blockIdx.x / (ev.K * ev.H); h = blockIdx.x % ev.H; }
+    else if constexpr (EVAL) b = blockIdx.x / ev.K;
+    else b = blockIdx.x + env_begin;
     const int mode = (EVAL && !ACT) ? (int)WF_MODE_INTERFACE : mode_;
     if (mask && !mask[b]) return;
     const int T = m.T;
     const int lane = threadIdx.x;
     const size_t row = (size_t)b * T;
     const size_t orow = EVAL ? (size_t)blockIdx.x * T : row;  // row of the yaw command / action and of the outputs
+    if (ROLL && h > 0) {  // a row after its candidate's truncating step (num_iter + h' + 1 == max_iter, h' < h) is not solved
+        const int h_trunc = m.max_iter - s.num_iter[b] - 1;
+        if (h_trunc >= 0 && h > h_trunc) { wf_zero_eval_row<float>(out, ev.amb, blockIdx.x, T, lane); return; }
+    }
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const SmemView sm = carve(smem_raw, T);  // sized by T: every env of the handle reserves the same shared memory
     // the env's turbine count: the one loop bound below.  Columns n..T-1 of its rows are padding (wf_device.cuh)
@@ -157,14 +166,14 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
         float ynew;
         if (mode == WF_MODE_ENV) {
             float a = action[orow + tt];
-            const float acc = s.acc[row + tt];
-            const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
-            const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
-            if (frac >= 0.1f) a = 0.0f;
-            if (m.continuous) a = fminf(fmaxf(a, -m.yaw_step_f), m.yaw_step_f);
-            else a = __fmul_rn(__fsub_rn(a, 1.0f), m.yaw_step_f);
-            const float y0 = fminf(fmaxf((float)s.yaw[row + tt], m.yaw_lo_f), m.yaw_hi_f);
-            ynew = fminf(fmaxf(__fadd_rn(y0, a), m.yaw_lo_f), m.yaw_hi_f);
+            float acc = s.acc[row + tt];
+            float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
+            float y_h = 0.f;  // a rollout row: the yaw after steps 0..h-1 of its sequence (action rows c - h .. c - 1)
+            if (ROLL && h > 0)
+                y_h = wf_replay(m, action, orow - (size_t)h * T, T, tt, m.multi_agent && tt != n - 1, nm, h, acc, acc_c,
+                                (float)s.yaw[row + tt]);
+            a = wf_applied_action(m, a, acc_c, nm + h);
+            ynew = wf_new_yaw(m, (ROLL && h > 0) ? y_h : (float)s.yaw[row + tt], a);
             if (!ACT) {
                 s.acc_prev[row + tt] = acc;
                 s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
@@ -610,7 +619,7 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
     const int ob = ACT ? (int)blockIdx.x : b;
     int it = 0;
     if (lane == 0) {
-        it = s.num_iter[b] + 1;
+        it = s.num_iter[b] + 1 + h;
         if (!ACT) s.num_iter[b] = it;
         if (out.truncated) out.truncated[ob] = (uint8_t)(it == m.max_iter);
         float fw0 = ws, fw1 = wd;
@@ -618,16 +627,21 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
         if (out.freewind) ((float2*)out.freewind)[ob] = make_float2(fw0, fw1);
         if (mode == WF_MODE_ENV) {
             if (!ACT) s.num_moves[b] = nm;
-            const float wn = (float)s.ws_norm[b];
+            const float wn = h > 0 ? ws : (float)s.ws_norm[b];  // a step leaves ws_norm = ws for the next one
             const float invT = 1.f / (float)n;  // the mean over the env's own turbines
             float reward = rsum_p * 1e3f / (wn * wn * wn) * invT - fc.load_coef * rsum_l * (0.25f * invT);
             if (m.shaper == 1) {
                 reward = (reward - fc.shaper_reference) / fc.shaper_reference;
             } else if (m.shaper == 2) {
-                const double ref = s.shaper_ref[b];
-                const float shaped = (ref == 0.0) ? 0.f : (float)(((double)reward - ref) / ref);
-                if (!ACT) s.shaper_ref[b] = (double)reward;
-                reward = shaped;
+                // a rollout keeps every row's unshaped reward, the reference of its next row; rows h >= 1 are shaped by
+                // wf_launch_eval_step_pct (wf_fast64.cu: one pass for both precisions), which reads that reference
+                if (ROLL && ev.rew) ev.rew[ob] = (double)reward;
+                if (h == 0) {
+                    const double ref = s.shaper_ref[b];
+                    const float shaped = (ref == 0.0) ? 0.f : (float)(((double)reward - ref) / ref);
+                    if (!ACT) s.shaper_ref[b] = (double)reward;
+                    reward = shaped;
+                }
             }
             if (!ACT && !isfinite(reward)) s.nonfinite[b] += 1;
             if (out.reward) ((float*)out.reward)[ob] = reward;
@@ -661,7 +675,8 @@ wf_step_fast_kernel(const int mode_, const int env_begin, const WfModel m, const
 
 cudaError_t wf_configure_fast_kernels() {
     for (auto k : {wf_step_fast_kernel<true>, wf_step_fast_kernel<false>, wf_step_fast_kernel<true, true>,
-                   wf_step_fast_kernel<false, true>, wf_step_fast_kernel<true, true, true>, wf_step_fast_kernel<false, true, true>}) {
+                   wf_step_fast_kernel<false, true>, wf_step_fast_kernel<true, true, true>, wf_step_fast_kernel<false, true, true>,
+                   wf_step_fast_kernel<true, true, true, true>, wf_step_fast_kernel<false, true, true, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -679,16 +694,19 @@ static cudaError_t launch_fast_t(int mode, const WfModel& m, const WfFastConst& 
     return cudaGetLastError();
 }
 
-template <bool BAKED, bool ACT>
+template <bool BAKED, bool ACT, bool ROLL = false>
 static cudaError_t launch_eval_t(const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
                                  const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream) {
-    wf_step_fast_kernel<BAKED, true, ACT><<<(unsigned)m.B * (unsigned)ev.K, 32, fast_smem_bytes(m.T), stream>>>(
+    wf_step_fast_kernel<BAKED, true, ACT, ROLL><<<(unsigned)m.B * (unsigned)ev.K * (unsigned)ev.H, 32, fast_smem_bytes(m.T), stream>>>(
         ACT ? WF_MODE_ENV : WF_MODE_INTERFACE, 0, m, fc, s, nullptr, d_action, d_yaw, out, ev);
     return cudaGetLastError();
 }
 
 cudaError_t wf_launch_eval_fast(bool baked, const WfModel& m, const WfFastConst& fc, const WfState& s, const WfEvalArgs& ev,
                                 const double* d_yaw, const float* d_action, const WfStepOut& out, cudaStream_t stream) {
+    if (d_action && ev.H > 1)
+        return baked ? launch_eval_t<true, true, true>(m, fc, s, ev, nullptr, d_action, out, stream)
+                     : launch_eval_t<false, true, true>(m, fc, s, ev, nullptr, d_action, out, stream);
     if (d_action)
         return baked ? launch_eval_t<true, true>(m, fc, s, ev, nullptr, d_action, out, stream)
                      : launch_eval_t<false, true>(m, fc, s, ev, nullptr, d_action, out, stream);

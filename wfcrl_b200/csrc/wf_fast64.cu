@@ -193,7 +193,10 @@ __device__ __forceinline__ void load_row12(const double* __restrict__ p, double*
 // `cand`, its flag to ev.amb[cand] (FIX: 1, else 0), and the state is read and never written.  Env mode (wf_evaluate_actions):
 // the action row `cand` (FIX: the transitioned yaw row `cand` of ev.yaw).  Interface mode (wf_evaluate_yaw): the yaw row
 // `cand` of `yaw_cmd`.
-template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false>
+// ROLL = rollout row (wf_evaluate_rollouts, H > 1): step h = cand % H of its candidate's sequence (wf_replay, the step-h
+// epilogue rules of wf_fast.cu).  Without it h = 0 is a compile-time constant, and the one-step evaluations compile to the
+// code they had before rollouts existed.
+template <int W, typename OutT, bool FIX, bool GATHER = false, bool EVAL = false, bool ROLL = false>
 __device__ __forceinline__ void solve_env64(const int b, const int mode, const bool use_vtab, const WfModel& m,
                                             const WfFastConst64& fc, const WfState& s, const float* __restrict__ action,
                                             const double* __restrict__ yaw_cmd, const WfStepOut& out,
@@ -210,6 +213,8 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     // rests on the compiler's choices: the bit-equality tests of both evaluations (tests/test_evaluate_yaw_gpu.py,
     // tests/test_evaluate_actions_gpu.py) catch a compiler that makes others
     const bool commit = !EVAL || ev.K < 1;
+    // EVAL: the row's step h in its candidate's action sequence (wf_evaluate_rollouts; 0 for every other evaluation)
+    const int h = ROLL ? cand % ev.H : 0;
     // the env's turbine count, the bound of every loop below; columns n..T-1 of its rows are padding (wf_device.cuh).
     // Shared memory and the table's row strides stay those of T.
     const int n = s.turbine_count[b];
@@ -232,14 +237,14 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         double ynew;
         if (!FIX && mode == WF_MODE_ENV) {
             float a = action[orow + tt];
-            const float acc = s.acc[row + tt];
-            const float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
-            const float frac = __fdiv_rn(__fdiv_rn(__fdiv_rn(acc_c, m.rate_f), (float)nm), m.dt_f);
-            if (frac >= 0.1f) a = 0.0f;
-            if (m.continuous) a = fminf(fmaxf(a, -m.yaw_step_f), m.yaw_step_f);
-            else a = __fmul_rn(__fsub_rn(a, 1.0f), m.yaw_step_f);
-            const float y0 = fminf(fmaxf((float)s.yaw[row + tt], m.yaw_lo_f), m.yaw_hi_f);
-            const float y1 = fminf(fmaxf(__fadd_rn(y0, a), m.yaw_lo_f), m.yaw_hi_f);
+            float acc = s.acc[row + tt];
+            float acc_c = (m.multi_agent && tt != n - 1) ? s.acc_prev[row + tt] : acc;
+            float y_h = 0.f;  // a rollout row: the yaw after steps 0..h-1 of its sequence (action rows cand - h .. cand - 1)
+            if (ROLL && h > 0)
+                y_h = wf_replay(m, action, orow - (size_t)h * T, T, tt, m.multi_agent && tt != n - 1, nm, h, acc, acc_c,
+                                (float)s.yaw[row + tt]);
+            a = wf_applied_action(m, a, acc_c, nm + h);
+            const float y1 = wf_new_yaw(m, (ROLL && h > 0) ? y_h : (float)s.yaw[row + tt], a);
             if (commit) {
                 s.acc_prev[row + tt] = acc;
                 s.acc[row + tt] = __fadd_rn(acc, fabsf(a));
@@ -856,7 +861,7 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
     const int ob = EVAL ? cand : b;
     int it = 0;
     if (lane == 0) {
-        it = s.num_iter[b] + 1;
+        it = s.num_iter[b] + 1 + h;
         if (commit) s.num_iter[b] = it;
         if (out.truncated) out.truncated[ob] = (uint8_t)(it == m.max_iter);
         double fw0 = ws, fw1 = wd;
@@ -865,15 +870,19 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
         if (FIX && rec) { rec[0] = __int_as_float(b); rec[1] = 0.f; rec[2] = (float)fw0; rec[3] = (float)fw1; rec[4] = (it == m.max_iter) ? 1.f : 0.f; }
         if (mode == WF_MODE_ENV) {
             if (commit) s.num_moves[b] = nm;
-            const double wn = s.ws_norm[b];
+            const double wn = h > 0 ? ws : s.ws_norm[b];  // a step leaves ws_norm = ws for the next one
             double reward = rsum_p * 1e3 / (wn * wn * wn) / n - m.load_coef * (rsum_l / (4.0 * n));  // mean over the env's turbines
             if (m.shaper == 1) {
                 reward = (reward - m.shaper_reference) / m.shaper_reference;
             } else if (m.shaper == 2) {
-                const double ref = s.shaper_ref[b];
-                const double shaped = (ref == 0.0) ? 0.0 : (reward - ref) / ref;
-                if (commit) s.shaper_ref[b] = reward;
-                reward = shaped;
+                // a rollout keeps every row's unshaped reward, the reference of its next row (see wf_fast.cu)
+                if (ROLL && ev.rew) ev.rew[ob] = reward;
+                if (h == 0) {
+                    const double ref = s.shaper_ref[b];
+                    const double shaped = (ref == 0.0) ? 0.0 : (reward - ref) / ref;
+                    if (commit) s.shaper_ref[b] = reward;
+                    reward = shaped;
+                }
             }
             if (commit && !isfinite(reward)) s.nonfinite[b] += 1;
             if (out.reward) ((OutT*)out.reward)[ob] = (OutT)reward;
@@ -897,16 +906,30 @@ __device__ __forceinline__ void solve_env64(const int b, const int mode, const b
 // sub-partition with two others (12 per SM), one of 128 registers with three (16 per SM; 12-48 bytes of spills).  The kernels
 // are latency-bound, throughput grows with the resident envs (measured on Turb32_Row5: 6 per SM 4.9 M env-steps/s, 9: 6.2 M,
 // 12: 7.6 M, 16: 8.2 M); at 80 turbines shared memory holds 14 envs of the gather kernel per SM (9 of the scatter kernel).
-// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw in interface mode, wf_evaluate_actions in env mode)
-template <bool GATHER, bool EVAL = false>
+// EVAL: CTA c evaluates candidate c of env c / K (wf_evaluate_yaw in interface mode, wf_evaluate_actions in env mode);
+// EVAL + ROLL: row c of env c / (K H) (wf_evaluate_rollouts with H > 1)
+template <bool GATHER, bool EVAL = false, bool ROLL = false>
 __global__ void __launch_bounds__(32, 16)
 wf_step_fast64_kernel(const int mode, const int env_begin, const bool use_vtab, const WfModel m, const __grid_constant__ WfFastConst64 fc,
                       const WfState s, const uint8_t* __restrict__ mask, const float* __restrict__ action,
                       const double* __restrict__ yaw_cmd, const WfStepOut out, const WfEvalArgs ev) {
     int b;
-    if constexpr (EVAL) b = blockIdx.x / ev.K; else b = blockIdx.x + env_begin;
+    if constexpr (ROLL) {
+        b = blockIdx.x / (ev.K * ev.H);
+        // a row after its candidate's truncating step is not solved (step 0 never is one).  Here rather than in
+        // solve_env64: there the test changed the compiler's floating-point contractions of the solve (DESIGN.md 5b)
+        const int h = blockIdx.x % ev.H;
+        if (h > 0) {
+            const int h_trunc = m.max_iter - s.num_iter[b] - 1;
+            if (h_trunc >= 0 && h > h_trunc) { wf_zero_eval_row<double>(out, ev.amb, blockIdx.x, m.T, threadIdx.x); return; }
+        }
+    } else if constexpr (EVAL) {
+        b = blockIdx.x / ev.K;
+    } else {
+        b = blockIdx.x + env_begin;
+    }
     if (mask && !mask[b]) return;
-    solve_env64<1, double, false, GATHER, EVAL>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
+    solve_env64<1, double, false, GATHER, EVAL, ROLL>(b, mode, use_vtab, m, fc, s, action, yaw_cmd, out, nullptr, ev, blockIdx.x);
 }
 
 // Re-solve, in FP64, of the envs an FP32 launch flagged (their ids sit in s.fix_list[0, n), n in s.fix_count[0]); launched
@@ -933,9 +956,10 @@ wf_fixup64_kernel(const int mode, const bool use_vtab, const WfModel m, const __
     }
 }
 
-// Evaluation instantiation of the re-solve: the candidates an evaluation launch flagged (ev.fix_list / ev.fix_count,
-// candidate c = env c / K), from the transitioned yaw rows in ev.yaw (env mode, wf_evaluate_actions) or the yaw rows of
-// `yaw_cmd` (interface mode, wf_evaluate_yaw); they write every output row of the candidate and its flag and commit nothing.
+// Evaluation instantiation of the re-solve: the rows an evaluation launch flagged (ev.fix_list / ev.fix_count, row c = env
+// c / (K H), step c % H), from the transitioned yaw rows in ev.yaw (env mode, wf_evaluate_actions / wf_evaluate_rollouts)
+// or the yaw rows of `yaw_cmd` (interface mode, wf_evaluate_yaw); they write every output row and the flag of the row and
+// commit nothing.
 // A kernel of its own rather than a flag of wf_fixup64_kernel, whose parameter list (and so code) stays as it was.
 template <int W>
 __global__ void __launch_bounds__(32 * W, W == 1 ? 8 : 1)
@@ -944,7 +968,7 @@ wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, con
     const int n = *(volatile int*)&ev.fix_count[0];
     for (int k = blockIdx.x; k < n; k += gridDim.x) {
         const int c = ev.fix_list[k];
-        solve_env64<W, float, true, false, true>(c / ev.K, mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
+        solve_env64<W, float, true, false, true, true>(c / (ev.K * ev.H), mode, use_vtab, m, fc, s, nullptr, yaw_cmd, out, nullptr, ev, c);
         __syncthreads();
     }
     if (threadIdx.x == 0) {  // the last CTA to leave re-arms the evaluation counters
@@ -962,7 +986,8 @@ wf_fixup64_eval_kernel(const int mode, const bool use_vtab, const WfModel m, con
 // Dynamic shared memory up to 100 KB for every FP64 kernel; the step kernels also prefer the largest shared-memory carveout.
 cudaError_t wf_configure_fast64_kernels() {
     for (auto k : {wf_step_fast64_kernel<false>, wf_step_fast64_kernel<true>, wf_step_fast64_kernel<false, true>,
-                   wf_step_fast64_kernel<true, true>}) {
+                   wf_step_fast64_kernel<true, true>, wf_step_fast64_kernel<false, true, true>,
+                   wf_step_fast64_kernel<true, true, true>}) {
         cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
         if (e == cudaSuccess)
             e = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -1017,10 +1042,37 @@ cudaError_t wf_launch_fixup64(int mode, bool use_vtab, const WfModel& m, const W
     return launch_fixup_sized<false>(mode, use_vtab, m, fc, s, out, env_count, d_rec, rec_cap, nullptr, WfEvalArgs{}, stream);
 }
 
-// W is chosen from the B*K CTAs of the evaluation launch by the step's rule
+// W is chosen from the B*K*H CTAs of the evaluation launch by the step's rule
 cudaError_t wf_launch_eval_fixup64(int mode, bool use_vtab, const WfModel& m, const WfFastConst64& fc, const WfState& s,
                                    const WfEvalArgs& ev, const double* d_yaw, const WfStepOut& out, cudaStream_t stream) {
-    return launch_fixup_sized<true>(mode, use_vtab, m, fc, s, out, m.B * ev.K, nullptr, 0, d_yaw, ev, stream);
+    return launch_fixup_sized<true>(mode, use_vtab, m, fc, s, out, m.B * ev.K * ev.H, nullptr, 0, d_yaw, ev, stream);
+}
+
+// StepPercentage through a rollout: a step shapes its reward with the previous step's unshaped one as the reference.  Row
+// h = 0 was shaped in the evaluation kernels with the committed shaper_ref; rows h >= 1 are shaped here, one thread per
+// candidate walking its rows in order up to its truncating step, from the unshaped rewards ev.rew the kernels left (the
+// float reward widened to double, or a re-solved row's double reward, as the step commits to shaper_ref).  Same expression
+// as the step kernels.
+template <typename OutT>
+__global__ void __launch_bounds__(256)
+wf_eval_step_pct_kernel(const WfModel m, const WfState s, const WfEvalArgs ev, OutT* __restrict__ reward) {
+    const int bk = blockIdx.x * blockDim.x + threadIdx.x;
+    if (bk >= m.B * ev.K) return;
+    const int h_trunc = m.max_iter - s.num_iter[bk / ev.K] - 1;
+    const int h_end = (h_trunc >= 0 && h_trunc < ev.H - 1) ? h_trunc : ev.H - 1;
+    const size_t c0 = (size_t)bk * ev.H;
+    for (int h = 1; h <= h_end; ++h) {
+        const double ref = ev.rew[c0 + h - 1];
+        reward[c0 + h] = (ref == 0.0) ? (OutT)0 : (OutT)((ev.rew[c0 + h] - ref) / ref);
+    }
+}
+
+cudaError_t wf_launch_eval_step_pct(bool f64, const WfModel& m, const WfState& s, const WfEvalArgs& ev, void* d_reward,
+                                    cudaStream_t stream) {
+    const unsigned grid = (unsigned)(((long long)m.B * ev.K + 255) / 256);
+    if (f64) wf_eval_step_pct_kernel<double><<<grid, 256, 0, stream>>>(m, s, ev, (double*)d_reward);
+    else wf_eval_step_pct_kernel<float><<<grid, 256, 0, stream>>>(m, s, ev, (float*)d_reward);
+    return cudaGetLastError();
 }
 
 bool wf_fast64_gathers(const WfModel& m, const WfState& s) { return m.vtab_tmajor && s.vtab && s.vwg && s.tab_glo; }
@@ -1046,10 +1098,15 @@ cudaError_t wf_launch_eval_fast64(bool use_vtab, const WfModel& m, const WfFastC
     // the same form as the step kernel of this handle in its current state (a stale table: the scatter form, pairs direct)
     const bool gather = wf_fast64_gathers(m, s) && use_vtab;
     const size_t smem = fast64_smem_bytes(m.T, gather);
-    const unsigned grid = (unsigned)m.B * (unsigned)ev.K;
+    const unsigned grid = (unsigned)m.B * (unsigned)ev.K * (unsigned)ev.H;
     const int mode = d_action ? WF_MODE_ENV : WF_MODE_INTERFACE;
-    if (gather)
+    if (gather && ev.H > 1)
+        wf_step_fast64_kernel<true, true, true><<<grid, 32, smem, stream>>>(mode, 0, true, m, fc, s, nullptr, d_action, d_yaw, out, ev);
+    else if (gather)
         wf_step_fast64_kernel<true, true><<<grid, 32, smem, stream>>>(mode, 0, true, m, fc, s, nullptr, d_action, d_yaw, out, ev);
+    else if (ev.H > 1)
+        wf_step_fast64_kernel<false, true, true><<<grid, 32, smem, stream>>>(mode, 0, use_vtab, m, fc, s, nullptr, d_action, d_yaw, out,
+                                                                            ev);
     else
         wf_step_fast64_kernel<false, true><<<grid, 32, smem, stream>>>(mode, 0, use_vtab, m, fc, s, nullptr, d_action, d_yaw, out, ev);
     return cudaGetLastError();

@@ -333,30 +333,63 @@ class VecWindFarmEnv:
 
     def evaluate_actions(self, action):
         """One-step lookahead: what ``step`` would return for each of K candidate actions per env, from where each env is
-        now, without stepping (``FlorisBatch.evaluate_actions``).  ``action``: [B, K, T] (or ``{"yaw": ...}``).  Returns
+        now, without stepping (``evaluate_rollouts`` with H = 1).  ``action``: [B, K, T] (or ``{"yaw": ...}``).  Returns
         ``(obs, reward, terminated, truncated, info)`` with a K axis after the batch axis, exactly as ``step`` would return
         them for each candidate, without the auto-reset handling: a candidate that truncates reports ``truncated`` and its
         final observation, and nothing is reset.  The env's state, its cohort countdowns included, does not change.
         Views of buffers the next call overwrites unless ``copy_outputs``.  Not available in wind-time-series mode, where a
         step moves the wind before it solves."""
-        assert not self._needs_reset, "Call reset before `evaluate_actions`"
+        self._check_evaluable()
+        obs, reward, terminated, truncated, info = self._evaluation(self.backend.evaluate_actions(self._action_tensor(action)))
+        return obs, reward, terminated, truncated, info
+
+    def evaluate_rollouts(self, actions, observations: bool = True):
+        """Open-loop H-step lookahead: what H successive ``step`` calls would return for each of K candidate action
+        sequences per env, from where each env is now, without stepping (``FlorisBatch.evaluate_rollouts``).  ``actions``:
+        [B, K, H, T] (or ``{"yaw": ...}``), row [b, k, h] the action at step h.  Returns ``(obs, reward, terminated,
+        truncated, info)`` with K and H axes after the batch axis.  A candidate's rollout ends with its first truncating
+        step (nothing is reset): ``info["valid"]`` (bool [B, K, H]) marks the rows up to and including it, and the rows
+        after it read 0.  ``observations=False`` computes reward, truncated and valid only; obs, ``info["power"]`` and
+        ``info["load"]`` are then None.  The env's state, its cohort countdowns included, does not change.  Views of
+        buffers the next call overwrites unless ``copy_outputs``.  Not available in wind-time-series mode."""
+        self._check_evaluable()
+        fields = ("yaw", "wind_speed", "wind_direction", "power", "load", "reward", "freewind", "truncated") \
+            if observations else ("reward", "truncated")
+        out = self.backend.evaluate_rollouts(self._action_tensor(actions), fields)
+        obs, reward, terminated, truncated, info = self._evaluation(out, observations)
+        steps = out["truncated"].to(torch.int32)
+        info["valid"] = (steps.cumsum(2) - steps) == 0  # no truncation before the row
+        return obs, reward, terminated, truncated, info
+
+    def _check_evaluable(self):
+        assert not self._needs_reset, "Call reset before evaluating actions"
         if self._series is not None:
-            raise ValueError("evaluate_actions is not available in wind-time-series mode: a step there moves the wind (and "
+            raise ValueError("action evaluation is not available in wind-time-series mode: a step there moves the wind (and "
                              "the geometry) before it solves, which an evaluation cannot do without changing the state")
+
+    def _evaluation(self, out, observations: bool = True):
+        """The step tuple of the backend evaluation results ``out`` (leading axes [B, K] or [B, K, H])."""
+        c = (lambda t: t.clone()) if self.copy_outputs else (lambda t: t)
+        reward, truncated = c(out["reward"]), c(out["truncated"].view(torch.bool))
+        terminated = torch.zeros(reward.shape, dtype=torch.bool, device=self.device)
+        info = {"power": None, "load": None}
+        if not observations:
+            return None, reward, terminated, truncated, info
+        obs = OrderedDict([("yaw", c(out["yaw"])), ("freewind_measurements", c(out["freewind"])),
+                           ("wind_speed", c(out["wind_speed"])), ("wind_direction", c(out["wind_direction"]))])
+        if self.pad_turbines:
+            lead = (self.num_envs,) + (1,) * (reward.dim() - 1)
+            obs["turbine_mask"] = self._turbine_mask.view(lead + (self.num_turbines,)).expand(*reward.shape, -1)
+        info["power"], info["load"] = c(out["power"]), c(out["load"])
+        return obs, reward, terminated, truncated, info
+
+    def _action_tensor(self, action) -> torch.Tensor:
+        """The float32 device tensor of ``action`` (a tensor, an array or ``{"yaw": ...}``)."""
         if isinstance(action, dict):
             action = action["yaw"]
         if not torch.is_tensor(action):
             action = torch.as_tensor(np.asarray(action, dtype=np.float32), device=self.device)
-        out = self.backend.evaluate_actions(action.to(device=self.device, dtype=torch.float32).contiguous())
-        c = (lambda t: t.clone()) if self.copy_outputs else (lambda t: t)
-        obs = OrderedDict([("yaw", c(out["yaw"])), ("freewind_measurements", c(out["freewind"])),
-                           ("wind_speed", c(out["wind_speed"])), ("wind_direction", c(out["wind_direction"]))])
-        K = out["reward"].shape[1]
-        if self.pad_turbines:
-            obs["turbine_mask"] = self._turbine_mask[:, None, :].expand(-1, K, -1)
-        terminated = torch.zeros(self.num_envs, K, dtype=torch.bool, device=self.device)
-        info = {"power": c(out["power"]), "load": c(out["load"])}
-        return obs, c(out["reward"]), terminated, c(out["truncated"].view(torch.bool)), info
+        return action.to(device=self.device, dtype=torch.float32).contiguous()
 
     @property
     def layout_ids(self):
@@ -439,6 +472,22 @@ class VecMAWindFarmEnv(VecWindFarmEnv):
         split = {a: OrderedDict((k, v[:, :, i]) for k, v in obs.items() if k != "freewind_measurements")
                  for a, i in self.agent_name_mapping.items()}
         per_agent_info = {a: {"power": info["power"][:, :, i], "load": info["load"][:, :, i]}
+                          for a, i in self.agent_name_mapping.items()}
+        return (split, {a: reward for a in self.possible_agents}, {a: terminated for a in self.possible_agents},
+                {a: truncated for a in self.possible_agents}, per_agent_info)
+
+    def evaluate_rollouts(self, actions, observations: bool = True):
+        """``VecWindFarmEnv.evaluate_rollouts`` for the agents: ``actions`` is the joint float32 [B, K, H, T] tensor
+        (column k = agent k) or ``{agent: {"yaw": tensor[B, K, H]}}``; returns per-agent dicts as ``step`` does, with the K
+        and H axes, and ``info[agent]["valid"]``."""
+        if isinstance(actions, dict) and actions and next(iter(actions)) in self.agent_name_mapping:
+            actions = torch.stack([torch.as_tensor(actions[a]["yaw"], device=self.device) for a in self.possible_agents], 3)
+        obs, reward, terminated, truncated, info = super().evaluate_rollouts(actions, observations)
+        split = None if obs is None else {
+            a: OrderedDict((k, v[:, :, :, i]) for k, v in obs.items() if k != "freewind_measurements")
+            for a, i in self.agent_name_mapping.items()}
+        per_agent_info = {a: {"power": None if info["power"] is None else info["power"][:, :, :, i],
+                              "load": None if info["load"] is None else info["load"][:, :, :, i], "valid": info["valid"]}
                           for a, i in self.agent_name_mapping.items()}
         return (split, {a: reward for a in self.possible_agents}, {a: terminated for a in self.possible_agents},
                 {a: truncated for a in self.possible_agents}, per_agent_info)
